@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the alignment hot path (BASELINE.json: audio-hours aligned per second).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs B] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one batch of B synthetic pairs per GPU of the C2 shape (22-min
 video audio vs 27-min description, 202 s start offset, injected skips; SURVEY.md 8d): features of both
@@ -32,6 +32,8 @@ import numpy as np
 
 # one CUDA stream per pair in flight: ask for the maximum number of hardware queues before CUDA starts
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
+# the benchmark may run from a read-only tree: it writes nothing there, bytecode caches included
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -66,7 +68,48 @@ def parse_args():
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the rank to the CPUs of its GPU's NUMA node")
     ap.add_argument("--no-long-pair", action="store_true", help="N > 1: skip the long-pair (C5) check that runs on all ranks after the timed steps")
     ap.add_argument("--long-scale", type=float, default=0.1, help="scale of the C5 pair used for the N > 1 long-pair check")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last device-resident step computed as DIR/<name>.npy: pass-1 path, "
+                         "features and final path rows of its first %d distinct pairs, copied inside that step (C5: the nodes "
+                         "and path of the pair); a seeded sample of rows where that exceeds 64 MB" % DUMP_PAIRS)
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm keeps no outputs")
+    return args
+
+
+DUMP_PAIRS = 4
+DUMP_BYTES = 60 << 20       # the arrays; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """arrays: name -> float32 / float64 array, written as out_dir/<name>.npy.  When they hold more than DUMP_BYTES,
+    every array over 1 MB keeps the same fraction of its rows, chosen with a fixed seed and kept in order, and
+    out_dir/<name>_rows.npy lists which rows those are."""
+    os.makedirs(out_dir, exist_ok=True)
+    large = [name for name, a in arrays.items() if a.nbytes > 1 << 20]
+    budget = DUMP_BYTES - sum(a.nbytes for name, a in arrays.items() if name not in large)
+    frac = 1.0
+    if sum(arrays[name].nbytes for name in large) > budget:
+        frac = budget / sum(arrays[name].nbytes + 8 * len(arrays[name]) for name in large)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if name in large and frac < 1.0:
+            rows = np.sort(np.random.default_rng(seed).choice(len(a), size=int(frac * len(a)), replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def pair_arrays(x, y, video_features, audio_features):
+    """What the batch engine hands a caller at the end of stage A, copied out of its slot buffers."""
+    out = {"path1": np.stack([x, y], axis=1).astype(np.float64)}
+    for track, feats in (("video", video_features), ("audio", audio_features)):
+        for f, arr in enumerate(feats):
+            out[f"{track}_feature{f}"] = np.array(arr, dtype=np.float32)
+    return out
 
 
 def make_pairs(n, first_seed, scale, world=1, config="C2"):
@@ -483,6 +526,11 @@ def run_long(args, rank, world, local_rank):
     ms_dev, ph_dev, det, out = run_steps(False)
     launches = (ctx.launches() - l0) * args.steps // (args.steps + args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        nx, ny, sim, path, med = out
+        dump_outputs(args.dump_outputs, {"nodes_x": np.asarray(nx, np.float64), "nodes_y": np.asarray(ny, np.float64),
+                                         "path2": np.asarray(path, np.float64), "similarity": np.array([sim], np.float64),
+                                         "median_slope": np.array([med], np.float64)})
     ms_e2e, ph_e2e, _, _ = run_steps(True)
     lt = torch.tensor([float(launches)], device="cuda", dtype=torch.float64)
     if world > 1:
@@ -638,9 +686,10 @@ def run_ours(args, rank, world, local_rank):
         host_cache[("c4", job.tag)] = {"x": job.x, "y": job.y, **{name: getattr(job, name) for name in
                                        ("kept_x", "kept_y", "gains", "n_audio_scaled", "n_video_scaled", "fit", "clusters", "lines")}}
 
-    def c4_step(host_input: bool):
+    def c4_step(host_input: bool, keep=None):
         """One batch.align_batch call over the 64 episodes (every rank passes the same list; a rank only
-        touches the pairs align_batch assigns to it)."""
+        touches the pairs align_batch assigns to it).  keep: dict that receives the outputs of this rank's
+        first DUMP_PAIRS episodes."""
         lst = [None] * c4_total
         for pos, k in enumerate(c4_mine):
             if host_input:
@@ -658,16 +707,20 @@ def run_ours(args, rank, world, local_rank):
         for k, job in out:
             if isinstance(job, Exception):
                 raise job
+            if keep is not None and len(keep) < DUMP_PAIRS:
+                keep[k] = {**pair_arrays(job.x, job.y, job.video_features, job.audio_features), "path2": job.path}
             results.append({"kernel_ms": job.timings, "work": job.stats, "n_path1": len(job.x), "n_path2": len(job.path), "t_done": 0.0})
         return start.elapsed_time(stop), results
 
-    def one_step(host_input: bool, n_pairs=None, first=0):
+    def one_step(host_input: bool, n_pairs=None, first=0, keep=None):
         if c4_total is not None and n_pairs is None:
-            return c4_step(host_input)
+            return c4_step(host_input, keep)
         """n_pairs pairs through stage A -> (cached) host fit -> stage B, W on the device at a time, all
         driven by this one thread through the engine's event queue.  Returns the device time between an
-        event recorded before the first submit and one recorded after the last result reached the host."""
+        event recorded before the first submit and one recorded after the last result reached the host.
+        keep: dict that receives the outputs of the first DUMP_PAIRS pairs (one per distinct input)."""
         n_pairs = B if n_pairs is None else n_pairs
+        n_keep = 0 if keep is None else min(DUMP_PAIRS, distinct, n_pairs)
         results = [None] * n_pairs
         start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0 = time.perf_counter()
@@ -688,8 +741,12 @@ def run_ours(args, rank, world, local_rank):
                 raise RuntimeError(f"pair {evt.tag} failed on the device: {eng.error(evt)}")
             k = int(evt.tag)
             if evt.kind == _cabi.EVENT_STAGE_A:
+                if k - first < n_keep:
+                    keep[k] = pair_arrays(*eng.path1(evt), eng.features(evt, _cabi.VIDEO), eng.features(evt, _cabi.AUDIO))
                 eng.submit_b(evt.slot, struct=stage_b_struct_for(k, evt))
             else:
+                if k - first < n_keep:
+                    keep[k]["path2"] = eng.rows(evt).copy()
                 results[k - first] = {"kernel_ms": eng.timings(evt), "work": evt.stats.as_dict(), "n_path1": int(evt.n_path1),
                                       "n_path2": int(evt.n_path2), "t_done": time.perf_counter() - t0}
                 eng.release(evt.slot)
@@ -700,15 +757,15 @@ def run_ours(args, rank, world, local_rank):
 
     alloc0 = {}
 
-    def run_steps(host_input):
+    def run_steps(host_input, keep=None):
         for _ in range(args.warmup):
             one_step(host_input)
         barrier()
         l0 = ctx.launches()
         alloc0.update(_cabi.alloc_stats())
         total, res = 0.0, None
-        for _ in range(args.steps):
-            ms, res = one_step(host_input)
+        for s in range(args.steps):
+            ms, res = one_step(host_input, keep=keep if s == args.steps - 1 else None)
             total += ms
         barrier()
         return total / args.steps, ctx.launches() - l0, res
@@ -719,12 +776,15 @@ def run_ours(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     cpu0, wall0 = os.times(), time.perf_counter()
-    ms_dev, launches, res_dev = run_steps(False)
+    kept = {} if rank == 0 and args.dump_outputs else None
+    ms_dev, launches, res_dev = run_steps(False, kept)
     cpu1, wall1 = os.times(), time.perf_counter()
     cpu_cores_busy = ((cpu1.user - cpu0.user) + (cpu1.system - cpu0.system)) / max(wall1 - wall0, 1e-9)
     alloc1 = _cabi.alloc_stats()
     alloc_before = dict(alloc0)     # the e2e steps below update the dict run_steps writes to
     clocks = sampler.stop() if rank == 0 else None
+    if kept is not None:
+        dump_outputs(args.dump_outputs, {f"pair{k}_{name}": arr for k in sorted(kept) for name, arr in kept[k].items()})
     sched0 = eng.counters()
     ms_e2e, _, res_e2e = run_steps(True)
     per_rank = [{"rank": rank, "ms_per_step": ms_dev, "ms_per_step_e2e": ms_e2e, "host_cores_busy": cpu_cores_busy,
