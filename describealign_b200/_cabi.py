@@ -24,7 +24,7 @@ EXPORTS = [
     "dab_pair_get_points2", "dab_pair_get_stats", "dab_pair_get_timings", "dab_launch_count",
     "dab_pair_stage_a_match", "dab_pair_export_points1", "dab_pair_import_points1", "dab_pair_dp1",
     "dab_alloc_pinned", "dab_free_pinned", "dab_trim_pinned", "dab_alloc_stats", "dab_host_copy",
-    "dab_set_host_wait", "dab_pair_get_timeline", "dab_pair_stage_b_gains",
+    "dab_set_host_wait", "dab_pair_get_timeline",
     "dab_set_log10f_correction", "dab_eval_log10f",
     "dab_pair_set_gate_energy", "dab_pair_stage_b_clusters", "dab_pair_get_corridors",
     "dab_pair_stage_b_score", "dab_pair_export_quals2", "dab_pair_import_quals2", "dab_pair_dp2",
@@ -83,9 +83,8 @@ class Event(ctypes.Structure):
 class StageBIn(ctypes.Structure):
     """dab_stage_b_in"""
     _fields_ = [("gain", ctypes.c_float * 3), ("audio_std", ctypes.c_float * 3),
-                ("audio_energy_max", ctypes.c_float), ("video_energy_max", ctypes.c_float),
-                ("n_audio", ctypes.c_int64), ("n_video", ctypes.c_int64), ("corridors", ctypes.c_void_p),
-                ("n_corridors", ctypes.c_int32), ("n_clusters", ctypes.c_int32), ("clusters", ctypes.c_void_p)]
+                ("n_audio", ctypes.c_int64), ("n_video", ctypes.c_int64),
+                ("n_clusters", ctypes.c_int32), ("clusters", ctypes.c_void_p)]
 
 
 EVENT_STAGE_A, EVENT_STAGE_B = 1, 2
@@ -196,7 +195,7 @@ def load() -> ctypes.CDLL:
     lib.dab_engine_slot_pair.restype = vp
     lib.dab_engine_counters.argtypes = [vp, ctypes.POINTER(ctypes.c_int64 * 4)]
     lib.dab_engine_counters.restype = None
-    if lib.dab_abi_version() != 1:
+    if lib.dab_abi_version() != 2:
         raise DabError("libdescribealign_b200.so has an unexpected ABI version")
     _lib = lib
     return lib
@@ -466,27 +465,6 @@ class Pair:
         self.n_points2, self.n_path2 = npts.value, npath.value
         return npts.value, npath.value
 
-    def stage_b_gains(self, gains, audio_stds, audio_scaled: np.ndarray, video_scaled: np.ndarray, plans, n_clusters: int):
-        """Stage B for a pair that holds its features on the device: the scaled arrays are rebuilt
-        there from the six scalars; the host copies only provide lengths and energy maxima."""
-        g = (ctypes.c_float * 3)(*[float(x) for x in gains])
-        sd = (ctypes.c_float * 3)(*[float(x) for x in audio_stds])
-        plans = [p for p in plans if p[2] > p[1]]
-        arr = (Corridor * max(len(plans), 1))()
-        for k, (idx, lo, hi, slope, offset) in enumerate(plans):
-            arr[k] = Corridor(int(idx), int(lo), int(hi), 0, float(slope), float(offset))
-        npts, npath = ctypes.c_int64(), ctypes.c_int64()
-        fn = self.lib.dab_pair_stage_b_gains
-        fn.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_float * 3), ctypes.POINTER(ctypes.c_float * 3),
-                       ctypes.c_int64, ctypes.c_int64, ctypes.c_float, ctypes.c_float, ctypes.c_void_p, ctypes.c_int32,
-                       ctypes.c_int32, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]
-        self.ctx.check(fn(self.handle, ctypes.byref(g), ctypes.byref(sd), audio_scaled.shape[0], video_scaled.shape[0],
-                          float(audio_scaled[:, 0].max()), float(video_scaled[:, 0].max()),
-                          ctypes.cast(arr, ctypes.c_void_p), len(plans), int(n_clusters),
-                          ctypes.byref(npts), ctypes.byref(npath)))
-        self.n_points2, self.n_path2 = npts.value, npath.value
-        return npts.value, npath.value
-
     def stage_b_clusters(self, gains, audio_stds, n_audio: int, n_video: int, lines):
         """Stage B from the host fit's line clusters [(cluster index, x_first, x_last, offset, slope), ...]:
         scaling, corridor planning (describealign.py:895-932), scoring, DP 2 and traceback on the device."""
@@ -687,40 +665,22 @@ class Engine:
         return {name: float(evt.timings_ms[k]) for k, name in enumerate(TIMING_SLOTS)}
 
     @staticmethod
-    def stage_b_struct(gains, audio_stds, n_audio: int, n_video: int, audio_energy_max: float = 0.0,
-                       video_energy_max: float = 0.0, plans=(), n_clusters: int = 0, lines=None):
+    def stage_b_struct(gains, audio_stds, n_audio: int, n_video: int, lines):
         """The dab_stage_b_in of a host fit (reusable: the engine copies the arrays on submit).
-        lines: the fit's line clusters (host_fit.cluster_lines) - the corridors are then planned on the
-        device; else plans: pre-planned corridors with the energy maxima."""
+        lines: the fit's line clusters (host_fit.cluster_lines); the corridors are planned on the device."""
         b = StageBIn()
-        if lines is not None:
-            for k in range(3):
-                b.gain[k] = float(gains[k])
-                b.audio_std[k] = float(audio_stds[k])
-            b.n_audio, b.n_video = int(n_audio), int(n_video)
-            arr = cluster_array(lines)
-            b.clusters = ctypes.cast(arr, ctypes.c_void_p)
-            b.n_corridors, b.n_clusters = 0, len(lines)
-            b._cluster_array = arr
-            return b
         for k in range(3):
             b.gain[k] = float(gains[k])
             b.audio_std[k] = float(audio_stds[k])
-        b.audio_energy_max, b.video_energy_max = float(audio_energy_max), float(video_energy_max)
         b.n_audio, b.n_video = int(n_audio), int(n_video)
-        plans = [p for p in plans if p[2] > p[1]]
-        arr = (Corridor * max(len(plans), 1))()
-        for k, (idx, lo, hi, slope, offset) in enumerate(plans):
-            arr[k] = Corridor(int(idx), int(lo), int(hi), 0, float(slope), float(offset))
-        b.corridors = ctypes.cast(arr, ctypes.c_void_p)
-        b.n_corridors, b.n_clusters = len(plans), int(n_clusters)
-        b._corridor_array = arr          # keeps the array alive as long as the struct
+        arr = cluster_array(lines)
+        b.clusters = ctypes.cast(arr, ctypes.c_void_p)
+        b.n_clusters = len(lines)
+        b._cluster_array = arr           # keeps the array alive as long as the struct
         return b
 
-    def submit_b(self, slot: int, gains=None, audio_stds=None, n_audio=0, n_video=0, audio_energy_max=0.0,
-                 video_energy_max=0.0, plans=(), n_clusters=0, lines=None, struct: StageBIn | None = None):
-        b = struct if struct is not None else self.stage_b_struct(gains, audio_stds, n_audio, n_video, audio_energy_max,
-                                                                   video_energy_max, plans, n_clusters, lines)
+    def submit_b(self, slot: int, gains=None, audio_stds=None, n_audio=0, n_video=0, lines=(), struct: StageBIn | None = None):
+        b = struct if struct is not None else self.stage_b_struct(gains, audio_stds, n_audio, n_video, lines)
         self.ctx.check(self.lib.dab_engine_submit_b(self.handle, int(slot), ctypes.byref(b)))
 
     def release(self, slot: int):

@@ -176,9 +176,6 @@ class AlignJob:
         self._own = pair is None and not detached
         self.video_features = self.audio_features = None
         self.want_all_features = False
-        self.device_scaling = True   # stage B scales the pair's device-resident features itself (6 floats up)
-        self.device_planning = True  # ... and plans the corridors there (describealign.py:895-932, csrc/refine.cuh)
-        self.test_planner = None     # tests: a host-side corridor planner to compare the device's planning with
         self.gains = None
         self.h2d_bytes = self.d2h_bytes = 0
         self.host_ms = {}        # wall time of each host-side call of this job (diagnostics)
@@ -253,7 +250,7 @@ class AlignJob:
             raise RuntimeError(FAILED_MSG)
 
     def stage_b_input(self):
-        """What dab_engine_submit_b / dab_pair_stage_b_gains need from the host fit."""
+        """What dab_engine_submit_b / dab_pair_stage_b_clusters need from the host fit."""
         return dict(gains=self.gains[0], audio_stds=self.gains[1], n_audio=self.n_audio_scaled,
                     n_video=self.n_video_scaled, lines=self.lines)
 
@@ -271,24 +268,10 @@ class AlignJob:
 
     def device_stage_b(self):
         """Scaling (describealign.py:737-741), corridor planning (:895-932), scoring, DP 2 and traceback on
-        the device, from the host fit's six scalars and line clusters.  (device_planning / device_scaling
-        off: the oracle's numpy planning / uploaded scaled arrays instead - test switches.)"""
-        if self.device_planning and self.device_scaling:
-            self._timed("stage_b", self.pair.stage_b_clusters, self.gains[0], self.gains[1], self.n_audio_scaled,
-                        self.n_video_scaled, self.lines)
-            self.h2d_bytes += 24 + 40 * len(self.lines)
-        else:
-            audio_scaled, video_scaled = host_fit.scale_features(self.video_features, self.audio_features, self.kept_x, self.kept_y)
-            if self.test_planner is None:
-                raise RuntimeError("device_planning / device_scaling are test switches: they need job.test_planner")
-            plans = self.test_planner(self.clusters, audio_scaled, video_scaled)
-            if self.device_scaling:
-                self._timed("stage_b", self.pair.stage_b_gains, self.gains[0], self.gains[1], audio_scaled,
-                            video_scaled, plans, len(self.clusters))
-                self.h2d_bytes += 24
-            else:
-                self._timed("stage_b", self.pair.stage_b, audio_scaled, video_scaled, plans, len(self.clusters))
-                self.h2d_bytes += audio_scaled.nbytes + video_scaled.nbytes
+        the device, from the host fit's six scalars and line clusters."""
+        self._timed("stage_b", self.pair.stage_b_clusters, self.gains[0], self.gains[1], self.n_audio_scaled,
+                    self.n_video_scaled, self.lines)
+        self.h2d_bytes += 24 + 40 * len(self.lines)
         self.path = self._timed("path2", self.pair.path2)
         self.d2h_bytes += self.path.nbytes
         if len(self.path) < self.min_len:

@@ -200,8 +200,6 @@ void dab_destroy(dab_ctx *ctx) { delete ctx; }
 
 int dab_set_option(dab_ctx *ctx, const char *name, int64_t value) {
   if (!ctx || !name) return DAB_E_ARG;
-  if (strcmp(name, "dp2_generic") == 0) { ctx->opt_dp2_generic = value != 0; return DAB_OK; }
-  if (strcmp(name, "dp_reserve_kb") == 0 && value >= 0 && value <= 176) { ctx->opt_dp_reserve_kb = (int)value; return DAB_OK; }
   if (strcmp(name, "dp2_impl") == 0 && (value == 0 || value == 2)) { ctx->opt_dp2_impl = (int)value; return DAB_OK; }
   dab_set_err(ctx, std::string("dab_set_option: unknown option ") + name);
   return DAB_E_ARG;
@@ -532,47 +530,11 @@ int dab_pair_dp1(dab_pair *pr, int64_t *n_path) {
   return DAB_OK;
 }
 
-// shared by the stage-B entry points: corridor checks and upload, then the stage is enqueued
-static int stage_b_enqueue_common(dab_pair *pr, int64_t n_audio, int64_t n_video, const dab_corridor *corridors,
-                                  int32_t n_corridors, int32_t n_clusters, float amax, float vmax) {
+// the end of every synchronous stage-B entry: counts to the host, wait, collect
+static int finish_stage_b(dab_pair *pr, int64_t *n_points, int64_t *n_path) {
   dab_ctx *ctx = pr->ctx;
-  cudaStream_t st = pr->stream;
-  for (int k = 0; k < n_corridors; ++k) {
-    const dab_corridor &c = corridors[k];
-    if (c.cluster < 0 || c.cluster >= n_clusters || c.lo < 0 || c.hi > n_audio ||
-        (k > 0 && c.cluster <= corridors[k - 1].cluster)) {
-      dab_set_err(ctx, "dab_pair_stage_b: corridors must be in ascending cluster order with rows inside the audio track");
-      return DAB_E_ARG;
-    }
-    if (c.hi > c.lo) {
-      // the line must stay inside the video feature array for every scored row (:898-899)
-      const double j0 = c.slope * (double)c.lo + c.offset, j1 = c.slope * (double)(c.hi - 1) + c.offset;
-      const double jmin = j0 < j1 ? j0 : j1, jmax = j0 < j1 ? j1 : j0;
-      if (!(jmin >= 0.0) || !(jmax < (double)(n_video - 1))) {
-        dab_set_err(ctx, "dab_pair_stage_b: corridor line leaves the video track");
-        return DAB_E_ARG;
-      }
-    }
-  }
-  pr->b_device_planned = false;
-  pr->h_cor.assign(corridors, corridors + n_corridors);
-  DAB_TRY(dab_ensure(ctx, pr->corridors, sizeof(dab_corridor) * (size_t)(n_corridors + 1)));
-  if (n_corridors > 0)
-    DAB_CUDA(cudaMemcpyAsync(pr->corridors.p, corridors, sizeof(dab_corridor) * (size_t)n_corridors, cudaMemcpyHostToDevice, st));
-  pr->b_amax = amax;
-  pr->b_vmax = vmax;
-  pr->stats.n_audio_frames = n_audio;
-  pr->stats.n_video_frames = n_video;
-  return dab_enqueue_stage_b(pr, n_corridors, n_clusters);
-}
-
-static int stage_b_common(dab_pair *pr, int64_t n_audio, int64_t n_video, const dab_corridor *corridors,
-                          int32_t n_corridors, int32_t n_clusters, float amax, float vmax, int64_t *n_points,
-                          int64_t *n_path) {
-  dab_ctx *ctx = pr->ctx;
-  DAB_TRY(stage_b_enqueue_common(pr, n_audio, n_video, corridors, n_corridors, n_clusters, amax, vmax));
   DAB_TRY(dab_enqueue_counts(pr));
-  DAB_CUDA(dab_wait_stream(pr->stream));     // (corridors is the caller's array: it has been consumed by now)
+  DAB_CUDA(dab_wait_stream(pr->stream));
   DAB_TRY(dab_collect_stage_b(pr));
   if (n_points) *n_points = pr->n_points2;
   if (n_path) *n_path = pr->n_path2;
@@ -591,17 +553,39 @@ int dab_pair_stage_b(dab_pair *pr, const float *audio_scaled, int64_t n_audio, c
     dab_set_err(ctx, "dab_pair_stage_b: invalid argument");
     return DAB_E_ARG;
   }
+  for (int k = 0; k < n_corridors; ++k) {
+    const dab_corridor &c = corridors[k];
+    if (c.cluster < 0 || c.cluster >= n_clusters || c.lo < 0 || c.hi > n_audio ||
+        (k > 0 && c.cluster <= corridors[k - 1].cluster)) {
+      dab_set_err(ctx, "dab_pair_stage_b: corridors must be in ascending cluster order with rows inside the audio track");
+      return DAB_E_ARG;
+    }
+    if (c.hi > c.lo) {
+      // the line must stay inside the video feature array for every scored row (:898-899)
+      const double j0 = c.slope * (double)c.lo + c.offset, j1 = c.slope * (double)(c.hi - 1) + c.offset;
+      const double jmin = j0 < j1 ? j0 : j1, jmax = j0 < j1 ? j1 : j0;
+      if (!(jmin >= 0.0) || !(jmax < (double)(n_video - 1))) {
+        dab_set_err(ctx, "dab_pair_stage_b: corridor line leaves the video track");
+        return DAB_E_ARG;
+      }
+    }
+  }
   DAB_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = pr->stream;
   DAB_TRY(dab_ensure(ctx, pr->a_scaled, sizeof(float) * 3 * (size_t)n_audio));
   DAB_TRY(dab_ensure(ctx, pr->v_scaled, sizeof(float) * 3 * (size_t)n_video));
   DAB_CUDA(cudaMemcpyAsync(pr->a_scaled.p, audio_scaled, sizeof(float) * 3 * (size_t)n_audio, cudaMemcpyHostToDevice, st));
   DAB_CUDA(cudaMemcpyAsync(pr->v_scaled.p, video_scaled, sizeof(float) * 3 * (size_t)n_video, cudaMemcpyHostToDevice, st));
-  // np.max of the energy columns (:908-909)
-  float amax = audio_scaled[0], vmax = video_scaled[0];
-  for (int64_t k = 1; k < n_audio; ++k) amax = audio_scaled[3 * k] > amax ? audio_scaled[3 * k] : amax;
-  for (int64_t k = 1; k < n_video; ++k) vmax = video_scaled[3 * k] > vmax ? video_scaled[3 * k] : vmax;
-  return stage_b_common(pr, n_audio, n_video, corridors, n_corridors, n_clusters, amax, vmax, n_points, n_path);
+  DAB_TRY(dab_enqueue_column_maxes(pr, n_audio, n_video));
+  pr->b_device_planned = false;
+  pr->h_cor.assign(corridors, corridors + n_corridors);
+  DAB_TRY(dab_ensure(ctx, pr->corridors, sizeof(dab_corridor) * (size_t)(n_corridors + 1)));
+  if (n_corridors > 0)
+    DAB_CUDA(cudaMemcpyAsync(pr->corridors.p, corridors, sizeof(dab_corridor) * (size_t)n_corridors, cudaMemcpyHostToDevice, st));
+  pr->stats.n_audio_frames = n_audio;
+  pr->stats.n_video_frames = n_video;
+  DAB_TRY(dab_enqueue_stage_b(pr, n_corridors, n_clusters));
+  return finish_stage_b(pr, n_points, n_path);   // (the caller's arrays have been consumed once it returns)
 }
 
 }  // extern "C"
@@ -620,21 +604,7 @@ __global__ void scale_features_kernel(const float *f0, const float *f1, const fl
   out[3 * k + 2] = __fdiv_rn(x2, s2);
 }
 
-// Stage B for a pair that holds its features: scaling kernels + the stage, enqueued without waiting.
-// `corridors` must stay valid until the stream has consumed it (page-locked memory owned by the caller).
 static int enqueue_scaling(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video);
-
-int dab_enqueue_stage_b_gains(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video,
-                              float amax, float vmax, const dab_corridor *corridors, int32_t n_corridors, int32_t n_clusters,
-                              const dab_corridor *) {
-  dab_ctx *ctx = pr->ctx;
-  if (n_corridors < 0 || n_clusters < 0 || (n_corridors > 0 && !corridors)) {
-    dab_set_err(ctx, "dab_pair_stage_b_gains: invalid argument");
-    return DAB_E_ARG;
-  }
-  DAB_TRY(enqueue_scaling(pr, gain, audio_std, n_audio, n_video));
-  return stage_b_enqueue_common(pr, n_audio, n_video, corridors, n_corridors, n_clusters, amax, vmax);
-}
 
 // stage B from line clusters: scaling, corridor planning on the device, then the stage itself
 int dab_enqueue_stage_b_clusters(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video,
@@ -658,10 +628,10 @@ static int enqueue_scaling(dab_pair *pr, const float gain[3], const float audio_
     return DAB_E_ARG;
   }
   Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
-  if (!V.have_features || !A.have_features) { dab_set_err(ctx, "dab_pair_stage_b_gains: the pair holds no features"); return DAB_E_STATE; }
+  if (!V.have_features || !A.have_features) { dab_set_err(ctx, "stage B: the pair holds no features"); return DAB_E_STATE; }
   // np.stack truncates to the shortest of the three vectors (energy may be one longer)
   const int64_t na = A.L < A.Le ? A.L : A.Le, nv = V.L < V.Le ? V.L : V.Le;
-  if (n_audio != na || n_video != nv) { dab_set_err(ctx, "dab_pair_stage_b_gains: lengths differ from the pair's features"); return DAB_E_ARG; }
+  if (n_audio != na || n_video != nv) { dab_set_err(ctx, "stage B: lengths differ from the pair's features"); return DAB_E_ARG; }
   DAB_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = pr->stream;
   DAB_TRY(dab_ensure(ctx, pr->a_scaled, sizeof(float) * 3 * (size_t)n_audio));
@@ -677,38 +647,14 @@ static int enqueue_scaling(dab_pair *pr, const float gain[3], const float audio_
 
 extern "C" {
 
-int dab_pair_stage_b_gains(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio,
-                           int64_t n_video, float audio_energy_max, float video_energy_max,
-                           const dab_corridor *corridors, int32_t n_corridors, int32_t n_clusters,
-                           int64_t *n_points, int64_t *n_path) {
-  if (!pr) return DAB_E_ARG;
-  dab_ctx *ctx = pr->ctx;
-  StreamScope scope__(pr->stream);
-  ApiTimer timer__(&pr->api_us[2]);
-  DAB_TRY(dab_enqueue_stage_b_gains(pr, gain, audio_std, n_audio, n_video, audio_energy_max, video_energy_max, corridors,
-                                    n_corridors, n_clusters, nullptr));
-  DAB_TRY(dab_enqueue_counts(pr));
-  DAB_CUDA(dab_wait_stream(pr->stream));
-  DAB_TRY(dab_collect_stage_b(pr));
-  if (n_points) *n_points = pr->n_points2;
-  if (n_path) *n_path = pr->n_path2;
-  return DAB_OK;
-}
-
 int dab_pair_stage_b_clusters(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio,
                               int64_t n_video, const dab_cluster *clusters, int32_t n_clusters,
                               int64_t *n_points, int64_t *n_path) {
   if (!pr) return DAB_E_ARG;
-  dab_ctx *ctx = pr->ctx;
   StreamScope scope__(pr->stream);
   ApiTimer timer__(&pr->api_us[2]);
   DAB_TRY(dab_enqueue_stage_b_clusters(pr, gain, audio_std, n_audio, n_video, clusters, n_clusters));
-  DAB_TRY(dab_enqueue_counts(pr));
-  DAB_CUDA(dab_wait_stream(pr->stream));
-  DAB_TRY(dab_collect_stage_b(pr));
-  if (n_points) *n_points = pr->n_points2;
-  if (n_path) *n_path = pr->n_path2;
-  return DAB_OK;
+  return finish_stage_b(pr, n_points, n_path);
 }
 
 // ---- stage B in steps, for one very long pair split over several GPUs (SURVEY.md 8e) ----
@@ -787,11 +733,7 @@ int dab_pair_dp2(dab_pair *pr, int64_t *n_path) {
   ApiTimer timer__(&pr->api_us[2]);
   DAB_CUDA(cudaSetDevice(ctx->device));
   DAB_TRY(dab_enqueue_stage_b_dp(pr, pr->b_n_cor, pr->b_n_clusters));
-  DAB_TRY(dab_enqueue_counts(pr));
-  DAB_CUDA(dab_wait_stream(pr->stream));
-  DAB_TRY(dab_collect_stage_b(pr));
-  if (n_path) *n_path = pr->n_path2;
-  return DAB_OK;
+  return finish_stage_b(pr, nullptr, n_path);
 }
 
 int dab_pair_get_corridors(dab_pair *pr, dab_corridor *out, int32_t cap, int32_t *n_corridors) {

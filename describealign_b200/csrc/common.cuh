@@ -29,8 +29,6 @@ struct dab_ctx {
   std::mutex err_mu;
   std::atomic<int64_t> launches{0};   // kernels launched through this context (many host threads)
   int sm_count = 148;
-  int opt_dp2_generic = 0;   // force the tree DP for pass 2 (testing)
-  int opt_dp_reserve_kb = 0; // dynamic shared memory the pass-2 DP kernel asks for without using it (see dab_set_option)
   int opt_dp2_impl = 0;      // 0 scan kernel (dp2_scan.cuh), 2 generic tree DP (both exact; the tests compare them)
 };
 
@@ -106,9 +104,8 @@ struct dab_pair {
   DevBuf path2;                // f64 (n,5)
   int64_t n_points2 = 0, n_path2 = 0;
   int64_t cap_points2 = 0;     // upper bound of pass-2 points of the current stage_b call (sum of corridor rows)
-  float b_amax = 0.f, b_vmax = 0.f;   // np.max of the scaled energy columns (describealign.py:908-909)
   int32_t b_n_cor = 0, b_n_clusters = 0;   // of the stage-B call in progress (dab_pair_stage_b_score .. dab_pair_dp2)
-  bool b_device_planned = false;      // corridors and energy maxima come from the device (dab_pair_stage_b_clusters)
+  bool b_device_planned = false;      // corridors were planned on the device (dab_enqueue_plan_corridors), not uploaded
   DevBuf clusters, refine_partial, maxes;
   dab_stats stats = {};
   cudaEvent_t ev[32] = {};
@@ -217,11 +214,11 @@ int dab_enqueue_stage_b_points(dab_pair *pr, int32_t n_corridors, int32_t n_clus
 int dab_enqueue_stage_b_dp(dab_pair *pr, int32_t n_corridors, int32_t n_clusters);
 int dab_enqueue_set_quals2(dab_pair *pr, const double *d_q_all);
 int dab_row_range_points2(dab_pair *pr, int64_t lo, int64_t hi, int64_t *first, int64_t *count);
+int dab_enqueue_column_maxes(dab_pair *pr, int64_t n_audio, int64_t n_video);
 int dab_enqueue_plan_corridors(dab_pair *pr, const dab_cluster *clusters, int32_t n_clusters, int64_t n_audio, int64_t n_video);
 int dab_collect_stage_b(dab_pair *pr);
 int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *v_video, const double *qual,
                            int64_t n, int src_on_device);
-int dab_run_stage_b(dab_pair *pr, int32_t n_corridors, int32_t n_clusters);
 
 #define DAB_LAUNCHED(pr) ((pr)->ctx->launches++)
 

@@ -45,9 +45,8 @@ struct Slot {
   int status = DAB_OK;
   std::string err;
   int attempts = 0;
-  PinBuf path_x, path_y, feat[2][3], rows, cor;
+  PinBuf path_x, path_y, feat[2][3], rows, cor;   // cor: the line clusters of the stage-B input
   dab_stage_b_in b_in = {};
-  bool b_from_clusters = false;
   int64_t host_us = 0;               // scheduler time spent enqueueing this pair's work
   int64_t t_submit_us = 0, t_a_done_us = 0, t_b_submit_us = 0;
 };
@@ -190,10 +189,7 @@ void publish_a(dab_engine *e, int slot) {
 
 }  // namespace
 
-// scale_features_kernel lives in api.cu
-int dab_enqueue_stage_b_gains(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video,
-                              float amax, float vmax, const dab_corridor *corridors, int32_t n_corridors, int32_t n_clusters,
-                              const dab_corridor *corridors_pinned);
+// in api.cu
 int dab_enqueue_stage_b_clusters(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video,
                                  const dab_cluster *clusters, int32_t n_clusters);
 
@@ -205,14 +201,8 @@ void enqueue_b(dab_engine *e, int slot) {
   StreamScope scope__(pr->stream);
   const int64_t t0 = now_us();
   const dab_stage_b_in &b = s.b_in;
-  if (s.b_from_clusters)
-    ENG_TRY(dab_enqueue_stage_b_clusters(pr, b.gain, b.audio_std, b.n_audio, b.n_video,
-                                         reinterpret_cast<const dab_cluster *>(s.cor.p), b.n_clusters), DAB_EVENT_STAGE_B);
-  else
-    ENG_TRY(dab_enqueue_stage_b_gains(pr, b.gain, b.audio_std, b.n_audio, b.n_video, b.audio_energy_max, b.video_energy_max,
-                                      reinterpret_cast<const dab_corridor *>(s.cor.p), b.n_corridors, b.n_clusters,
-                                      reinterpret_cast<const dab_corridor *>(s.cor.p)),
-            DAB_EVENT_STAGE_B);
+  ENG_TRY(dab_enqueue_stage_b_clusters(pr, b.gain, b.audio_std, b.n_audio, b.n_video,
+                                       reinterpret_cast<const dab_cluster *>(s.cor.p), b.n_clusters), DAB_EVENT_STAGE_B);
   ENG_TRY(dab_enqueue_counts(pr), DAB_EVENT_STAGE_B);
   ENG_CUDA(cudaEventRecord(s.ev, pr->stream), DAB_EVENT_STAGE_B);
   s.state = S_B_RUN;
@@ -397,21 +387,13 @@ int dab_engine_next(dab_engine *e, dab_event *out, int32_t timeout_ms) {
 }
 
 int dab_engine_submit_b(dab_engine *e, int32_t slot, const dab_stage_b_in *in) {
-  if (!e || !in || slot < 0 || slot >= (int)e->slots.size() || in->n_corridors < 0 || in->n_clusters < 0 ||
-      (in->n_corridors > 0 && !in->corridors && !in->clusters))
+  if (!e || !in || slot < 0 || slot >= (int)e->slots.size() || in->n_clusters < 0 || (in->n_clusters > 0 && !in->clusters))
     return DAB_E_ARG;
   Slot &s = e->slots[(size_t)slot];
   // the slot is in S_A_HOST: it belongs to the caller until this request is queued
-  s.b_from_clusters = in->clusters != nullptr;
-  if (s.b_from_clusters) {
-    if (s.cor.ensure(sizeof(dab_cluster) * (size_t)(in->n_clusters + 1))) return DAB_E_CUDA;
-    if (in->n_clusters) memcpy(s.cor.p, in->clusters, sizeof(dab_cluster) * (size_t)in->n_clusters);
-  } else {
-    if (s.cor.ensure(sizeof(dab_corridor) * (size_t)(in->n_corridors + 1))) return DAB_E_CUDA;
-    if (in->n_corridors) memcpy(s.cor.p, in->corridors, sizeof(dab_corridor) * (size_t)in->n_corridors);
-  }
+  if (s.cor.ensure(sizeof(dab_cluster) * (size_t)(in->n_clusters + 1))) return DAB_E_CUDA;
+  if (in->n_clusters) memcpy(s.cor.p, in->clusters, sizeof(dab_cluster) * (size_t)in->n_clusters);
   s.b_in = *in;
-  s.b_in.corridors = nullptr;
   s.b_in.clusters = nullptr;
   s.t_b_submit_us = now_us();
   {

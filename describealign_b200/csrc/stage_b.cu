@@ -37,8 +37,7 @@ struct ScoreBArgs {
   int64_t n_a, n_v;
   const dab_corridor *cor;
   int32_t n_cor;
-  float a_max, v_max;
-  const float *maxes;      // device copy of (a_max, v_max) when they were computed on the device, else null
+  const float *maxes;      // np.max of the audio / video energy columns (dab_enqueue_column_maxes)
   int32_t *row_count;
   const int32_t *row_off;
   int32_t *p_i, *p_c, *p_rank;
@@ -117,7 +116,7 @@ __global__ void corridor_kernel(ScoreBArgs s) {
       const double t1 = -.5 - log10(1e-4 + fabs((double)a1 - vl1));
       const double t2 = -.5 - log10(1e-4 + fabs((double)a2 - vl2));
       q = (t0 + t1) + t2;
-      const float v_max = s.maxes ? s.maxes[1] : s.v_max, a_max = s.maxes ? s.maxes[0] : s.a_max;
+      const float v_max = s.maxes[1], a_max = s.maxes[0];
       q = q * fmin(fmax((vl0 + 2.5) - (double)v_max, 0.0), 1.0);
       // the audio gate is evaluated in float32 by numpy (f32 array, weak Python scalars)
       float ag = (a0 + 2.5f) - a_max;
@@ -443,7 +442,7 @@ struct Dp2LArgs {
 // The corridor-state DP needs: at most 32 corridors, positive slopes, every coordinate >= 3 (so the
 // seeded prev_cache cell 0 is never in reach; x_limits keeps lines >= 4, describealign.py:898).
 static bool corridor_dp_eligible(const dab_pair *pr, int32_t n_cor) {
-  if (pr->ctx->opt_dp2_generic || pr->ctx->opt_dp2_impl == 2 || n_cor > 32) return false;   // dp2_impl 2: the tree DP (cross-checks)
+  if (pr->ctx->opt_dp2_impl == 2 || n_cor > 32) return false;   // dp2_impl 2: the tree DP (cross-checks)
   for (int k = 0; k < n_cor; ++k) {
     const dab_corridor &c = pr->h_cor[k];
     if (!(c.slope > 0.0)) return false;
@@ -466,6 +465,20 @@ static void host_x_limits(double x_first, double x_last, double offset, double s
   const long long h2 = to_ll(floor(((double)(n_v - 4) - offset) / slope));
   if (l2 > lo) lo = l2;
   if (h2 < hi) hi = h2;
+}
+
+// np.max of the energy columns of the scaled arrays (describealign.py:908-909) into pr->maxes[0] (audio),
+// pr->maxes[1] (video); enqueued after the scaled arrays, before the corridor scoring that reads them.
+int dab_enqueue_column_maxes(dab_pair *pr, int64_t n_a, int64_t n_v) {
+  dab_ctx *ctx = pr->ctx;
+  cudaStream_t st = pr->stream;
+  DAB_TRY(dab_ensure(ctx, pr->maxes, sizeof(float) * 4));
+  unsigned int *max_keys = reinterpret_cast<unsigned int *>(pr->maxes.as<float>() + 2);
+  DAB_CUDA(cudaMemsetAsync(max_keys, 0, 2 * sizeof(unsigned int), st));
+  column_max_kernel<<<dim3(64, 2), 256, 0, st>>>(pr->a_scaled.as<float>(), n_a, pr->v_scaled.as<float>(), n_v, max_keys);
+  column_max_decode_kernel<<<1, 32, 0, st>>>(max_keys, pr->maxes.as<float>());
+  ctx->launches += 2;
+  return DAB_OK;
 }
 
 // Corridor planning on the device (refine.cuh).  `clusters` is read by an asynchronous copy: it must stay
@@ -500,12 +513,7 @@ int dab_enqueue_plan_corridors(dab_pair *pr, const dab_cluster *clusters, int32_
   DAB_TRY(dab_ensure(ctx, pr->clusters, sizeof(dab_cluster) * (size_t)(n_clusters + 1)));
   DAB_TRY(dab_ensure(ctx, pr->corridors, sizeof(dab_corridor) * (size_t)(n_clusters + 1)));
   DAB_TRY(dab_ensure(ctx, pr->refine_partial, sizeof(double) * 4 * (size_t)max_blocks * (size_t)(n_clusters + 1)));
-  DAB_TRY(dab_ensure(ctx, pr->maxes, sizeof(float) * 4));
-  unsigned int *max_keys = reinterpret_cast<unsigned int *>(pr->maxes.as<float>() + 2);
-  DAB_CUDA(cudaMemsetAsync(max_keys, 0, 2 * sizeof(unsigned int), st));
-  column_max_kernel<<<dim3(64, 2), 256, 0, st>>>(pr->a_scaled.as<float>(), n_a, pr->v_scaled.as<float>(), n_v, max_keys);
-  column_max_decode_kernel<<<1, 32, 0, st>>>(max_keys, pr->maxes.as<float>());
-  ctx->launches += 2;
+  DAB_TRY(dab_enqueue_column_maxes(pr, n_a, n_v));
   if (n_clusters > 0) {
     DAB_CUDA(cudaMemcpyAsync(pr->clusters.p, clusters, sizeof(dab_cluster) * (size_t)n_clusters, cudaMemcpyHostToDevice, st));
     RefineArgs ra;
@@ -553,9 +561,7 @@ int dab_enqueue_stage_b_points(dab_pair *pr, int32_t n_cor, int32_t n_clusters, 
   sb.a_scaled = pr->a_scaled.as<float>(); sb.v_scaled = pr->v_scaled.as<float>();
   sb.n_a = n_a; sb.n_v = n_v;
   sb.cor = pr->corridors.as<dab_corridor>(); sb.n_cor = n_cor;
-  sb.a_max = pr->b_amax;
-  sb.v_max = pr->b_vmax;
-  sb.maxes = pr->b_device_planned ? pr->maxes.as<float>() : nullptr;
+  sb.maxes = pr->maxes.as<float>();
   sb.want_rank = fast ? 0 : 1;
   sb.q_lo = q_lo; sb.q_hi = q_hi;
   DAB_TRY(dab_ensure(ctx, pr->row2_count, sizeof(int32_t) * (size_t)(n_a + 2)));
@@ -740,12 +746,4 @@ int dab_collect_stage_b(dab_pair *pr) {
   pr->stats.n_dp2_neighbour = cnt[2];
   pr->stats.n_dp2_run_points = cnt[3];
   return DAB_OK;
-}
-
-int dab_run_stage_b(dab_pair *pr, int32_t n_cor, int32_t n_clusters) {
-  dab_ctx *ctx = pr->ctx;
-  DAB_TRY(dab_enqueue_stage_b(pr, n_cor, n_clusters));
-  DAB_TRY(dab_enqueue_counts(pr));
-  DAB_CUDA(dab_wait_stream(pr->stream));
-  return dab_collect_stage_b(pr);
 }

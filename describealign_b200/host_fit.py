@@ -112,40 +112,28 @@ def continuity_error_numpy(x, y, deriv=False, window=None):
     return err
 
 
-def scale_features(video_features, audio_features, x, y, return_gains=False):
+def scale_features(video_features, audio_features, x, y):
     """Least-squares gain per feature, keep the first three, stack as (len, 3) float32
-    (describealign.py:733-741).  x = audio indices, y = video indices of the kept path.
-    return_gains: also return (gains, audio_stds), the six scalars the scaled arrays are made from
-    (float32 arrays of 3, or None when a feature is not float32 and the device cannot redo the
-    arithmetic from them)."""
-    a_cols, v_cols, gains, stds = [], [], [], []
+    (describealign.py:733-741).  x = audio indices, y = video indices of the kept path."""
+    a_cols, v_cols = [], []
     for v_feat, a_feat in list(zip(video_features, audio_features))[:3]:
         a_std = np.std(a_feat)
         gain = np.linalg.lstsq(v_feat[y][:, None], a_feat[x], rcond=None)[0]
         a_cols.append(a_feat / a_std)
         v_cols.append(v_feat * gain / a_std)
-        gains.append(gain)
-        stds.append(a_std)
     na = min(len(c) for c in a_cols)
     nv = min(len(c) for c in v_cols)
     audio_scaled = np.stack([c[:na] for c in a_cols], axis=1)
     video_scaled = np.stack([c[:nv] for c in v_cols], axis=1)
-    audio_scaled, video_scaled = np.ascontiguousarray(audio_scaled), np.ascontiguousarray(video_scaled)
-    if not return_gains:
-        return audio_scaled, video_scaled
-    f32 = all(np.asarray(f).dtype == np.float32 for f in list(video_features)[:3] + list(audio_features)[:3]) and \
-        all(np.asarray(g).dtype == np.float32 and np.asarray(g).shape == (1,) for g in gains) and \
-        all(np.asarray(sd).dtype == np.float32 for sd in stds) and audio_scaled.dtype == np.float32
-    if not f32:
-        return audio_scaled, video_scaled, None
-    return audio_scaled, video_scaled, (np.array([g[0] for g in gains], np.float32), np.array(stds, np.float32))
+    return np.ascontiguousarray(audio_scaled), np.ascontiguousarray(video_scaled)
 
 
 def feature_gains(video_features, audio_features, x, y):
     """The six scalars the scaled feature arrays are made from (describealign.py:733-741): per feature
     the least-squares gain and the audio standard deviation, plus the lengths of the stacked arrays.
     Returns (gains f32[3], audio_stds f32[3], n_audio, n_video); the arrays themselves are rebuilt on
-    the device (dab_pair_stage_b_gains / _clusters)."""
+    the device (dab_pair_stage_b_clusters, dab_engine_submit_b).  Raises TypeError unless the first three
+    features are float32: the device cannot redo numpy's arithmetic on other types from float32 scalars."""
     gains, stds = [], []
     for v_feat, a_feat in list(zip(video_features, audio_features))[:3]:
         if np.asarray(v_feat).dtype != np.float32 or np.asarray(a_feat).dtype != np.float32:

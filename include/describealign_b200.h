@@ -15,7 +15,7 @@
  *   get_freq_bands              :575-593             "
  *   align, device stage A       :596-700             dab_pair_stage_a + dab_pair_get_path1
  *   align, host stage           :702-893             stays in Python (describealign_b200/host_fit.py)
- *   align, device stage B       :895-993             dab_pair_stage_b + dab_pair_get_path2
+ *   align, device stage B       :895-993             dab_pair_stage_b_clusters + dab_pair_get_path2
  *
  * Conventions: plain pointers and sizes only; every function returns 0 on success or a
  * DAB_E_* code, with a message available from dab_last_error(); the caller owns every
@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define DAB_ABI_VERSION 1
+#define DAB_ABI_VERSION 2
 
 enum {
   DAB_OK = 0,
@@ -131,10 +131,9 @@ int dab_set_host_wait(int device, int mode);
 /* device < 0: current device. */
 int dab_create(int device, dab_ctx **out);
 void dab_destroy(dab_ctx *ctx);
-/* Testing switches.  "dp2_generic" = 1 or "dp2_impl" = 2 force the generic tree-based pass-2 DP (the
- * fallback for more than 32 corridors or non-positive slopes) instead of the scan DP ("dp2_impl" = 0, the
- * default); both are exact and the tests compare them.  "dp_reserve_kb" is accepted and ignored (it tuned
- * the one-warp DP kernel of an earlier version).  Unknown names return DAB_E_ARG. */
+/* Testing switch.  "dp2_impl" = 2 forces the generic tree-based pass-2 DP (the fallback for more than 32
+ * corridors or non-positive slopes) instead of the scan DP ("dp2_impl" = 0, the default); both are exact and
+ * the tests compare them.  Unknown names or values return DAB_E_ARG. */
 int dab_set_option(dab_ctx *ctx, const char *name, int64_t value);
 const char *dab_last_error(const dab_ctx *ctx);   /* ctx may be NULL for dab_create failures */
 
@@ -202,27 +201,24 @@ int dab_pair_import_points1(dab_pair *pair, const int32_t *i_audio, const int32_
 int dab_pair_dp1(dab_pair *pair, int64_t *n_path);
 
 /* ---- stage B (reference :895-993) -------------------------------------------------------
- * audio_scaled / video_scaled: float32 row-major (n, 3) arrays from the host stage (:740-741),
- * host pointers.  corridors: the scored clusters in cluster order with their final
- * (refined) lines.  n_clusters: number of line clusters (>= max cluster index + 1). */
+ * The explicit-input entry, used by tests to feed inputs no line cluster can produce.
+ * audio_scaled / video_scaled: float32 row-major (n, 3) arrays (:740-741), host pointers.
+ * corridors: the scored clusters in cluster order with their final (refined) lines.
+ * n_clusters: number of line clusters (>= max cluster index + 1).  np.max of the energy
+ * columns (:908-909) is taken on the device. */
 int dab_pair_stage_b(dab_pair *pair, const float *audio_scaled, int64_t n_audio,
                      const float *video_scaled, int64_t n_video, const dab_corridor *corridors,
                      int32_t n_corridors, int32_t n_clusters, int64_t *n_points, int64_t *n_path);
-/* The same stage for a pair that still holds its feature vectors on the device (after dab_pair_set_pcm
- * or dab_pair_set_features): the scaled arrays of describealign.py:737-741 are produced on the device
+/* The whole of stage B on the device for a pair that still holds its feature vectors there (after
+ * dab_pair_set_pcm or dab_pair_set_features), from the host fit's line clusters (in cluster order,
+ * ascending cluster index).  The scaled arrays of describealign.py:737-741 are produced on the device
  * from the least-squares gains and the audio standard deviations of the first three features (numpy
  * float32 roundings: audio / std ; video * gain / std), so only 6 floats travel instead of
  * 12 (n_audio + n_video) bytes.  n_audio / n_video: lengths of the scaled arrays (the shortest of the
- * three vectors of each track); *_energy_max: np.max of column 0 of each scaled array (:908-909). */
-int dab_pair_stage_b_gains(dab_pair *pair, const float gain[3], const float audio_std[3], int64_t n_audio,
-                           int64_t n_video, float audio_energy_max, float video_energy_max,
-                           const dab_corridor *corridors, int32_t n_corridors, int32_t n_clusters,
-                           int64_t *n_points, int64_t *n_path);
-/* The whole of stage B on the device, from the host fit's line clusters (in cluster order, ascending
- * cluster index): corridor planning incl. the offset refinement (:895-932), np.max of the scaled energy
- * columns (:908-909), scoring, DP #2, traceback.  The refinement's least-squares coefficient is the
- * quotient of float64 sums (the reference: np.linalg.lstsq), so refined offsets agree with the
- * reference's to ~1e-15 relative rather than bit for bit. */
+ * three vectors of each track).  Then corridor planning incl. the offset refinement (:895-932), np.max
+ * of the scaled energy columns (:908-909), scoring, DP #2, traceback.  The refinement's least-squares
+ * coefficient is the quotient of float64 sums (the reference: np.linalg.lstsq), so refined offsets
+ * agree with the reference's to ~1e-15 relative rather than bit for bit. */
 int dab_pair_stage_b_clusters(dab_pair *pair, const float gain[3], const float audio_std[3], int64_t n_audio,
                               int64_t n_video, const dab_cluster *clusters, int32_t n_clusters,
                               int64_t *n_points, int64_t *n_path);
@@ -309,14 +305,12 @@ typedef struct {
   float timings_ms[16];
 } dab_event;
 
-/* input of stage B, as dab_pair_stage_b_gains */
+/* input of stage B, as dab_pair_stage_b_clusters */
 typedef struct {
   float gain[3], audio_std[3];
-  float audio_energy_max, video_energy_max;
   int64_t n_audio, n_video;
-  const dab_corridor *corridors;   /* pre-planned corridors (copied by dab_engine_submit_b), or NULL: */
-  int32_t n_corridors, n_clusters;
-  const dab_cluster *clusters;     /* n_clusters line clusters, planned on the device (energy maxima ignored) */
+  int32_t n_clusters;
+  const dab_cluster *clusters;     /* n_clusters line clusters (copied by dab_engine_submit_b) */
 } dab_stage_b_in;
 
 int dab_engine_create(dab_ctx *ctx, int32_t slots, dab_engine **out);

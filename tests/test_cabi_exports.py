@@ -42,8 +42,9 @@ def test_binding_covers_header():
 
 def test_abi_version_and_struct_layout(lib):
     from describealign_b200 import _cabi
-    assert lib.dab_abi_version() == 1
+    assert lib.dab_abi_version() == 2
     assert ctypes.sizeof(_cabi.Corridor) == 32       # 4 x int32 + 2 x double
+    assert ctypes.sizeof(_cabi.StageBIn) == 56       # 6 x float, 2 x int64, int32 + padding, pointer
     assert ctypes.sizeof(_cabi.Stats) == 15 * 8
 
 
@@ -161,26 +162,26 @@ def test_host_wait_mode_is_validated(lib):
 
 
 def test_scaled_features_follow_from_six_scalars():
-    """host_fit.scale_features(return_gains=True): the scaled arrays are exactly audio / std and
-    video * gain / std in float32 - what dab_pair_stage_b_gains redoes on the device."""
+    """host_fit.scale_features against the six scalars of host_fit.feature_gains: the scaled arrays are
+    exactly audio / std and video * gain / std in float32 - what dab_pair_stage_b_clusters redoes on the device."""
     from describealign_b200 import host_fit
     rng = np.random.default_rng(5)
     n_v, n_a = 5000, 5600
     video = [rng.standard_normal(n_v + (k == 0)).astype(np.float32) for k in range(5)]
     audio = [rng.standard_normal(n_a + (k == 0)).astype(np.float32) for k in range(5)]
     y = np.sort(rng.integers(0, n_v, 900)); x = np.sort(rng.integers(0, n_a, 900))
-    a_s, v_s, gains = host_fit.scale_features(video, audio, x, y, return_gains=True)
-    a_ref, v_ref = host_fit.scale_features(video, audio, x, y)
-    np.testing.assert_array_equal(a_s, a_ref); np.testing.assert_array_equal(v_s, v_ref)
-    assert gains is not None and a_s.shape == (n_a, 3) and v_s.shape == (n_v, 3)
-    g, sd = gains
-    assert g.dtype == np.float32 and sd.dtype == np.float32
+    a_s, v_s = host_fit.scale_features(video, audio, x, y)
+    g, sd, na, nv = host_fit.feature_gains(video, audio, x, y)
+    assert a_s.shape == (n_a, 3) and v_s.shape == (n_v, 3) and (na, nv) == (n_a, n_v)
+    assert a_s.dtype == v_s.dtype == np.float32
+    assert g.dtype == np.float32 and sd.dtype == np.float32 and g.shape == sd.shape == (3,)
     for k in range(3):
         np.testing.assert_array_equal(a_s[:, k], (audio[k][:n_a] / sd[k]).astype(np.float32))
         np.testing.assert_array_equal(v_s[:, k], ((video[k][:n_v] * g[k]).astype(np.float32) / sd[k]).astype(np.float32))
     # float64 features: the device cannot redo numpy's arithmetic from float32 scalars
     video64 = [f.astype(np.float64) for f in video]
-    assert host_fit.scale_features(video64, audio, x, y, return_gains=True)[2] is None
+    with pytest.raises(TypeError):
+        host_fit.feature_gains(video64, audio, x, y)
 
 
 def test_worker_threads_use_the_process_device(monkeypatch):
