@@ -46,12 +46,15 @@ class Cluster(ctypes.Structure):
                 ("x_last", ctypes.c_double), ("offset", ctypes.c_double), ("slope", ctypes.c_double)]
 
 
-def cluster_array(lines):
-    """ctypes array of dab_cluster from [(cluster index, x_first, x_last, offset, slope), ...]"""
+def _stage_b_args(gains, audio_stds, lines):
+    """The stage-B input of a host fit as ctypes values: gain[3], audio_std[3] and the dab_cluster array
+    of the line clusters [(cluster index, x_first, x_last, offset, slope), ...]."""
+    g = (ctypes.c_float * 3)(*[float(x) for x in gains])
+    sd = (ctypes.c_float * 3)(*[float(x) for x in audio_stds])
     arr = (Cluster * max(len(lines), 1))()
     for k, (idx, xf, xl, offset, slope) in enumerate(lines):
         arr[k] = Cluster(int(idx), 0, float(xf), float(xl), float(offset), float(slope))
-    return arr
+    return g, sd, arr
 
 
 class Stats(ctypes.Structure):
@@ -180,6 +183,7 @@ def load() -> ctypes.CDLL:
     lib.dab_pair_get_points2.argtypes = [vp, vp, vp, vp, vp]
     lib.dab_pair_get_stats.argtypes = [vp, ctypes.POINTER(Stats)]
     lib.dab_pair_get_timings.argtypes = [vp, ctypes.POINTER(ctypes.c_float * 16)]
+    lib.dab_pair_get_timeline.argtypes = [vp, vp, ctypes.POINTER(ctypes.c_float * 9), ctypes.POINTER(ctypes.c_float * 9)]
     lib.dab_launch_count.argtypes = [vp]
     lib.dab_launch_count.restype = i64
     lib.dab_engine_create.argtypes = [vp, ctypes.c_int32, ctypes.POINTER(vp)]
@@ -468,9 +472,7 @@ class Pair:
     def stage_b_clusters(self, gains, audio_stds, n_audio: int, n_video: int, lines):
         """Stage B from the host fit's line clusters [(cluster index, x_first, x_last, offset, slope), ...]:
         scaling, corridor planning (describealign.py:895-932), scoring, DP 2 and traceback on the device."""
-        g = (ctypes.c_float * 3)(*[float(x) for x in gains])
-        sd = (ctypes.c_float * 3)(*[float(x) for x in audio_stds])
-        arr = cluster_array(lines)
+        g, sd, arr = _stage_b_args(gains, audio_stds, lines)
         npts, npath = ctypes.c_int64(), ctypes.c_int64()
         self.ctx.check(self.lib.dab_pair_stage_b_clusters(self.handle, ctypes.byref(g), ctypes.byref(sd), int(n_audio), int(n_video),
                                                           ctypes.cast(arr, ctypes.c_void_p), len(lines),
@@ -483,9 +485,7 @@ class Pair:
         """Plans the corridors and builds the whole pass-2 point list; quals only for audio rows
         [row_lo, row_hi).  Returns (n_points, first_point, n_mine): this rank's points are
         [first_point, first_point + n_mine)."""
-        g = (ctypes.c_float * 3)(*[float(x) for x in gains])
-        sd = (ctypes.c_float * 3)(*[float(x) for x in audio_stds])
-        arr = cluster_array(lines)
+        g, sd, arr = _stage_b_args(gains, audio_stds, lines)
         npts, first, mine = ctypes.c_int64(), ctypes.c_int64(), ctypes.c_int64()
         self.ctx.check(self.lib.dab_pair_stage_b_score(self.handle, ctypes.byref(g), ctypes.byref(sd), int(n_audio), int(n_video),
                                                        ctypes.cast(arr, ctypes.c_void_p), len(lines), int(row_lo), int(row_hi),
@@ -548,8 +548,6 @@ class Pair:
     def timeline(self, ref_event: int) -> dict:
         """(start, end) of the device stages in ms after `ref_event` (a cudaEvent_t handle)."""
         t0, t1 = (ctypes.c_float * 9)(), (ctypes.c_float * 9)()
-        self.lib.dab_pair_get_timeline.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(ctypes.c_float * 9),
-                                                   ctypes.POINTER(ctypes.c_float * 9)]
         self.ctx.check(self.lib.dab_pair_get_timeline(self.handle, ctypes.c_void_p(ref_event), ctypes.byref(t0), ctypes.byref(t1)))
         return {name: (float(t0[k]), float(t1[k])) for k, name in enumerate(TIMING_SLOTS[:9]) if t0[k] >= 0}
 
@@ -669,11 +667,8 @@ class Engine:
         """The dab_stage_b_in of a host fit (reusable: the engine copies the arrays on submit).
         lines: the fit's line clusters (host_fit.cluster_lines); the corridors are planned on the device."""
         b = StageBIn()
-        for k in range(3):
-            b.gain[k] = float(gains[k])
-            b.audio_std[k] = float(audio_stds[k])
+        b.gain, b.audio_std, arr = _stage_b_args(gains, audio_stds, lines)
         b.n_audio, b.n_video = int(n_audio), int(n_video)
-        arr = cluster_array(lines)
         b.clusters = ctypes.cast(arr, ctypes.c_void_p)
         b.n_clusters = len(lines)
         b._cluster_array = arr           # keeps the array alive as long as the struct

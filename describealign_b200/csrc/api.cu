@@ -406,19 +406,26 @@ int dab_pair_get_features(dab_pair *pr, int track, float *energy, float *zc, flo
   return DAB_OK;
 }
 
+// stage A enqueued, waited for and collected; run again while a buffer overflows
+static int stage_a_sync(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp) {
+  dab_ctx *ctx = pr->ctx;
+  int rc = DAB_E_CAPACITY;
+  for (int attempt = 0; attempt < DAB_STAGE_A_ATTEMPTS && rc == DAB_E_CAPACITY; ++attempt) {
+    DAB_TRY(dab_enqueue_stage_a(pr, row_lo, row_hi, with_dp));
+    DAB_CUDA(dab_wait_stream(pr->stream));
+    rc = dab_collect_stage_a(pr, with_dp);
+  }
+  return rc;
+}
+
 int dab_pair_stage_a(dab_pair *pr, int64_t *n_points, int64_t *n_path) {
   if (!pr) return DAB_E_ARG;
   dab_ctx *ctx = pr->ctx;
   StreamScope scope__(pr->stream);
   ApiTimer timer__(&pr->api_us[1]);
-  for (int t = 0; t < 2; ++t) {
-    if (!pr->trk[t].have_features) { dab_set_err(ctx, "stage_a: features of both tracks are required first"); return DAB_E_STATE; }
-    const int64_t lmin = pr->trk[t].Le < pr->trk[t].L ? pr->trk[t].Le : pr->trk[t].L;
-    if (lmin < 2 * DAB_WIN) { dab_set_err(ctx, "stage_a: track shorter than 82 frames"); return DAB_E_TOO_SHORT; }
-  }
+  DAB_TRY(dab_check_stage_a_inputs(pr, "stage_a"));
   DAB_CUDA(cudaSetDevice(ctx->device));
-  DAB_TRY(dab_run_stage_a(pr));
-  pr->matched = true;
+  DAB_TRY(stage_a_sync(pr, 0, INT64_MAX, true));
   if (n_points) *n_points = pr->n_points1;
   if (n_path) *n_path = pr->n_path1;
   return DAB_OK;
@@ -483,26 +490,15 @@ int dab_pair_export_points1(dab_pair *pr, int32_t *i_audio, int32_t *v_video, do
   return export_points1(pr, i_audio, v_video, qual, dst_on_device);
 }
 
-static int check_stage_a_inputs(dab_pair *pr, const char *who) {
-  dab_ctx *ctx = pr->ctx;
-  for (int t = 0; t < 2; ++t) {
-    if (!pr->trk[t].have_features) { dab_set_err(ctx, std::string(who) + ": features of both tracks are required first"); return DAB_E_STATE; }
-    const int64_t lmin = pr->trk[t].Le < pr->trk[t].L ? pr->trk[t].Le : pr->trk[t].L;
-    if (lmin < 2 * DAB_WIN) { dab_set_err(ctx, std::string(who) + ": track shorter than 82 frames"); return DAB_E_TOO_SHORT; }
-  }
-  return DAB_OK;
-}
-
 int dab_pair_stage_a_match(dab_pair *pr, int64_t row_lo, int64_t row_hi, int64_t *n_points) {
   if (!pr) return DAB_E_ARG;
   dab_ctx *ctx = pr->ctx;
   StreamScope scope__(pr->stream);
   ApiTimer timer__(&pr->api_us[1]);
   if (row_lo < 0 || row_hi < row_lo) { dab_set_err(ctx, "dab_pair_stage_a_match: invalid row range"); return DAB_E_ARG; }
-  DAB_TRY(check_stage_a_inputs(pr, "stage_a_match"));
+  DAB_TRY(dab_check_stage_a_inputs(pr, "stage_a_match"));
   DAB_CUDA(cudaSetDevice(ctx->device));
-  DAB_TRY(dab_run_stage_a_match(pr, row_lo, row_hi));
-  pr->matched = true;
+  DAB_TRY(stage_a_sync(pr, row_lo, row_hi, false));
   if (n_points) *n_points = pr->n_points1;
   return DAB_OK;
 }
@@ -525,17 +521,19 @@ int dab_pair_dp1(dab_pair *pr, int64_t *n_path) {
   ApiTimer timer__(&pr->api_us[1]);
   if (!pr->matched) { dab_set_err(ctx, "dp1: no match points (run stage_a_match / import_points1 first)"); return DAB_E_STATE; }
   DAB_CUDA(cudaSetDevice(ctx->device));
-  DAB_TRY(dab_run_stage_a_dp(pr));
+  DAB_TRY(dab_enqueue_stage_a_dp(pr));
+  DAB_TRY(dab_enqueue_counts(pr));
+  DAB_CUDA(dab_wait_stream(pr->stream));
+  dab_collect_stage_a_dp(pr);
   if (n_path) *n_path = pr->n_path1;
   return DAB_OK;
 }
 
-// the end of every synchronous stage-B entry: counts to the host, wait, collect
-static int finish_stage_b(dab_pair *pr, int64_t *n_points, int64_t *n_path) {
+// the end of every synchronous stage-B entry: wait for the enqueued stage and its counts, collect
+static int finish_stage_b(dab_pair *pr, bool with_dp, int64_t *n_points, int64_t *n_path) {
   dab_ctx *ctx = pr->ctx;
-  DAB_TRY(dab_enqueue_counts(pr));
   DAB_CUDA(dab_wait_stream(pr->stream));
-  DAB_TRY(dab_collect_stage_b(pr));
+  DAB_TRY(dab_collect_stage_b(pr, with_dp));
   if (n_points) *n_points = pr->n_points2;
   if (n_path) *n_path = pr->n_path2;
   return DAB_OK;
@@ -577,75 +575,13 @@ int dab_pair_stage_b(dab_pair *pr, const float *audio_scaled, int64_t n_audio, c
   DAB_CUDA(cudaMemcpyAsync(pr->a_scaled.p, audio_scaled, sizeof(float) * 3 * (size_t)n_audio, cudaMemcpyHostToDevice, st));
   DAB_CUDA(cudaMemcpyAsync(pr->v_scaled.p, video_scaled, sizeof(float) * 3 * (size_t)n_video, cudaMemcpyHostToDevice, st));
   DAB_TRY(dab_enqueue_column_maxes(pr, n_audio, n_video));
-  pr->b_device_planned = false;
-  pr->h_cor.assign(corridors, corridors + n_corridors);
   DAB_TRY(dab_ensure(ctx, pr->corridors, sizeof(dab_corridor) * (size_t)(n_corridors + 1)));
   if (n_corridors > 0)
     DAB_CUDA(cudaMemcpyAsync(pr->corridors.p, corridors, sizeof(dab_corridor) * (size_t)n_corridors, cudaMemcpyHostToDevice, st));
-  pr->stats.n_audio_frames = n_audio;
-  pr->stats.n_video_frames = n_video;
-  DAB_TRY(dab_enqueue_stage_b(pr, n_corridors, n_clusters));
-  return finish_stage_b(pr, n_points, n_path);   // (the caller's arrays have been consumed once it returns)
+  dab_set_stage_b_plan(pr, n_audio, n_video, std::vector<dab_corridor>(corridors, corridors + n_corridors), n_clusters, false);
+  DAB_TRY(dab_enqueue_stage_b(pr, 0, INT64_MAX, true));
+  return finish_stage_b(pr, true, n_points, n_path);   // (the caller's arrays have been consumed once it returns)
 }
-
-}  // extern "C"
-
-// describealign.py:737-741 on the device: audio_scaled = audio / std(audio), video_scaled =
-// video * gain / std(audio), float32 with numpy's roundings (one division; one multiply then one
-// division), stacked as (n, 3).  The feature vectors are the pair's own device copies.
-__global__ void scale_features_kernel(const float *f0, const float *f1, const float *f2, int64_t n, float g0, float g1,
-                                      float g2, float s0, float s1, float s2, int with_gain, float *out) {
-  const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (k >= n) return;
-  float x0 = f0[k], x1 = f1[k], x2 = f2[k];
-  if (with_gain) { x0 = __fmul_rn(x0, g0); x1 = __fmul_rn(x1, g1); x2 = __fmul_rn(x2, g2); }
-  out[3 * k + 0] = __fdiv_rn(x0, s0);
-  out[3 * k + 1] = __fdiv_rn(x1, s1);
-  out[3 * k + 2] = __fdiv_rn(x2, s2);
-}
-
-static int enqueue_scaling(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video);
-
-// stage B from line clusters: scaling, corridor planning on the device, then the stage itself
-int dab_enqueue_stage_b_clusters(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video,
-                                 const dab_cluster *clusters, int32_t n_clusters) {
-  dab_ctx *ctx = pr->ctx;
-  if (n_clusters < 0 || (n_clusters > 0 && !clusters)) {
-    dab_set_err(ctx, "dab_pair_stage_b_clusters: invalid argument");
-    return DAB_E_ARG;
-  }
-  DAB_TRY(enqueue_scaling(pr, gain, audio_std, n_audio, n_video));
-  DAB_TRY(dab_enqueue_plan_corridors(pr, clusters, n_clusters, n_audio, n_video));
-  pr->stats.n_audio_frames = n_audio;
-  pr->stats.n_video_frames = n_video;
-  return dab_enqueue_stage_b(pr, n_clusters, n_clusters > 0 ? clusters[n_clusters - 1].cluster + 1 : 0);
-}
-
-static int enqueue_scaling(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video) {
-  dab_ctx *ctx = pr->ctx;
-  if (!gain || !audio_std || n_audio <= 0 || n_video <= 8) {
-    dab_set_err(ctx, "stage B: invalid argument");
-    return DAB_E_ARG;
-  }
-  Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
-  if (!V.have_features || !A.have_features) { dab_set_err(ctx, "stage B: the pair holds no features"); return DAB_E_STATE; }
-  // np.stack truncates to the shortest of the three vectors (energy may be one longer)
-  const int64_t na = A.L < A.Le ? A.L : A.Le, nv = V.L < V.Le ? V.L : V.Le;
-  if (n_audio != na || n_video != nv) { dab_set_err(ctx, "stage B: lengths differ from the pair's features"); return DAB_E_ARG; }
-  DAB_CUDA(cudaSetDevice(ctx->device));
-  cudaStream_t st = pr->stream;
-  DAB_TRY(dab_ensure(ctx, pr->a_scaled, sizeof(float) * 3 * (size_t)n_audio));
-  DAB_TRY(dab_ensure(ctx, pr->v_scaled, sizeof(float) * 3 * (size_t)n_video));
-  scale_features_kernel<<<(unsigned)cdiv(n_audio, 256), 256, 0, st>>>(A.energy.as<float>(), A.zc.as<float>(), A.b0.as<float>(),
-      n_audio, 1.f, 1.f, 1.f, audio_std[0], audio_std[1], audio_std[2], 0, pr->a_scaled.as<float>());
-  scale_features_kernel<<<(unsigned)cdiv(n_video, 256), 256, 0, st>>>(V.energy.as<float>(), V.zc.as<float>(), V.b0.as<float>(),
-      n_video, gain[0], gain[1], gain[2], audio_std[0], audio_std[1], audio_std[2], 1, pr->v_scaled.as<float>());
-  ctx->launches += 2;
-  DAB_CUDA(cudaGetLastError());
-  return DAB_OK;
-}
-
-extern "C" {
 
 int dab_pair_stage_b_clusters(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio,
                               int64_t n_video, const dab_cluster *clusters, int32_t n_clusters,
@@ -653,8 +589,9 @@ int dab_pair_stage_b_clusters(dab_pair *pr, const float gain[3], const float aud
   if (!pr) return DAB_E_ARG;
   StreamScope scope__(pr->stream);
   ApiTimer timer__(&pr->api_us[2]);
-  DAB_TRY(dab_enqueue_stage_b_clusters(pr, gain, audio_std, n_audio, n_video, clusters, n_clusters));
-  return finish_stage_b(pr, n_points, n_path);
+  DAB_TRY(dab_enqueue_stage_b_clusters(pr, gain, audio_std, n_audio, n_video, clusters, n_clusters, 0, INT64_MAX, true,
+                                       "dab_pair_stage_b_clusters"));
+  return finish_stage_b(pr, true, n_points, n_path);
 }
 
 // ---- stage B in steps, for one very long pair split over several GPUs (SURVEY.md 8e) ----
@@ -662,26 +599,11 @@ int dab_pair_stage_b_score(dab_pair *pr, const float gain[3], const float audio_
                            const dab_cluster *clusters, int32_t n_clusters, int64_t row_lo, int64_t row_hi,
                            int64_t *n_points, int64_t *first_point, int64_t *n_mine) {
   if (!pr) return DAB_E_ARG;
-  dab_ctx *ctx = pr->ctx;
   StreamScope scope__(pr->stream);
   ApiTimer timer__(&pr->api_us[2]);
-  if (n_clusters < 0 || (n_clusters > 0 && !clusters) || row_lo < 0 || row_hi < row_lo) {
-    dab_set_err(ctx, "dab_pair_stage_b_score: invalid argument");
-    return DAB_E_ARG;
-  }
-  DAB_TRY(enqueue_scaling(pr, gain, audio_std, n_audio, n_video));
-  DAB_TRY(dab_enqueue_plan_corridors(pr, clusters, n_clusters, n_audio, n_video));
-  pr->stats.n_audio_frames = n_audio;
-  pr->stats.n_video_frames = n_video;
-  pr->b_n_cor = n_clusters;
-  pr->b_n_clusters = n_clusters > 0 ? clusters[n_clusters - 1].cluster + 1 : 0;
-  DAB_TRY(dab_enqueue_stage_b_points(pr, pr->b_n_cor, pr->b_n_clusters, row_lo, row_hi));
-  DAB_TRY(dab_enqueue_counts(pr));
-  DAB_CUDA(dab_wait_stream(pr->stream));
-  const int32_t *hc = reinterpret_cast<const int32_t *>(pr->h_counters);
-  if (hc[DC_OVERFLOW_B] & DAB_OVF_ROWCOR) { dab_set_err(ctx, "more than 32 corridors overlap one audio row"); return DAB_E_CAPACITY; }
-  pr->n_points2 = hc[DC_N_PTS2];
-  pr->stats.n_points2 = pr->n_points2;
+  DAB_TRY(dab_enqueue_stage_b_clusters(pr, gain, audio_std, n_audio, n_video, clusters, n_clusters, row_lo, row_hi, false,
+                                       "dab_pair_stage_b_score"));
+  DAB_TRY(finish_stage_b(pr, false, nullptr, nullptr));
   int64_t first = 0, count = 0;
   DAB_TRY(dab_row_range_points2(pr, row_lo, row_hi, &first, &count));
   if (n_points) *n_points = pr->n_points2;
@@ -732,14 +654,15 @@ int dab_pair_dp2(dab_pair *pr, int64_t *n_path) {
   StreamScope scope__(pr->stream);
   ApiTimer timer__(&pr->api_us[2]);
   DAB_CUDA(cudaSetDevice(ctx->device));
-  DAB_TRY(dab_enqueue_stage_b_dp(pr, pr->b_n_cor, pr->b_n_clusters));
-  return finish_stage_b(pr, nullptr, n_path);
+  DAB_TRY(dab_enqueue_stage_b_dp(pr));
+  DAB_TRY(dab_enqueue_counts(pr));
+  return finish_stage_b(pr, true, nullptr, n_path);
 }
 
 int dab_pair_get_corridors(dab_pair *pr, dab_corridor *out, int32_t cap, int32_t *n_corridors) {
   if (!pr || !n_corridors) return DAB_E_ARG;
   dab_ctx *ctx = pr->ctx;
-  const int32_t n = (int32_t)pr->h_cor.size();
+  const int32_t n = (int32_t)pr->plan_b.cor.size();
   *n_corridors = n;
   if (!out || cap <= 0 || n == 0) return DAB_OK;
   const int32_t m = n < cap ? n : cap;

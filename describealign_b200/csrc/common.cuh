@@ -55,6 +55,18 @@ struct Track {
   int64_t n_list = 0;
 };
 
+// What one stage-B call decided, read by every later step of that call (points, DP 2, the exchange of
+// quals of a row-sharded pair).  Set once per call by dab_set_stage_b_plan.
+struct StageBPlan {
+  int64_t n_audio = 0, n_video = 0;
+  std::vector<dab_corridor> cor;   // host row bounds; device-planned: ranges that contain the planned ones
+  int32_t n_clusters = 0;          // cluster indices are below this
+  bool device_planned = false;     // corridors planned on the device from clusters, not uploaded
+  int64_t pm_off[32] = {};         // first PM row of each corridor (scan DP)
+  int64_t rows = 0;                // total corridor rows: bounds the pass-2 points
+  bool scan_dp = false;            // the corridor-state DP runs, not the generic tree DP
+};
+
 struct dab_pair {
   dab_ctx *ctx = nullptr;
   cudaStream_t stream = nullptr;
@@ -95,7 +107,7 @@ struct dab_pair {
   DevBuf p2_i, p2_c, p2_rank, p2_k;  // i32
   DevBuf pm2, pmoff2;          // corridor-state DP: per-corridor running maxima, row offsets
   DevBuf lift_up, lift_dep;    // pointer-jumping traceback
-  std::vector<dab_corridor> h_cor;   // host copy of the corridors of the current stage_b call
+  StageBPlan plan_b;
   DevBuf p2_j, p2_q;           // f64
   DevBuf tree2;                // frontier tree of pass 2
   DevBuf cache2;               // prev_cache rows
@@ -103,9 +115,6 @@ struct dab_pair {
   DevBuf len2, cp2, backid2;   // i32
   DevBuf path2;                // f64 (n,5)
   int64_t n_points2 = 0, n_path2 = 0;
-  int64_t cap_points2 = 0;     // upper bound of pass-2 points of the current stage_b call (sum of corridor rows)
-  int32_t b_n_cor = 0, b_n_clusters = 0;   // of the stage-B call in progress (dab_pair_stage_b_score .. dab_pair_dp2)
-  bool b_device_planned = false;      // corridors were planned on the device (dab_enqueue_plan_corridors), not uploaded
   DevBuf clusters, refine_partial, maxes;
   dab_stats stats = {};
   cudaEvent_t ev[32] = {};
@@ -200,25 +209,36 @@ enum { DAB_OVF_ENTRIES = 1, DAB_OVF_CAND = 2, DAB_OVF_ROWCOR = 4, DAB_OVF_PTS2 =
 
 // stage entry points implemented in the .cu files
 int dab_run_features(dab_pair *pr, int track, const void *d_pcm, int format);
-int dab_run_stage_a(dab_pair *pr);
-int dab_run_stage_a_match(dab_pair *pr, int64_t row_lo, int64_t row_hi);   // prep .. match points of audio rows [lo, hi)
-int dab_run_stage_a_dp(dab_pair *pr);                                       // DP #1 + traceback over the pair's points
-// the same stages, enqueued on the pair's stream without waiting (counts stay on the device); the counts
-// block is copied to the mapped host page by dab_enqueue_counts and interpreted by dab_collect_*
-int dab_enqueue_stage_a_match(dab_pair *pr, int64_t row_lo, int64_t row_hi);
-int dab_enqueue_stage_a_dp(dab_pair *pr);
+// A device stage is enqueued on the pair's stream without waiting (counts stay on the device) and ends with
+// dab_enqueue_counts, which copies the counts block to the mapped host page; once the stream has passed that
+// point, dab_collect_* interprets it.
 int dab_enqueue_counts(dab_pair *pr);
+// Stage A.  On a capacity overflow dab_collect_stage_a grows the buffer and returns DAB_E_CAPACITY: the caller
+// enqueues the stage again, up to DAB_STAGE_A_ATTEMPTS runs in all.
+constexpr int DAB_STAGE_A_ATTEMPTS = 8;
+int dab_check_stage_a_inputs(dab_pair *pr, const char *who);
+// match points of audio rows [row_lo, row_hi), then DP 1 + traceback if with_dp, then the counts
+int dab_enqueue_stage_a(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp);
+int dab_enqueue_stage_a_dp(dab_pair *pr);      // DP 1 + traceback over the pair's points
 int dab_collect_stage_a(dab_pair *pr, bool with_dp);
-int dab_enqueue_stage_b(dab_pair *pr, int32_t n_corridors, int32_t n_clusters);
-int dab_enqueue_stage_b_points(dab_pair *pr, int32_t n_corridors, int32_t n_clusters, int64_t q_lo, int64_t q_hi);
-int dab_enqueue_stage_b_dp(dab_pair *pr, int32_t n_corridors, int32_t n_clusters);
-int dab_enqueue_set_quals2(dab_pair *pr, const double *d_q_all);
-int dab_row_range_points2(dab_pair *pr, int64_t lo, int64_t hi, int64_t *first, int64_t *count);
-int dab_enqueue_column_maxes(dab_pair *pr, int64_t n_audio, int64_t n_video);
-int dab_enqueue_plan_corridors(dab_pair *pr, const dab_cluster *clusters, int32_t n_clusters, int64_t n_audio, int64_t n_video);
-int dab_collect_stage_b(dab_pair *pr);
+void dab_collect_stage_a_dp(dab_pair *pr);
 int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *v_video, const double *qual,
                            int64_t n, int src_on_device);
+// Stage B.  Its sizes come from pr->plan_b, set by device planning from clusters or by the explicit upload of
+// dab_pair_stage_b.
+void dab_set_stage_b_plan(dab_pair *pr, int64_t n_audio, int64_t n_video, std::vector<dab_corridor> cor, int32_t n_clusters,
+                          bool device_planned);
+int dab_enqueue_column_maxes(dab_pair *pr, int64_t n_audio, int64_t n_video);
+// checks, scaling, corridor planning, then dab_enqueue_stage_b (`who` names the caller in argument errors)
+int dab_enqueue_stage_b_clusters(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video,
+                                 const dab_cluster *clusters, int32_t n_clusters, int64_t row_lo, int64_t row_hi, bool with_dp,
+                                 const char *who);
+// points with quals for audio rows [row_lo, row_hi), then DP 2 + traceback if with_dp, then the counts
+int dab_enqueue_stage_b(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp);
+int dab_enqueue_stage_b_dp(dab_pair *pr);
+int dab_enqueue_set_quals2(dab_pair *pr, const double *d_q_all);
+int dab_row_range_points2(dab_pair *pr, int64_t lo, int64_t hi, int64_t *first, int64_t *count);
+int dab_collect_stage_b(dab_pair *pr, bool with_dp);
 
 #define DAB_LAUNCHED(pr) ((pr)->ctx->launches++)
 

@@ -113,19 +113,9 @@ void enqueue_a(dab_engine *e, int slot, bool upload) {
       ENG_TRY(dab_pair_set_pcm(pr, t, s.job.pcm[t], s.job.samples[t], s.job.channels[t], s.job.format, s.job.on_device),
               DAB_EVENT_STAGE_A);
   }
-  for (int t = 0; t < 2; ++t) {
-    const int64_t lmin = pr->trk[t].Le < pr->trk[t].L ? pr->trk[t].Le : pr->trk[t].L;
-    if (lmin < 2 * DAB_WIN) {
-      dab_set_err(e->ctx, "stage_a: track shorter than 82 frames");
-      fail_slot(e, s, slot, DAB_E_TOO_SHORT, DAB_EVENT_STAGE_A);
-      return;
-    }
-  }
-  ENG_TRY(dab_enqueue_stage_a_match(pr, 0, INT64_MAX), DAB_EVENT_STAGE_A);
-  ENG_TRY(dab_enqueue_stage_a_dp(pr), DAB_EVENT_STAGE_A);
-  ENG_TRY(dab_enqueue_counts(pr), DAB_EVENT_STAGE_A);
+  ENG_TRY(dab_check_stage_a_inputs(pr, "stage_a"), DAB_EVENT_STAGE_A);
+  ENG_TRY(dab_enqueue_stage_a(pr, 0, INT64_MAX, true), DAB_EVENT_STAGE_A);
   ENG_CUDA(cudaEventRecord(s.ev, pr->stream), DAB_EVENT_STAGE_A);
-  pr->matched = true;
   s.state = S_A_RUN;
   s.host_us += now_us() - t0;
 }
@@ -138,7 +128,7 @@ void after_a(dab_engine *e, int slot) {
   StreamScope scope__(pr->stream);
   const int64_t t0 = now_us();
   const int rc = dab_collect_stage_a(pr, true);
-  if (rc == DAB_E_CAPACITY && ++s.attempts < 8) { enqueue_a(e, slot, false); return; }
+  if (rc == DAB_E_CAPACITY && ++s.attempts < DAB_STAGE_A_ATTEMPTS) { enqueue_a(e, slot, false); return; }
   ENG_TRY(rc, DAB_EVENT_STAGE_A);
   cudaStream_t st = pr->stream;
   const size_t pb = sizeof(int32_t) * (size_t)pr->n_path1;
@@ -187,23 +177,14 @@ void publish_a(dab_engine *e, int slot) {
   e->cv_out.notify_all();
 }
 
-}  // namespace
-
-// in api.cu
-int dab_enqueue_stage_b_clusters(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video,
-                                 const dab_cluster *clusters, int32_t n_clusters);
-
-namespace {
-
 void enqueue_b(dab_engine *e, int slot) {
   Slot &s = e->slots[slot];
   dab_pair *pr = s.pair;
   StreamScope scope__(pr->stream);
   const int64_t t0 = now_us();
   const dab_stage_b_in &b = s.b_in;
-  ENG_TRY(dab_enqueue_stage_b_clusters(pr, b.gain, b.audio_std, b.n_audio, b.n_video,
-                                       reinterpret_cast<const dab_cluster *>(s.cor.p), b.n_clusters), DAB_EVENT_STAGE_B);
-  ENG_TRY(dab_enqueue_counts(pr), DAB_EVENT_STAGE_B);
+  ENG_TRY(dab_enqueue_stage_b_clusters(pr, b.gain, b.audio_std, b.n_audio, b.n_video, reinterpret_cast<const dab_cluster *>(s.cor.p),
+                                       b.n_clusters, 0, INT64_MAX, true, "dab_pair_stage_b_clusters"), DAB_EVENT_STAGE_B);
   ENG_CUDA(cudaEventRecord(s.ev, pr->stream), DAB_EVENT_STAGE_B);
   s.state = S_B_RUN;
   s.host_us += now_us() - t0;
@@ -213,7 +194,7 @@ void after_b(dab_engine *e, int slot) {
   Slot &s = e->slots[slot];
   dab_pair *pr = s.pair;
   const int64_t t0 = now_us();
-  ENG_TRY(dab_collect_stage_b(pr), DAB_EVENT_STAGE_B);
+  ENG_TRY(dab_collect_stage_b(pr, true), DAB_EVENT_STAGE_B);
   const size_t rb = sizeof(double) * 5 * (size_t)pr->n_path2;
   if (s.rows.ensure(rb + 8)) { dab_set_err(e->ctx, "out of page-locked memory"); fail_slot(e, s, slot, DAB_E_CUDA, DAB_EVENT_STAGE_B); return; }
   if (rb) ENG_CUDA(cudaMemcpyAsync(s.rows.p, pr->path2.p, rb, cudaMemcpyDeviceToHost, pr->stream), DAB_EVENT_STAGE_B);

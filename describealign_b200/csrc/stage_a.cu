@@ -1138,7 +1138,7 @@ static void default_caps(dab_pair *pr) {
 }
 
 // ---- match stage, enqueued without a host round trip: prep, codes, lists, tables, gate, scoring ----
-int dab_enqueue_stage_a_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
+static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
   dab_ctx *ctx = pr->ctx;
   DAB_TRY(ensure_hann(ctx));
   Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
@@ -1295,13 +1295,33 @@ int dab_enqueue_stage_a_dp(dab_pair *pr) {
   return DAB_OK;
 }
 
-// The counts of the stage, copied to the pair's mapped host page by the stream (dab_enqueue_counts) and
-// read here once the stream has passed that point.  Returns DAB_E_CAPACITY after growing the capacity
-// that overflowed: the caller runs the stage again.
+int dab_enqueue_stage_a(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp) {
+  DAB_TRY(enqueue_match(pr, row_lo, row_hi));
+  if (with_dp) DAB_TRY(dab_enqueue_stage_a_dp(pr));
+  return dab_enqueue_counts(pr);
+}
+
 int dab_enqueue_counts(dab_pair *pr) {
   dab_ctx *ctx = pr->ctx;
   DAB_CUDA(dab_readback(pr, pr->h_counters, pr->counters.as<int32_t>(), sizeof(int32_t) * DC_WORDS));
   return DAB_OK;
+}
+
+int dab_check_stage_a_inputs(dab_pair *pr, const char *who) {
+  dab_ctx *ctx = pr->ctx;
+  for (int t = 0; t < 2; ++t) {
+    if (!pr->trk[t].have_features) { dab_set_err(ctx, std::string(who) + ": features of both tracks are required first"); return DAB_E_STATE; }
+    const int64_t lmin = pr->trk[t].Le < pr->trk[t].L ? pr->trk[t].Le : pr->trk[t].L;
+    if (lmin < 2 * DAB_WIN) { dab_set_err(ctx, std::string(who) + ": track shorter than 82 frames"); return DAB_E_TOO_SHORT; }
+  }
+  return DAB_OK;
+}
+
+// dp1_kernel ends with DC_DP1_END = -1 when there is no path (also when there are no points)
+void dab_collect_stage_a_dp(dab_pair *pr) {
+  const int32_t *hc = reinterpret_cast<const int32_t *>(pr->h_counters);
+  pr->n_path1 = hc[DC_DP1_END] < 0 ? 0 : hc[DC_N_PATH1];
+  pr->stats.n_path1 = pr->n_path1;
 }
 
 int dab_collect_stage_a(dab_pair *pr, bool with_dp) {
@@ -1324,48 +1344,9 @@ int dab_collect_stage_a(dab_pair *pr, bool with_dp) {
   }
   pr->n_points1 = hc[DC_N_PTS1];
   pr->stats.n_points1 = pr->n_points1;
-  if (with_dp) {
-    pr->n_path1 = hc[DC_DP1_END] < 0 ? 0 : hc[DC_N_PATH1];
-    pr->stats.n_path1 = pr->n_path1;
-  }
+  if (with_dp) dab_collect_stage_a_dp(pr);
+  pr->matched = true;
   return DAB_OK;
-}
-
-int dab_run_stage_a_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
-  dab_ctx *ctx = pr->ctx;
-  for (int attempt = 0; attempt < 8; ++attempt) {
-    DAB_TRY(dab_enqueue_stage_a_match(pr, row_lo, row_hi));
-    DAB_TRY(dab_enqueue_counts(pr));
-    DAB_CUDA(dab_wait_stream(pr->stream));
-    const int rc = dab_collect_stage_a(pr, false);
-    if (rc != DAB_E_CAPACITY) return rc;
-  }
-  return DAB_E_CAPACITY;
-}
-
-int dab_run_stage_a_dp(dab_pair *pr) {
-  dab_ctx *ctx = pr->ctx;
-  if (pr->cap_points1 < pr->n_points1) pr->cap_points1 = pr->n_points1;
-  DAB_TRY(dab_enqueue_stage_a_dp(pr));
-  DAB_TRY(dab_enqueue_counts(pr));
-  DAB_CUDA(dab_wait_stream(pr->stream));
-  const int32_t *hc = reinterpret_cast<const int32_t *>(pr->h_counters);
-  pr->n_path1 = (pr->n_points1 <= 0 || hc[DC_DP1_END] < 0) ? 0 : hc[DC_N_PATH1];
-  pr->stats.n_path1 = pr->n_path1;
-  return DAB_OK;
-}
-
-int dab_run_stage_a(dab_pair *pr) {
-  dab_ctx *ctx = pr->ctx;
-  for (int attempt = 0; attempt < 8; ++attempt) {
-    DAB_TRY(dab_enqueue_stage_a_match(pr, 0, INT64_MAX));
-    DAB_TRY(dab_enqueue_stage_a_dp(pr));
-    DAB_TRY(dab_enqueue_counts(pr));
-    DAB_CUDA(dab_wait_stream(pr->stream));
-    const int rc = dab_collect_stage_a(pr, true);
-    if (rc != DAB_E_CAPACITY) return rc;
-  }
-  return DAB_E_CAPACITY;
 }
 
 // ---- row-sharded match stage: exchange of match points -----------------------------------
@@ -1432,5 +1413,6 @@ int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *
   pr->n_points1 = n;
   pr->stats.n_points1 = n;
   pr->n_path1 = 0;
+  if (pr->cap_points1 < n) pr->cap_points1 = n;   // DP 1 sizes its buffers from it
   return DAB_OK;
 }

@@ -441,16 +441,71 @@ struct Dp2LArgs {
 
 // The corridor-state DP needs: at most 32 corridors, positive slopes, every coordinate >= 3 (so the
 // seeded prev_cache cell 0 is never in reach; x_limits keeps lines >= 4, describealign.py:898).
-static bool corridor_dp_eligible(const dab_pair *pr, int32_t n_cor) {
-  if (pr->ctx->opt_dp2_impl == 2 || n_cor > 32) return false;   // dp2_impl 2: the tree DP (cross-checks)
-  for (int k = 0; k < n_cor; ++k) {
-    const dab_corridor &c = pr->h_cor[k];
+static bool corridor_dp_eligible(const StageBPlan &b, int dp2_impl) {
+  if (dp2_impl == 2 || b.cor.size() > 32) return false;   // dp2_impl 2: the tree DP (cross-checks)
+  for (const dab_corridor &c : b.cor) {
     if (!(c.slope > 0.0)) return false;
-    // (device-planned corridors: h_cor holds row ranges that contain the planned ones; the planned lines
+    // (device-planned corridors: the host holds row ranges that contain the planned ones; the planned lines
     // start at coordinate >= 4 by construction, describealign.py:898)
-    if (!pr->b_device_planned && c.hi > c.lo && !(c.slope * (double)c.lo + c.offset >= 3.0)) return false;
+    if (!b.device_planned && c.hi > c.lo && !(c.slope * (double)c.lo + c.offset >= 3.0)) return false;
   }
   return true;
+}
+
+void dab_set_stage_b_plan(dab_pair *pr, int64_t n_audio, int64_t n_video, std::vector<dab_corridor> cor, int32_t n_clusters,
+                          bool device_planned) {
+  StageBPlan b;
+  b.n_audio = n_audio;
+  b.n_video = n_video;
+  b.cor = std::move(cor);
+  b.n_clusters = n_clusters;
+  b.device_planned = device_planned;
+  for (size_t k = 0; k < b.cor.size(); ++k) {
+    if (k < 32) b.pm_off[k] = b.rows;
+    b.rows += b.cor[k].hi > b.cor[k].lo ? b.cor[k].hi - b.cor[k].lo : 0;
+  }
+  b.scan_dp = corridor_dp_eligible(b, pr->ctx->opt_dp2_impl);
+  pr->plan_b = std::move(b);
+  pr->stats.n_audio_frames = n_audio;
+  pr->stats.n_video_frames = n_video;
+}
+
+// describealign.py:737-741 on the device: audio_scaled = audio / std(audio), video_scaled =
+// video * gain / std(audio), float32 with numpy's roundings (one division; one multiply then one
+// division), stacked as (n, 3).  The feature vectors are the pair's own device copies.
+__global__ void scale_features_kernel(const float *f0, const float *f1, const float *f2, int64_t n, float g0, float g1,
+                                      float g2, float s0, float s1, float s2, int with_gain, float *out) {
+  const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  float x0 = f0[k], x1 = f1[k], x2 = f2[k];
+  if (with_gain) { x0 = __fmul_rn(x0, g0); x1 = __fmul_rn(x1, g1); x2 = __fmul_rn(x2, g2); }
+  out[3 * k + 0] = __fdiv_rn(x0, s0);
+  out[3 * k + 1] = __fdiv_rn(x1, s1);
+  out[3 * k + 2] = __fdiv_rn(x2, s2);
+}
+
+static int enqueue_scaling(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video) {
+  dab_ctx *ctx = pr->ctx;
+  if (!gain || !audio_std || n_audio <= 0 || n_video <= 8) {
+    dab_set_err(ctx, "stage B: invalid argument");
+    return DAB_E_ARG;
+  }
+  Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
+  if (!V.have_features || !A.have_features) { dab_set_err(ctx, "stage B: the pair holds no features"); return DAB_E_STATE; }
+  // np.stack truncates to the shortest of the three vectors (energy may be one longer)
+  const int64_t na = A.L < A.Le ? A.L : A.Le, nv = V.L < V.Le ? V.L : V.Le;
+  if (n_audio != na || n_video != nv) { dab_set_err(ctx, "stage B: lengths differ from the pair's features"); return DAB_E_ARG; }
+  DAB_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = pr->stream;
+  DAB_TRY(dab_ensure(ctx, pr->a_scaled, sizeof(float) * 3 * (size_t)n_audio));
+  DAB_TRY(dab_ensure(ctx, pr->v_scaled, sizeof(float) * 3 * (size_t)n_video));
+  scale_features_kernel<<<(unsigned)cdiv(n_audio, 256), 256, 0, st>>>(A.energy.as<float>(), A.zc.as<float>(), A.b0.as<float>(),
+      n_audio, 1.f, 1.f, 1.f, audio_std[0], audio_std[1], audio_std[2], 0, pr->a_scaled.as<float>());
+  scale_features_kernel<<<(unsigned)cdiv(n_video, 256), 256, 0, st>>>(V.energy.as<float>(), V.zc.as<float>(), V.b0.as<float>(),
+      n_video, gain[0], gain[1], gain[2], audio_std[0], audio_std[1], audio_std[2], 1, pr->v_scaled.as<float>());
+  ctx->launches += 2;
+  DAB_CUDA(cudaGetLastError());
+  return DAB_OK;
 }
 
 // describealign.py:895-900 on the host, for buffer sizes only (the device computes the ranges it scores)
@@ -482,12 +537,12 @@ int dab_enqueue_column_maxes(dab_pair *pr, int64_t n_a, int64_t n_v) {
 }
 
 // Corridor planning on the device (refine.cuh).  `clusters` is read by an asynchronous copy: it must stay
-// valid until the stream has consumed it.  Leaves pr->h_cor with row ranges that CONTAIN the planned ones
-// (the refined offset moves the limits by at most 2 / slope rows), for buffer sizes.
-int dab_enqueue_plan_corridors(dab_pair *pr, const dab_cluster *clusters, int32_t n_clusters, int64_t n_a, int64_t n_v) {
+// valid until the stream has consumed it.  The plan's host corridors are row ranges that CONTAIN the planned
+// ones (the refined offset moves the limits by at most 2 / slope rows), for buffer sizes.
+static int enqueue_plan_corridors(dab_pair *pr, const dab_cluster *clusters, int32_t n_clusters, int64_t n_a, int64_t n_v) {
   dab_ctx *ctx = pr->ctx;
   cudaStream_t st = pr->stream;
-  pr->h_cor.clear();
+  std::vector<dab_corridor> cor;
   for (int k = 0; k < n_clusters; ++k) {
     const dab_cluster &c = clusters[k];
     if (c.cluster < 0 || (k > 0 && c.cluster <= clusters[k - 1].cluster) || !(c.slope == c.slope) || c.slope == 0.0) {
@@ -507,7 +562,7 @@ int dab_enqueue_plan_corridors(dab_pair *pr, const dab_cluster *clusters, int32_
       if (hi2 > n_a - 1) hi2 = n_a - 1;
       if (hi2 > lo2) { out.lo = (int32_t)lo2; out.hi = (int32_t)hi2; }
     }
-    pr->h_cor.push_back(out);
+    cor.push_back(out);
   }
   const int max_blocks = (int)cdiv(n_a > 0 ? n_a : 1, RF_CHUNK);
   DAB_TRY(dab_ensure(ctx, pr->clusters, sizeof(dab_cluster) * (size_t)(n_clusters + 1)));
@@ -527,33 +582,31 @@ int dab_enqueue_plan_corridors(dab_pair *pr, const dab_cluster *clusters, int32_
     ctx->launches += 2;
   }
   DAB_CUDA(cudaGetLastError());
-  pr->b_device_planned = true;
+  dab_set_stage_b_plan(pr, n_a, n_v, std::move(cor), n_clusters > 0 ? clusters[n_clusters - 1].cluster + 1 : 0, true);
   return DAB_OK;
 }
 
-// Stage B enqueued on the pair's stream without a host round trip: every (corridor, row) yields at most
-// one point, so the sum of the corridor rows (known to the host) bounds all buffers; the actual point
-// count stays on the device and every later kernel reads it from there.
-int dab_enqueue_stage_b(dab_pair *pr, int32_t n_cor, int32_t n_clusters) {
-  DAB_TRY(dab_enqueue_stage_b_points(pr, n_cor, n_clusters, 0, INT64_MAX));
-  return dab_enqueue_stage_b_dp(pr, n_cor, n_clusters);
+int dab_enqueue_stage_b_clusters(dab_pair *pr, const float gain[3], const float audio_std[3], int64_t n_audio, int64_t n_video,
+                                 const dab_cluster *clusters, int32_t n_clusters, int64_t row_lo, int64_t row_hi, bool with_dp,
+                                 const char *who) {
+  if (n_clusters < 0 || (n_clusters > 0 && !clusters) || row_lo < 0 || row_hi < row_lo) {
+    dab_set_err(pr->ctx, std::string(who) + ": invalid argument");
+    return DAB_E_ARG;
+  }
+  DAB_TRY(enqueue_scaling(pr, gain, audio_std, n_audio, n_video));
+  DAB_TRY(enqueue_plan_corridors(pr, clusters, n_clusters, n_audio, n_video));
+  return dab_enqueue_stage_b(pr, row_lo, row_hi, with_dp);
 }
 
 // corridor scoring: the sorted point list with flags; quals only for audio rows [q_lo, q_hi)
-int dab_enqueue_stage_b_points(dab_pair *pr, int32_t n_cor, int32_t n_clusters, int64_t q_lo, int64_t q_hi) {
+static int enqueue_points(dab_pair *pr, int64_t q_lo, int64_t q_hi) {
   dab_ctx *ctx = pr->ctx;
   cudaStream_t st = pr->stream;
-  const int64_t n_a = pr->stats.n_audio_frames, n_v = pr->stats.n_video_frames;  // set by the caller
-  (void)n_clusters; (void)n_v;
+  const StageBPlan &b = pr->plan_b;
+  const int64_t n_a = b.n_audio, n_v = b.n_video, rows = b.rows;
+  const int32_t n_cor = (int32_t)b.cor.size();
   pr->n_points2 = pr->n_path2 = 0;
-  const bool fast = corridor_dp_eligible(pr, n_cor);
-  int64_t pm_off[32], rows = 0;
-  for (int k = 0; k < n_cor; ++k) {
-    if (k < 32) pm_off[k] = rows;
-    rows += pr->h_cor[k].hi > pr->h_cor[k].lo ? pr->h_cor[k].hi - pr->h_cor[k].lo : 0;
-  }
   const int64_t cap = rows > 0 ? rows : 1;
-  pr->cap_points2 = cap;
   DAB_TRY(dab_ensure(ctx, pr->counters, sizeof(int32_t) * DC_WORDS));
   int32_t *dc = pr->counters.as<int32_t>();
   DAB_CUDA(cudaMemsetAsync(dc + DC_N_PTS2, 0, sizeof(int32_t) * (DC_WORDS - DC_N_PTS2), st));
@@ -562,7 +615,7 @@ int dab_enqueue_stage_b_points(dab_pair *pr, int32_t n_cor, int32_t n_clusters, 
   sb.n_a = n_a; sb.n_v = n_v;
   sb.cor = pr->corridors.as<dab_corridor>(); sb.n_cor = n_cor;
   sb.maxes = pr->maxes.as<float>();
-  sb.want_rank = fast ? 0 : 1;
+  sb.want_rank = b.scan_dp ? 0 : 1;
   sb.q_lo = q_lo; sb.q_hi = q_hi;
   DAB_TRY(dab_ensure(ctx, pr->row2_count, sizeof(int32_t) * (size_t)(n_a + 2)));
   DAB_TRY(dab_ensure(ctx, pr->row2_off, sizeof(int32_t) * (size_t)(n_a + 2)));
@@ -593,20 +646,16 @@ int dab_enqueue_stage_b_points(dab_pair *pr, int32_t n_cor, int32_t n_clusters, 
 }
 
 // DP #2 + traceback over the pair's pass-2 points
-int dab_enqueue_stage_b_dp(dab_pair *pr, int32_t n_cor, int32_t n_clusters) {
+int dab_enqueue_stage_b_dp(dab_pair *pr) {
   dab_ctx *ctx = pr->ctx;
   cudaStream_t st = pr->stream;
-  const int64_t n_v = pr->stats.n_video_frames;
-  const bool fast = corridor_dp_eligible(pr, n_cor);
-  int64_t pm_off[32], rows = 0;
-  for (int k = 0; k < n_cor; ++k) {
-    if (k < 32) pm_off[k] = rows;
-    rows += pr->h_cor[k].hi > pr->h_cor[k].lo ? pr->h_cor[k].hi - pr->h_cor[k].lo : 0;
-  }
+  const StageBPlan &b = pr->plan_b;
+  const int64_t n_v = b.n_video, rows = b.rows;
+  const int32_t n_cor = (int32_t)b.cor.size(), n_clusters = b.n_clusters;
   const int64_t cap = rows > 0 ? rows : 1;
   int32_t *dc = pr->counters.as<int32_t>();
   DAB_CUDA(cudaEventRecord(pr->ev[16], st));
-  if (rows > 0 && fast) {
+  if (rows > 0 && b.scan_dp) {
     // ---- scan DP + chunked traceback ----
     const int chunks = (int)cdiv(cap, TB_CHUNK);
     DAB_TRY(dab_ensure(ctx, pr->pm2, sizeof(PmEntry) * (size_t)(rows + 1)));
@@ -617,7 +666,7 @@ int dab_enqueue_stage_b_dp(dab_pair *pr, int32_t n_cor, int32_t n_clusters) {
     la.rec = pr->p2_k.as<P2Rec>(); la.p_j = pr->p2_j.as<double>();
     la.n_points = dc + DC_N_PTS2;
     la.cor = pr->corridors.as<dab_corridor>(); la.n_cor = n_cor;
-    for (int k = 0; k < 32; ++k) la.pm_off[k] = k < n_cor ? pm_off[k] : 0;
+    for (int k = 0; k < 32; ++k) la.pm_off[k] = b.pm_off[k];
     la.pm = pr->pm2.as<PmEntry>();
     la.back = pr->back2.as<BackRec>();
     la.result = dc + DC_DP2_END;
@@ -697,6 +746,15 @@ int dab_enqueue_stage_b_dp(dab_pair *pr, int32_t n_cor, int32_t n_clusters) {
   return DAB_OK;
 }
 
+// Stage B enqueued on the pair's stream without a host round trip: every (corridor, row) yields at most
+// one point, so the sum of the corridor rows (known to the host) bounds all buffers; the actual point
+// count stays on the device and every later kernel reads it from there.
+int dab_enqueue_stage_b(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp) {
+  DAB_TRY(enqueue_points(pr, row_lo, row_hi));
+  if (with_dp) DAB_TRY(dab_enqueue_stage_b_dp(pr));
+  return dab_enqueue_counts(pr);
+}
+
 // quals of all pass-2 points replaced by `q_all` (device memory): the exchange step of a long pair whose
 // corridor rows were scored on several GPUs
 static __global__ void set_quals_kernel(const double *q_all, const int32_t *n_dev, P2Rec *rec, double *p_q) {
@@ -709,7 +767,7 @@ static __global__ void set_quals_kernel(const double *q_all, const int32_t *n_de
 
 int dab_enqueue_set_quals2(dab_pair *pr, const double *d_q_all) {
   dab_ctx *ctx = pr->ctx;
-  const int64_t cap = pr->cap_points2 > 0 ? pr->cap_points2 : 1;
+  const int64_t cap = pr->plan_b.rows > 0 ? pr->plan_b.rows : 1;
   set_quals_kernel<<<(unsigned)cdiv(cap, 256), 256, 0, pr->stream>>>(d_q_all, pr->counters.as<int32_t>() + DC_N_PTS2,
                                                                     pr->p2_k.as<P2Rec>(), pr->p2_q.as<double>());
   ctx->launches += 1;
@@ -717,10 +775,10 @@ int dab_enqueue_set_quals2(dab_pair *pr, const double *d_q_all) {
   return DAB_OK;
 }
 
-// first point and number of points of the audio rows [lo, hi) (needs a finished dab_enqueue_stage_b_points)
+// first point and number of points of the audio rows [lo, hi) (needs a finished dab_enqueue_stage_b)
 int dab_row_range_points2(dab_pair *pr, int64_t lo, int64_t hi, int64_t *first, int64_t *count) {
   dab_ctx *ctx = pr->ctx;
-  const int64_t n_a = pr->stats.n_audio_frames;
+  const int64_t n_a = pr->plan_b.n_audio;
   lo = lo < 0 ? 0 : (lo > n_a ? n_a : lo);
   hi = hi < lo ? lo : (hi > n_a ? n_a : hi);
   int32_t off[2] = {0, 0};
@@ -732,12 +790,13 @@ int dab_row_range_points2(dab_pair *pr, int64_t lo, int64_t hi, int64_t *first, 
   return DAB_OK;
 }
 
-int dab_collect_stage_b(dab_pair *pr) {
+int dab_collect_stage_b(dab_pair *pr, bool with_dp) {
   dab_ctx *ctx = pr->ctx;
   const int32_t *hc = reinterpret_cast<const int32_t *>(pr->h_counters);
   if (hc[DC_OVERFLOW_B] & DAB_OVF_ROWCOR) { dab_set_err(ctx, "more than 32 corridors overlap one audio row"); return DAB_E_CAPACITY; }
   pr->n_points2 = hc[DC_N_PTS2];
   pr->stats.n_points2 = pr->n_points2;
+  if (!with_dp) return DAB_OK;
   pr->n_path2 = (pr->n_points2 > 0 && hc[DC_DP2_END] >= 0) ? hc[DC_N_PATH2] : 0;
   pr->stats.n_path2 = pr->n_path2;
   const int64_t *cnt = reinterpret_cast<const int64_t *>(hc + DC_DP2_CNT);
