@@ -202,6 +202,7 @@ enum {
   DC_OVERFLOW_B = 17,  // stage B: bit 2 more than 32 corridors on one audio row
   DC_DP2_END = 18,     // end id, path length, then the frontier value (double at words 20-21)
   DC_N_PATH2 = 19,
+  DC_NEED_ENTRIES = 22, DC_NEED_CAND = 23,    // unclamped table-entry and candidate totals (sizes the next run)
   DC_DP2_CNT = 24,     // 4 x u64 DP-2 work counters
   DC_WORDS = 32
 };
@@ -213,8 +214,9 @@ int dab_run_features(dab_pair *pr, int track, const void *d_pcm, int format);
 // dab_enqueue_counts, which copies the counts block to the mapped host page; once the stream has passed that
 // point, dab_collect_* interprets it.
 int dab_enqueue_counts(dab_pair *pr);
-// Stage A.  On a capacity overflow dab_collect_stage_a grows the buffer and returns DAB_E_CAPACITY: the caller
-// enqueues the stage again, up to DAB_STAGE_A_ATTEMPTS runs in all.
+// Stage A.  On a capacity overflow dab_collect_stage_a grows the buffer to at least the total the run needed and
+// returns DAB_E_CAPACITY: the caller enqueues the stage again, up to DAB_STAGE_A_ATTEMPTS runs in all.  An
+// entries overflow leaves the tables empty, so the candidate total is only known one run later: three runs at most.
 constexpr int DAB_STAGE_A_ATTEMPTS = 8;
 int dab_check_stage_a_inputs(dab_pair *pr, const char *who);
 // match points of audio rows [row_lo, row_hi), then DP 1 + traceback if with_dp, then the counts

@@ -1059,9 +1059,11 @@ static __global__ void counts_lists_kernel(int32_t *dc, const int32_t *v_off, in
   dc[DC_N_Q] = a_off[hi] - a_off[lo];
 }
 
-// a scan total against the capacity of the buffer it sizes: clamps the count and raises the overflow bit
-static __global__ void check_capacity_kernel(int32_t *dc, int word, int64_t cap, int bit) {
+// a scan total against the capacity of the buffer it sizes: keeps the total in need_word, then clamps the count and
+// raises the overflow bit
+static __global__ void check_capacity_kernel(int32_t *dc, int word, int need_word, int64_t cap, int bit) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  dc[need_word] = dc[word];
   if ((int64_t)dc[word] > cap) { dc[word] = 0; atomicOr(&dc[DC_OVERFLOW], bit); }
 }
 
@@ -1176,7 +1178,7 @@ static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
   int32_t *ecount = pr->tbl_ecount.as<int32_t>(), *ebase = ecount + (5 * vsel_ub + 1);
   table_expand_kernel<<<gt, 128, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, vsel_ub, ecount);
   DAB_TRY(dab_exclusive_scan(pr, ecount, ebase, 5 * vsel_ub, nullptr, dc + DC_N_ENTRIES));
-  check_capacity_kernel<<<1, 32, 0, st>>>(dc, DC_N_ENTRIES, cap_e, DAB_OVF_ENTRIES);
+  check_capacity_kernel<<<1, 32, 0, st>>>(dc, DC_N_ENTRIES, DC_NEED_ENTRIES, cap_e, DAB_OVF_ENTRIES);
   table_kernel<false><<<gt, 128, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, vsel_ub, ebase,
                                           pr->tbl_pos.as<int32_t>(), pr->tbl_count.as<int32_t>(), nullptr, nullptr, cap_e);
   DAB_TRY(dab_exclusive_scan(pr, pr->tbl_count.as<int32_t>(), pr->tbl_start.as<int32_t>(), nslots));
@@ -1219,7 +1221,7 @@ static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
   gate_entries_kernel<<<(unsigned)(8 * ctx->sm_count), GE_THREADS, 0, st>>>(ga, pr->gate_rec.as<GateQ>(), g_P);
   ctx->launches += 2;
   DAB_TRY(dab_exclusive_scan(pr, pr->row_count.as<int32_t>(), pr->row_off.as<int32_t>(), q_ub, nullptr, dc + DC_N_CAND));
-  check_capacity_kernel<<<1, 32, 0, st>>>(dc, DC_N_CAND, cap_c, DAB_OVF_CAND);
+  check_capacity_kernel<<<1, 32, 0, st>>>(dc, DC_N_CAND, DC_NEED_CAND, cap_c, DAB_OVF_CAND);
   gate_fill_small_kernel<<<(unsigned)cdiv(q_ub, 256), 256, 0, st>>>(ga);
   gate_fill_big_kernel<<<(unsigned)(2 * ctx->sm_count), 256, 0, st>>>(ga);
   ctx->launches += 4;
@@ -1337,8 +1339,10 @@ int dab_collect_stage_a(dab_pair *pr, bool with_dp) {
   pr->stats.n_candidates = hc[DC_N_CAND];
   const int ovf = hc[DC_OVERFLOW];
   if (ovf & (DAB_OVF_ENTRIES | DAB_OVF_CAND)) {
-    if (ovf & DAB_OVF_ENTRIES) pr->cap_entries *= 2;
-    if (ovf & DAB_OVF_CAND) pr->cap_cand *= 2;
+    // doubled, and at least the total this run needed: repeated audio (a shared tone, a looped bed) can need
+    // hundreds of times the first guess, more than doubling reaches within DAB_STAGE_A_ATTEMPTS runs
+    if (ovf & DAB_OVF_ENTRIES) pr->cap_entries = std::max<int64_t>(2 * pr->cap_entries, hc[DC_NEED_ENTRIES]);
+    if (ovf & DAB_OVF_CAND) pr->cap_cand = std::max<int64_t>(2 * pr->cap_cand, hc[DC_NEED_CAND]);
     dab_set_err(ctx, "stage A: a device buffer overflowed, capacity doubled");
     return DAB_E_CAPACITY;
   }
