@@ -13,8 +13,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdescribealign_b200.so")
-SOURCES = ["api.cu", "features.cu", "stage_a.cu", "stage_b.cu", "engine.cu", "pcm_reader.cu", "stretch.cu", "host_stage.cpp"]
-HEADERS = ["common.cuh", "dp2_scan.cuh", "refine.cuh", "traceback.cuh", "hann_tables.h", os.path.join("..", "..", "include", "describealign_b200.h")]
+SOURCES = ["api.cu", "features.cu", "stage_a.cu", "stage_b.cu", "traceback.cu", "engine.cu", "pcm_reader.cu", "stretch.cu", "host_stage.cpp"]
+HEADERS = ["common.cuh", "dp2_scan.cuh", "refine.cuh", "hann_tables.h", os.path.join("..", "..", "include", "describealign_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

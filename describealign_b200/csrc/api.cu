@@ -269,11 +269,11 @@ void dab_pair_destroy(dab_pair *pr) {
   }
   DevBuf *bs[] = {&pr->scan_tmp, &pr->tbl_count, &pr->tbl_start, &pr->tbl_items, &pr->tbl_ecount, &pr->tbl_pos, &pr->v_rec, &pr->clusters, &pr->refine_partial, &pr->maxes, &pr->row_count, &pr->row_off, &pr->row_stash, &pr->gate_rec, &pr->gate_best, &pr->gate_big,
                   &pr->cand_tmp, &pr->cand_s, &pr->cand_i, &pr->cand_q, &pr->keep_flag, &pr->keep_off, &pr->pt_i,
-                  &pr->pt_s, &pr->pt_q, &pr->counters, &pr->tree1, &pr->back1, &pr->len1, &pr->cp1, &pr->dpres,
-                  &pr->seglist, &pr->path1_x, &pr->path1_y, &pr->a_scaled, &pr->v_scaled, &pr->corridors,
+                  &pr->pt_s, &pr->pt_q, &pr->counters, &pr->tree1, &pr->back1, &pr->dpres,
+                  &pr->path1_x, &pr->path1_y, &pr->a_scaled, &pr->v_scaled, &pr->corridors,
                   &pr->row2_count, &pr->row2_off, &pr->p2_i, &pr->p2_c, &pr->p2_rank, &pr->p2_j, &pr->p2_q,
-                  &pr->tree2, &pr->cache2, &pr->back2, &pr->len2, &pr->cp2, &pr->backid2, &pr->path2,
-                  &pr->p2_k, &pr->pm2, &pr->pmoff2, &pr->lift_up, &pr->lift_dep};
+                  &pr->tree2, &pr->cache2, &pr->cluster_best2, &pr->back2, &pr->path2,
+                  &pr->p2_k, &pr->pm2, &pr->tb_up, &pr->tb_mark};
   for (DevBuf *b : bs) free_buf(*b);
   for (int k = 0; k < 32; ++k)
     if (pr->ev[k]) cudaEventDestroy(pr->ev[k]);

@@ -93,9 +93,8 @@ struct dab_pair {
   DevBuf counters;             // i64 [16] device counters
   // dp1
   DevBuf tree1;                // Node16 levels
-  DevBuf back1, len1, cp1;     // i32 [n_points]
+  DevBuf back1;                // BackRec [n_points]
   DevBuf dpres;                // i32/i64 results (end id, path len)
-  DevBuf seglist;              // i32 checkpoints
   DevBuf path1_x, path1_y;     // i32
   int64_t n_points1 = 0, n_path1 = 0;
   int64_t cap_entries = 0, cap_cand = 0, cap_points1 = 0;   // capacities of device-sized buffers (grown on overflow)
@@ -105,14 +104,14 @@ struct dab_pair {
   DevBuf corridors;            // dab_corridor[]
   DevBuf row2_count, row2_off; // i32 [n_audio + 1]
   DevBuf p2_i, p2_c, p2_rank, p2_k;  // i32
-  DevBuf pm2, pmoff2;          // corridor-state DP: per-corridor running maxima, row offsets
-  DevBuf lift_up, lift_dep;    // pointer-jumping traceback
+  DevBuf pm2;                  // corridor-state DP: per-corridor running maxima
+  DevBuf tb_up, tb_mark;       // traceback scratch of both DPs (they run one after the other on the stream)
   StageBPlan plan_b;
   DevBuf p2_j, p2_q;           // f64
   DevBuf tree2;                // frontier tree of pass 2
   DevBuf cache2;               // prev_cache rows
-  DevBuf back2;                // per point: predecessor tuple
-  DevBuf len2, cp2, backid2;   // i32
+  DevBuf cluster_best2;        // tree DP: per cluster, cum - 50 of its best point (f64) and its id (i32)
+  DevBuf back2;                // BackRec [n_points]
   DevBuf path2;                // f64 (n,5)
   int64_t n_points2 = 0, n_path2 = 0;
   DevBuf clusters, refine_partial, maxes;
@@ -192,16 +191,16 @@ enum {
   DC_ENUM_LO = 4, DC_ENUM_HI = 5,   // u64: bucket entries visited by the gate
   DC_N_CAND = 6,
   DC_N_PTS1 = 7,
-  DC_DP1_END = 8,      // end id, path length (two consecutive words, written by dp1_kernel)
-  DC_N_PATH1 = 9,
+  DC_DP1_END = 8,      // end id (-1: no path), written by dp1_kernel
+  DC_N_PATH1 = 9,      // path length, written by the traceback
   DC_Q_LO = 10, DC_Q_HI = 11, DC_N_Q = 12,    // query range of this shard in the not-quiet audio list
   DC_OVERFLOW = 13,    // bit 0 table entries, bit 1 candidates, bit 2 > 32 corridors on a row, bit 3 pass-2 points
   DC_BAD_IMPORT = 14,
   DC_N_BIGROWS = 15,   // gate rows with more than GATE_STASH candidates
   DC_N_PTS2 = 16,
   DC_OVERFLOW_B = 17,  // stage B: bit 2 more than 32 corridors on one audio row
-  DC_DP2_END = 18,     // end id, path length, then the frontier value (double at words 20-21)
-  DC_N_PATH2 = 19,
+  DC_DP2_END = 18,     // end id, then the frontier value (double at words 20-21)
+  DC_N_PATH2 = 19,     // path length, written by the traceback
   DC_NEED_ENTRIES = 22, DC_NEED_CAND = 23,    // unclamped table-entry and candidate totals (sizes the next run)
   DC_DP2_CNT = 24,     // 4 x u64 DP-2 work counters
   DC_WORDS = 32
@@ -241,6 +240,31 @@ int dab_enqueue_stage_b_dp(dab_pair *pr);
 int dab_enqueue_set_quals2(dab_pair *pr, const double *d_q_all);
 int dab_row_range_points2(dab_pair *pr, int64_t lo, int64_t hi, int64_t *first, int64_t *count);
 int dab_collect_stage_b(dab_pair *pr, bool with_dp);
+
+// What both frontier DPs keep per point for the traceback: the value the point started from and its
+// predecessor's id (-1: the seed).  A predecessor always has a smaller id than its point.
+struct __align__(16) BackRec {
+  double best;
+  int32_t pred;
+  int32_t pad;
+};
+
+// What the traceback writes for every path point, in path order.
+struct Path1Out {              // pass 1: audio frame x, video frame y
+  const int32_t *pt_i, *pt_s, *v_sel;
+  int32_t *x, *y;
+};
+struct Path2Out {              // pass 2: rows (j, i, cluster, qual, cum)
+  const int32_t *p_i, *p_c;
+  const double *p_j, *p_q;
+  double *rows;
+};
+// Traceback (traceback.cu) from the end id result[0] (-1: empty path) through the back records of the *n_dev <= cap
+// points; the path length goes to *n_path.  Pass 2 also reads the end point's frontier value, a double at result + 2.
+int dab_enqueue_traceback(dab_pair *pr, const BackRec *back, const int32_t *n_dev, const int32_t *result, int64_t cap,
+                          int32_t *n_path, const Path1Out &out);
+int dab_enqueue_traceback(dab_pair *pr, const BackRec *back, const int32_t *n_dev, const int32_t *result, int64_t cap,
+                          int32_t *n_path, const Path2Out &out);
 
 #define DAB_LAUNCHED(pr) ((pr)->ctx->launches++)
 

@@ -7,7 +7,7 @@
 //   gate      per audio query: (>= 2 of tables 0-2) and (table 3 or 4)         (:649-660)
 //   score     3 x 41-tap normalised correlation -> prob -> qual                (:662-673)
 //   dp1       frontier DP as a prefix-max over video rank, with back pointers  (:654-656, 674-682)
-//   trace     traceback through checkpointed back pointers                     (:690-697)
+//   trace     chunked traceback of the back pointers (traceback.cu)            (:690-697)
 //
 // Layout: every per-frame array is structure-of-arrays in HBM (feature-major) so that a warp
 // touching consecutive frames reads consecutive addresses.  The hash "dict of sets" of the
@@ -765,15 +765,14 @@ struct __align__(16) Node1 {
 };
 
 constexpr int DP_LEVELS = 4;
-constexpr int DP_CHECK = 256;   // checkpoint spacing for the parallel traceback
 
 struct Dp1Args {
   const int32_t *pt_s;
   const double *pt_q;
   const int32_t *n_points;       // device count
   Node1 *level[DP_LEVELS];
-  int4 *meta;                    // per point (back pointer, chain length, checkpoint id, -)
-  int32_t *result;               // [0] end id, [1] path length
+  BackRec *back;                 // per point (predecessor's cum, predecessor)
+  int32_t *result;               // [0] end id, -1: no path
 };
 
 __device__ __forceinline__ bool key_better(double ca, int ra, double cb, int rb) {
@@ -805,7 +804,7 @@ __global__ void __launch_bounds__(32, 1) dp1_kernel(Dp1Args a) {
   const int lane = threadIdx.x;
   const int n = *a.n_points;
   double top_cum = 0.0;
-  int top_id = -1, top_rank = -1, top_len = 0, top_cp = -1;
+  int top_id = -1, top_rank = -1;
   const int role = lane < DP_LEVELS ? lane : 0;
   int4 *const my_level = reinterpret_cast<int4 *>(a.level[role]);
   const int my_shift = 5 * role;
@@ -873,13 +872,9 @@ __global__ void __launch_bounds__(32, 1) dp1_kernel(Dp1Args a) {
         double old_cum = __shfl_up_sync(0xffffffffu, my_cum, 1);
         int old_id = base + lane - 1, old_rank = prev_r;
         if (first) { old_cum = top_cum; old_id = top_id; old_rank = top_rank; }
-        const int ln = top_len + 1 + (lane - t);
-        const unsigned fm = __ballot_sync(0xffffffffu, in_run && (ln % DP_CHECK == 0 || (first && top_id < 0)));
-        const unsigned fml = fm & ((2u << lane) - 1u);
-        const int cpv = fml ? base + 31 - __clz(fml) : top_cp;
         if (in_run) {
-          int4 m; m.x = old_id; m.y = ln; m.z = cpv; m.w = 0;
-          a.meta[base + lane] = m;
+          BackRec b; b.best = old_cum; b.pred = old_id; b.pad = 0;
+          a.back[base + lane] = b;
           if (lane == t + len - 1 || next_r != my_r) {       // the last point on a rank owns its leaf
             Node1 me; me.cum = my_cum; me.id = base + lane; me.rank = my_r;
             a.level[0][my_r] = me;
@@ -897,8 +892,6 @@ __global__ void __launch_bounds__(32, 1) dp1_kernel(Dp1Args a) {
         const int last = t + len - 1;
         top_cum = __shfl_sync(0xffffffffu, my_cum, last);
         top_rank = __shfl_sync(0xffffffffu, my_r, last);
-        top_len = __shfl_sync(0xffffffffu, ln, last);
-        top_cp = __shfl_sync(0xffffffffu, cpv, last);
         top_id = base + last;
         t += len;
         continue;
@@ -948,13 +941,7 @@ __global__ void __launch_bounds__(32, 1) dp1_kernel(Dp1Args a) {
           a.level[k][r >> (5 * k)] = me;
         }
       }
-      int ln = 1, cpv = p;
-      if (pid >= 0) {
-        const int4 pm = __ldcg(a.meta + pid);
-        ln = pm.y + 1;
-        cpv = (ln % DP_CHECK == 0) ? p : pm.z;
-      }
-      if (lane == 0) { int4 m; m.x = pid; m.y = ln; m.z = cpv; m.w = 0; a.meta[p] = m; }
+      if (lane == 0) { BackRec b; b.best = pc; b.pred = pid; b.pad = 0; a.back[p] = b; }
       if (key_better(cum, r, top_cum, top_rank)) {
         // the old top's ancestors are flushed where the new top lies in another block
         if (lane >= 1 && lane < DP_LEVELS && top_id >= 0 && (r >> my_shift) != (top_rank >> my_shift)) {
@@ -962,53 +949,13 @@ __global__ void __launch_bounds__(32, 1) dp1_kernel(Dp1Args a) {
           val.x = __double2loint(top_cum); val.y = __double2hiint(top_cum); val.z = top_id; val.w = top_rank;
           my_level[top_rank >> my_shift] = val;
         }
-        top_cum = cum; top_id = p; top_rank = r; top_len = ln; top_cp = cpv;
+        top_cum = cum; top_id = p; top_rank = r;
       }
       __syncwarp();
     }
     __syncwarp();
   }
-  if (lane == 0) {
-    a.result[0] = top_id;
-    a.result[1] = top_id < 0 ? 0 : top_len;
-  }
-}
-
-// Traceback: thread 0 hops from checkpoint to checkpoint (path_len / 256 dependent steps),
-// then every segment between checkpoints is walked by its own thread.
-struct TraceArgs {
-  const int4 *meta;              // (back, len, cp, -)
-  const int32_t *result;
-  const int32_t *pt_i, *pt_s, *v_sel;
-  int32_t *seg;          // scratch: segment start ids
-  int32_t *path_x, *path_y;
-};
-
-__global__ void trace1_kernel(TraceArgs a) {
-  __shared__ int nseg;
-  if (threadIdx.x == 0) {
-    int k = 0;
-    int cur = a.result[0];
-    while (cur >= 0) {
-      a.seg[k++] = cur;
-      const int c = a.meta[cur].z;  // last node of this segment (checkpoint or chain root)
-      cur = a.meta[c].x;
-    }
-    nseg = k;
-  }
-  __syncthreads();
-  for (int s = threadIdx.x; s < nseg; s += blockDim.x) {
-    int cur = a.seg[s];
-    const int stop = a.meta[cur].z;
-    while (true) {
-      const int4 m = a.meta[cur];
-      const int pos = m.y - 1;
-      a.path_x[pos] = a.pt_i[cur];
-      a.path_y[pos] = a.v_sel[a.pt_s[cur]];
-      if (cur == stop) break;
-      cur = m.x;
-    }
-  }
+  if (lane == 0) a.result[0] = top_id;
 }
 
 __global__ void fill_nodes_kernel(Node1 *p, int64_t n) {
@@ -1273,8 +1220,7 @@ int dab_enqueue_stage_a_dp(dab_pair *pr) {
   for (int k = 0; k < DP_LEVELS; ++k) { lv[k] = cdiv(m > 0 ? m : 1, 32) * 32; tot += lv[k]; m = cdiv(m, 32); }
   DAB_TRY(dab_ensure(ctx, pr->tree1, sizeof(Node1) * (size_t)tot));
   fill_nodes_kernel<<<(unsigned)cdiv(tot, 256), 256, 0, st>>>(pr->tree1.as<Node1>(), tot);
-  DAB_TRY(dab_ensure(ctx, pr->back1, sizeof(int4) * (size_t)(cap_p + 1)));
-  DAB_TRY(dab_ensure(ctx, pr->seglist, sizeof(int32_t) * (size_t)(cap_p / DP_CHECK + 16)));
+  DAB_TRY(dab_ensure(ctx, pr->back1, sizeof(BackRec) * (size_t)(cap_p + 1)));
   DAB_TRY(dab_ensure(ctx, pr->path1_x, sizeof(int32_t) * (size_t)(cap_p + 1)));
   DAB_TRY(dab_ensure(ctx, pr->path1_y, sizeof(int32_t) * (size_t)(cap_p + 1)));
   Dp1Args da;
@@ -1282,15 +1228,14 @@ int dab_enqueue_stage_a_dp(dab_pair *pr) {
   da.n_points = dc + DC_N_PTS1;
   Node1 *base = pr->tree1.as<Node1>();
   for (int k = 0; k < DP_LEVELS; ++k) { da.level[k] = base; base += lv[k]; }
-  da.meta = pr->back1.as<int4>();
+  da.back = pr->back1.as<BackRec>();
   da.result = dc + DC_DP1_END;
   dp1_kernel<<<1, 32, 0, st>>>(da);
-  TraceArgs ta;
-  ta.meta = da.meta; ta.result = da.result;
-  ta.pt_i = pr->pt_i.as<int32_t>(); ta.pt_s = pr->pt_s.as<int32_t>(); ta.v_sel = V.nq_list.as<int32_t>();
-  ta.seg = pr->seglist.as<int32_t>(); ta.path_x = pr->path1_x.as<int32_t>(); ta.path_y = pr->path1_y.as<int32_t>();
-  trace1_kernel<<<1, 256, 0, st>>>(ta);
-  ctx->launches += 3;
+  ctx->launches += 2;
+  Path1Out out;
+  out.pt_i = pr->pt_i.as<int32_t>(); out.pt_s = da.pt_s; out.v_sel = V.nq_list.as<int32_t>();
+  out.x = pr->path1_x.as<int32_t>(); out.y = pr->path1_y.as<int32_t>();
+  DAB_TRY(dab_enqueue_traceback(pr, da.back, da.n_points, da.result, cap_p, dc + DC_N_PATH1, out));
   DAB_CUDA(cudaEventRecord(pr->ev[13], st));
   pr->ev_used[6] = true;
   DAB_CUDA(cudaGetLastError());

@@ -3,7 +3,7 @@
 //                     cluster's line; qual from the linearly interpolated video features and the
 //                     energy gates; first cluster to claim (i, int(j)) wins          (:931-944)
 //   dp2               second frontier DP with global / same-cluster / local steps    (:946-983)
-//   trace             traceback, rows (j, i, cluster, qual, cum)                     (:985-990)
+//   trace             traceback (traceback.cu), rows (j, i, cluster, qual, cum)      (:985-990)
 //
 // The reference keys its frontier by the float video coordinate j.  Here every point gets
 // rank(j) = 1 + number of corridor rows (over all corridors) whose coordinate is < j, found by
@@ -198,7 +198,6 @@ struct __align__(16) Cell2 {   // prev_cache row
 };
 
 constexpr int L2N = 5;          // 32^5 ranks
-constexpr int CHECK2 = 256;
 
 struct Dp2Args {
   const int32_t *p_i, *p_c, *p_rank;
@@ -208,9 +207,8 @@ struct Dp2Args {
   Cell2 *cache;
   double *cb_val;     // per cluster: cum - 50 of its best point
   int32_t *cb_id;
-  int32_t *back_id, *len, *cp;
-  double *back_cum;
-  int32_t *result;    // [0] end id, [1] path length ; double result_val at +2
+  BackRec *back;
+  int32_t *result;    // [0] end id ; double result_val at +2
 };
 
 __device__ __forceinline__ unsigned long long order_bits(double v) {
@@ -291,11 +289,8 @@ __global__ void __launch_bounds__(32, 1) dp2_kernel(Dp2Args a) {
     if (lane == 0) {
       Cell2 me; me.j = j; me.q = q; me.cum = cum; me.i = i; me.c = c; me.id = p; me.pad = 0;
       a.cache[ij] = me;
-      a.back_id[p] = pred;
-      a.back_cum[p] = best;
-      const int ln = pred < 0 ? 1 : a.len[pred] + 1;
-      a.len[p] = ln;
-      a.cp[p] = (ln % CHECK2 == 0 || pred < 0) ? p : a.cp[pred];
+      // the BackRec {best, pred, 0} as one double2: a struct copy here costs this kernel 12 more registers
+      *reinterpret_cast<double2 *>(a.back + p) = make_double2(best, __hiloint2double(0, pred));
       if (cl_val < cum - 50.0) { a.cb_val[c] = cum - 50.0; a.cb_id[c] = p; }
     }
     const double jump = cum - 1000.0;
@@ -318,52 +313,7 @@ __global__ void __launch_bounds__(32, 1) dp2_kernel(Dp2Args a) {
   }
   if (lane == 0) {
     a.result[0] = top_id;
-    a.result[1] = top_id < 0 ? 0 : a.len[top_id];
     *reinterpret_cast<double *>(a.result + 2) = top_val;
-  }
-}
-
-struct Trace2Args {
-  const int32_t *back_id, *len, *cp, *result;
-  const double *back_cum;
-  const int32_t *p_i, *p_c;
-  const double *p_j, *p_q;
-  int32_t *seg;
-  double *rows;    // (n_path, 5)
-};
-
-__global__ void trace2_kernel(Trace2Args a) {
-  __shared__ int nseg;
-  if (threadIdx.x == 0) {
-    int k = 0;
-    int cur = a.result[0];
-    while (cur >= 0) {
-      a.seg[2 * k] = cur;
-      const int c = a.cp[cur];
-      const int nxt = a.back_id[c];
-      a.seg[2 * k + 1] = c;        // last node of the segment; its predecessor starts the next
-      ++k;
-      cur = nxt;
-    }
-    nseg = k;
-  }
-  __syncthreads();
-  const double top_val = *reinterpret_cast<const double *>(a.result + 2);
-  for (int s = threadIdx.x; s < nseg; s += blockDim.x) {
-    int cur = a.seg[2 * s];
-    const int stop = a.seg[2 * s + 1];
-    // 5th column of a row = the (penalised) cumulative value its successor started from;
-    // for the last row it is the frontier value of the end point
-    double col5;
-    if (s == 0) col5 = top_val;
-    else col5 = a.back_cum[a.seg[2 * (s - 1) + 1]];
-    while (true) {
-      double *row = a.rows + (int64_t)(a.len[cur] - 1) * 5;
-      row[0] = a.p_j[cur]; row[1] = (double)a.p_i[cur]; row[2] = (double)a.p_c[cur]; row[3] = a.p_q[cur]; row[4] = col5;
-      if (cur == stop) break;
-      col5 = a.back_cum[cur];
-      cur = a.back_id[cur];
-    }
   }
 }
 
@@ -413,12 +363,6 @@ struct __align__(16) PmEntry {
   int32_t pad;
 };
 
-struct __align__(16) BackRec {   // per point result: value it started from, predecessor id
-  double best;
-  int32_t pred;
-  int32_t pad;
-};
-
 struct Dp2LArgs {
   const P2Rec *rec;
   const double *p_j;
@@ -434,8 +378,6 @@ struct Dp2LArgs {
 
 #include "dp2_scan.cuh"
 #include "refine.cuh"
-
-#include "traceback.cuh"
 
 }  // namespace
 
@@ -655,13 +597,9 @@ int dab_enqueue_stage_b_dp(dab_pair *pr) {
   const int64_t cap = rows > 0 ? rows : 1;
   int32_t *dc = pr->counters.as<int32_t>();
   DAB_CUDA(cudaEventRecord(pr->ev[16], st));
+  if (rows > 0) DAB_TRY(dab_ensure(ctx, pr->back2, sizeof(BackRec) * (size_t)(cap + 2)));
   if (rows > 0 && b.scan_dp) {
-    // ---- scan DP + chunked traceback ----
-    const int chunks = (int)cdiv(cap, TB_CHUNK);
     DAB_TRY(dab_ensure(ctx, pr->pm2, sizeof(PmEntry) * (size_t)(rows + 1)));
-    DAB_TRY(dab_ensure(ctx, pr->back2, sizeof(BackRec) * (size_t)(cap + 2)));
-    DAB_TRY(dab_ensure(ctx, pr->lift_up, sizeof(int32_t) * (size_t)(cap + 2 * chunks + 8)));
-    DAB_TRY(dab_ensure(ctx, pr->lift_dep, (size_t)cap + 16));
     Dp2LArgs la;
     la.rec = pr->p2_k.as<P2Rec>(); la.p_j = pr->p2_j.as<double>();
     la.n_points = dc + DC_N_PTS2;
@@ -679,23 +617,7 @@ int dab_enqueue_stage_b_dp(dab_pair *pr) {
       }
       dp2_scan_kernel<<<1, SC_T, sizeof(ScanShared), st>>>(la);
     }
-    DAB_CUDA(cudaEventRecord(pr->ev[18], st));
-    TbArgs tb;
-    tb.back = la.back; tb.n_dev = dc + DC_N_PTS2; tb.result = la.result;
-    tb.exit_id = pr->lift_up.as<int32_t>();
-    tb.entry = tb.exit_id + cap;
-    tb.count = tb.entry + chunks;
-    tb.mark = pr->lift_dep.as<unsigned char>();
-    tb.p_i = pr->p2_i.as<int32_t>(); tb.p_c = pr->p2_c.as<int32_t>(); tb.p_j = la.p_j; tb.p_q = pr->p2_q.as<double>();
-    tb.rows = pr->path2.as<double>(); tb.n_path = dc + DC_N_PATH2; tb.chunks = chunks;
-    DAB_CUDA(cudaMemsetAsync(tb.entry, 0xff, sizeof(int32_t) * (size_t)chunks, st));
-    tb_exit_kernel<<<chunks, TB_THREADS, 0, st>>>(tb);
-    tb_chain_kernel<<<1, 32, 0, st>>>(tb);
-    tb_mark_kernel<<<chunks, TB_THREADS, 0, st>>>(tb);
-    tb_offsets_kernel<<<1, 1024, 0, st>>>(tb);
-    tb_emit_kernel<<<chunks, TB_THREADS, 0, st>>>(tb);
-    ctx->launches += 6;
-    DAB_CUDA(cudaEventRecord(pr->ev[17], st));
+    ctx->launches += 1;
   } else if (rows > 0) {
     // ---- generic tree DP (more than 32 corridors, or a line with non-positive slope) ----
     const int64_t dom = 1 + rows;        // rank domain: 1 + total corridor rows
@@ -704,18 +626,12 @@ int dab_enqueue_stage_b_dp(dab_pair *pr) {
     for (int k = 0; k < L2N; ++k) { lv[k] = cdiv(m > 0 ? m : 1, 32) * 32; loff[k] = tot; tot += lv[k]; m = cdiv(m, 32); }
     DAB_TRY(dab_ensure(ctx, pr->tree2, sizeof(Node2) * (size_t)tot + sizeof(int64_t) * L2N));
     DAB_TRY(dab_ensure(ctx, pr->cache2, sizeof(Cell2) * (size_t)(n_v + 1)));
-    DAB_TRY(dab_ensure(ctx, pr->back2, (sizeof(double) + sizeof(double)) * (size_t)(n_clusters + cap + 2) + 64));
-    DAB_TRY(dab_ensure(ctx, pr->backid2, sizeof(int32_t) * (size_t)(cap + n_clusters + 2)));
-    DAB_TRY(dab_ensure(ctx, pr->len2, sizeof(int32_t) * (size_t)(cap + 1)));
-    DAB_TRY(dab_ensure(ctx, pr->cp2, sizeof(int32_t) * (size_t)(cap + 1)));
-    DAB_TRY(dab_ensure(ctx, pr->seglist, sizeof(int32_t) * (size_t)(2 * (cap / CHECK2 + 16))));
+    DAB_TRY(dab_ensure(ctx, pr->cluster_best2, (sizeof(double) + sizeof(int32_t)) * (size_t)(n_clusters + 1)));
     Node2 *nodes = pr->tree2.as<Node2>();
     int64_t *d_loff = reinterpret_cast<int64_t *>(nodes + tot);
     DAB_CUDA(cudaMemcpyAsync(d_loff, loff, sizeof(int64_t) * L2N, cudaMemcpyHostToDevice, st));
-    double *back_cum = pr->back2.as<double>();
-    double *cb_val = back_cum + (cap + 1);
-    int32_t *back_id = pr->backid2.as<int32_t>();
-    int32_t *cb_id = back_id + (cap + 1);
+    double *cb_val = pr->cluster_best2.as<double>();
+    int32_t *cb_id = reinterpret_cast<int32_t *>(cb_val + (n_clusters + 1));
     int64_t span = tot > n_v ? tot : n_v;
     if (n_clusters > span) span = n_clusters;
     init_dp2_kernel<<<(unsigned)cdiv(span, 256), 256, 0, st>>>(nodes, tot, pr->cache2.as<Cell2>(), n_v, cb_val, cb_id,
@@ -726,21 +642,18 @@ int dab_enqueue_stage_b_dp(dab_pair *pr) {
     da.n_points = dc + DC_N_PTS2;
     for (int k = 0; k < L2N; ++k) da.level[k] = nodes + loff[k];
     da.cache = pr->cache2.as<Cell2>(); da.cb_val = cb_val; da.cb_id = cb_id;
-    da.back_id = back_id; da.len = pr->len2.as<int32_t>(); da.cp = pr->cp2.as<int32_t>();
-    da.back_cum = back_cum; da.result = dc + DC_DP2_END;
+    da.back = pr->back2.as<BackRec>(); da.result = dc + DC_DP2_END;
     dp2_kernel<<<1, 32, 0, st>>>(da);
-    DAB_CUDA(cudaEventRecord(pr->ev[18], st));
-    Trace2Args ta;
-    ta.back_id = back_id; ta.len = da.len; ta.cp = da.cp; ta.result = da.result; ta.back_cum = back_cum;
-    ta.p_i = da.p_i; ta.p_c = da.p_c; ta.p_j = da.p_j; ta.p_q = da.p_q;
-    ta.seg = pr->seglist.as<int32_t>(); ta.rows = pr->path2.as<double>();
-    trace2_kernel<<<1, 256, 0, st>>>(ta);
-    ctx->launches += 3;
-    DAB_CUDA(cudaEventRecord(pr->ev[17], st));
-  } else {
-    DAB_CUDA(cudaEventRecord(pr->ev[18], st));
-    DAB_CUDA(cudaEventRecord(pr->ev[17], st));
+    ctx->launches += 2;
   }
+  DAB_CUDA(cudaEventRecord(pr->ev[18], st));
+  if (rows > 0) {
+    Path2Out out;
+    out.p_i = pr->p2_i.as<int32_t>(); out.p_c = pr->p2_c.as<int32_t>();
+    out.p_j = pr->p2_j.as<double>(); out.p_q = pr->p2_q.as<double>(); out.rows = pr->path2.as<double>();
+    DAB_TRY(dab_enqueue_traceback(pr, pr->back2.as<BackRec>(), dc + DC_N_PTS2, dc + DC_DP2_END, cap, dc + DC_N_PATH2, out));
+  }
+  DAB_CUDA(cudaEventRecord(pr->ev[17], st));
   pr->ev_used[8] = true;
   DAB_CUDA(cudaGetLastError());
   return DAB_OK;

@@ -12,8 +12,10 @@ everywhere), quals in [0.046, 50]
   f1_*            one chain summed by the speculative run sum, one by tree queries, bit-equal sums
   f2_rounding     every add of a stretch of the chain is an exact rounding tie; runs straddle warp batches
   f3_tree         more than 32^3 ranks; predecessors found at each level of the 32-ary tree
-  f4_*            sizes around 32, paths around the 256-point traceback checkpoints, one large set
+  f4_*            sizes around 32, paths of 255 to 513 points, a path that leaves the top's chain, one large set
   f5_limit        the largest video the DP tree takes (2^20 hashed-frame slots), and one frame more
+  f6_*            paths placed on the traceback's chunks of 1024 point ids: predecessors across chunk
+                  boundaries, skipped chunks, an end alone in the last chunk, a late first point, one point
 
 Each F builder returns a dict with i, v, q (int32, int32, float64), Le (video length in frames whose hashed
 frames are 4 * arange), Lv (bound on v for ao.dp1) and what the tests check about it.
@@ -287,9 +289,9 @@ def f4_path(length: int, seed: int = 6):
 
 
 def f4_superseded(seed: int = 7):
-    """Chain M (rows 0..599, ranks 1000 + 2k, qual 1) passes traceback checkpoints 256 and 512 and is the top;
-    then branch B (rows 600..1199, ranks 1201.., qual 2) leaves M at its point 100 and overtakes it.  The path is
-    M[0..100] + B: the checkpoints M wrote are superseded by B's."""
+    """Chain M (rows 0..599, ranks 1000 + 2k, qual 1) is the top for 600 points; then branch B (rows 600..1199,
+    ranks 1201.., qual 2) leaves M at its point 100 and overtakes it.  The path is M[0..100] + B: the back records
+    of M's points 101..599 stay written but are no longer on the path."""
     i = list(range(600)) + list(range(600, 1200))
     r = [1000 + 2 * k for k in range(600)] + [1201 + k for k in range(600)]
     q = [1.0] * 600 + [2.0] * 600
@@ -338,6 +340,39 @@ def f5_limit(over: bool = False, seed: int = 9):
     out["Le"] = Le
     out["Lv"] = 4 * n_sel + 4
     return out
+
+
+TB_CHUNK = 1024                  # point ids per chunk of the traceback
+
+
+def f6_chunks(path_ids, n: int):
+    """n points, one per row, so a point's id is its row.  The points at path_ids (ascending) form the path: ranks
+    R, R + 1, ..., qual 1.  Every other point has qual 0.05 and cannot be a predecessor of a path point: before the
+    first path point the ranks lie above the path's, after it below, and both kinds fall with the id, so each noise
+    point chains from the seed (cum 0.05) and the path's cums 1, 2, ... win every comparison."""
+    path_ids = sorted(path_ids)
+    assert path_ids and path_ids[-1] < n
+    on_path = set(path_ids)
+    n_high = sum(1 for p in range(path_ids[0]) if p not in on_path)
+    n_low = n - len(path_ids) - n_high
+    R, L = n_low, len(path_ids)
+    high, low = iter(range(R + L + n_high - 1, R + L - 1, -1)), iter(range(R - 1, -1, -1))
+    r, q, k = [], [], 0
+    for p in range(n):
+        if p in on_path:
+            r.append(R + k); q.append(1.0); k += 1
+        else:
+            r.append(next(high) if p < path_ids[0] else next(low)); q.append(0.05)
+    return _case(np.arange(n), r, q, R + L + n_high, path_ids=np.array(path_ids))
+
+
+F6_CASES = {
+    "f6_across": lambda: f6_chunks([5, 700, 1023, 1024, 1500, 2047, 2048, 2600], 3000),   # preds 1023 -> 1024, 2047 -> 2048
+    "f6_skip": lambda: f6_chunks([10, 500, 4200, 4201, 6000], 6200),                    # chunks 1-3 and 6 not visited
+    "f6_end_alone": lambda: f6_chunks([3, 1030, 2000, 2048], 2049),                      # the last chunk is the end point
+    "f6_late_start": lambda: f6_chunks([1024, 1025, 2100, 3000], 3100),                  # nothing on chunk 0
+    "f6_single": lambda: f6_chunks([1700], 2500),
+}
 
 
 def literal_small(case) -> bool:

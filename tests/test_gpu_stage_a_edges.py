@@ -6,7 +6,7 @@ a grow-and-retry loop is run on them: a fresh pair, a reused pair, the row-shard
 and the public API.  Bars of test_stage_a_golden: (i, v) identical, quals rel 1e-12, pass-1 path identical, and
 the gate's candidate count equal to the oracle's.
 
-DP 1 sets F1-F5 are imported into a pair whose video has energy 1.0 everywhere (hashed frames 4 * arange):
+DP 1 sets F1-F6 are imported into a pair whose video has energy 1.0 everywhere (hashed frames 4 * arange):
 the pass-1 path must equal the oracle's.
 """
 import numpy as np
@@ -234,6 +234,7 @@ def _f_cases():
            ("f4_superseded", sc.f4_superseded), ("f4_large", sc.f4_large), ("f5_limit", sc.f5_limit)]
     out += [(f"f4_n{n}", (lambda n=n: sc.f4_small(n))) for n in sc.F4_SIZES]
     out += [(f"f4_path{n}", (lambda n=n: sc.f4_path(n))) for n in sc.F4_PATHS]
+    out += list(sc.F6_CASES.items())
     return out
 
 

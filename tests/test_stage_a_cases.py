@@ -24,6 +24,7 @@ def _small_cases():
         out[f"f4_n{n}"] = sc.f4_small(n)
     for n in sc.F4_PATHS:
         out[f"f4_path{n}"] = sc.f4_path(n)
+    out.update((name, build()) for name, build in sc.F6_CASES.items())
     return out
 
 
@@ -163,6 +164,29 @@ def test_f4_sizes_and_paths(oracle_lib):
     case = SMALL["f4_superseded"]
     px, pv, _, _ = _dp1(case)
     assert len(px) == case["want_len"] and px[100] == 100 and px[101] == 600
+
+
+def test_f6_paths_on_traceback_chunks(oracle_lib):
+    """The oracle's path is each case's path_ids (a point's id is its row), placed on the chunks as named."""
+    paths = {}
+    for name in sc.F6_CASES:
+        case = SMALL[name]
+        assert np.array_equal(case["i"], np.arange(len(case["i"])))
+        px, _, _, back = _dp1(case)
+        assert px.tolist() == case["path_ids"].tolist(), name
+        assert back[px[0]] == -1 and back[px[1:]].tolist() == px[:-1].tolist(), name
+        paths[name] = px.tolist()
+    c = sc.TB_CHUNK
+    p = paths["f6_across"]
+    for k in (c, 2 * c):
+        assert k in p and p[p.index(k) - 1] == k - 1
+    chunks = {x // c for x in paths["f6_skip"]}
+    assert {1, 2, 3} & chunks == set() and min(chunks) == 0 and max(chunks) > 3
+    assert (len(SMALL["f6_skip"]["i"]) - 1) // c not in chunks
+    p, n = paths["f6_end_alone"], len(SMALL["f6_end_alone"]["i"])
+    assert p[-1] == n - 1 and (n - 1) % c == 0 and p[-2] // c < p[-1] // c
+    assert paths["f6_late_start"][0] >= c
+    assert len(paths["f6_single"]) == 1
 
 
 def test_f4_large_shape(oracle_lib):
