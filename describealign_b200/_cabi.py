@@ -31,6 +31,7 @@ EXPORTS = [
     "dab_engine_create", "dab_engine_destroy", "dab_engine_submit", "dab_engine_next", "dab_engine_submit_b",
     "dab_engine_release", "dab_engine_slot_error", "dab_engine_slot_pair", "dab_engine_counters",
     "dab_host_continuity_error", "dab_host_continuity_error_f64", "dab_host_compress_path", "dab_host_lp_assemble", "dab_host_line_clusters", "dab_host_stretch_plan",
+    "dab_index_build", "dab_index_free", "dab_index_info", "dab_pair_stage_a_against",
     "dab_pcm_reader_open", "dab_pcm_reader_progress", "dab_pcm_reader_wait", "dab_pcm_reader_close", "dab_pcm_reader_copy_to_host", "dab_stretch_best_jumps",
 ]
 
@@ -163,6 +164,10 @@ def load() -> ctypes.CDLL:
     lib.dab_pair_feature_lens.argtypes = [vp, i32, ctypes.POINTER(i64 * 5)]
     lib.dab_pair_get_features.argtypes = [vp, i32, vp, vp, vp, vp, vp]
     lib.dab_pair_stage_a.argtypes = [vp, ctypes.POINTER(i64), ctypes.POINTER(i64)]
+    lib.dab_index_build.argtypes = [vp, ctypes.POINTER(vp)]
+    lib.dab_index_free.argtypes = [vp]
+    lib.dab_index_info.argtypes = [vp, ctypes.POINTER(i64 * 4)]
+    lib.dab_pair_stage_a_against.argtypes = [vp, vp, ctypes.POINTER(i64), ctypes.POINTER(i64)]
     lib.dab_pair_get_path1.argtypes = [vp, vp, vp]
     lib.dab_pair_get_points1.argtypes = [vp, vp, vp, vp]
     lib.dab_pair_stage_a_match.argtypes = [vp, i64, i64, ctypes.POINTER(i64)]
@@ -317,6 +322,35 @@ class Context:
             pass
 
 
+class Index:
+    """The video side of stage A of one video track (dab_index), built from `pair`'s VIDEO track and then
+    read-only: any number of pairs on their own streams and threads run stage_a_against it at once."""
+
+    def __init__(self, pair: "Pair"):
+        self.ctx = pair.ctx
+        self.lib = pair.lib
+        h = ctypes.c_void_p()
+        self.ctx.check(self.lib.dab_index_build(pair.handle, ctypes.byref(h)))
+        self.handle = h
+
+    def info(self) -> dict:
+        out = (ctypes.c_int64 * 4)()
+        self.ctx.check(self.lib.dab_index_info(self.handle, ctypes.byref(out)))
+        return dict(n_video_frames=out[0], n_video_selected=out[1], n_table_entries=out[2], users=out[3])
+
+    def free(self):
+        """Raises DabError (and frees nothing) while a stage_a_against call on the index is running."""
+        if getattr(self, "handle", None):
+            self.ctx.check(self.lib.dab_index_free(self.handle))
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
 class Pair:
     """Device-resident state of one (video, description) pair (dab_pair)."""
 
@@ -397,6 +431,15 @@ class Pair:
     def stage_a(self):
         npts, npath = ctypes.c_int64(), ctypes.c_int64()
         self.ctx.check(self.lib.dab_pair_stage_a(self.handle, ctypes.byref(npts), ctypes.byref(npath)))
+        self._keep.clear()
+        self.n_points1, self.n_path1 = npts.value, npath.value
+        return npts.value, npath.value
+
+    def stage_a_against(self, index: "Index"):
+        """Stage A of this pair's description track (AUDIO) against a shared video index: only the counts
+        come back (path1() copies the path on request).  Returns (n_points, n_path)."""
+        npts, npath = ctypes.c_int64(), ctypes.c_int64()
+        self.ctx.check(self.lib.dab_pair_stage_a_against(self.handle, index.handle, ctypes.byref(npts), ctypes.byref(npath)))
         self._keep.clear()
         self.n_points1, self.n_path1 = npts.value, npath.value
         return npts.value, npath.value

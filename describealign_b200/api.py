@@ -110,6 +110,15 @@ def _interleaved(arr: np.ndarray) -> np.ndarray:
     return np.ascontiguousarray(arr.T)
 
 
+def host_pcm(p) -> np.ndarray:
+    """Host PCM as Pair.set_pcm takes it: interleaved int16 (S, ch) stays, the reference's float16 (ch, S)
+    array is interleaved."""
+    p = np.asarray(p)
+    if p.dtype == np.float16 and p.ndim == 2 and p.shape[0] in (1, 2) and p.shape[1] > 2:
+        return _interleaved(p)
+    return p
+
+
 def track_features(arr: np.ndarray):
     """All five feature vectors of one track from one pass over the PCM on the GPU.
     The reference calls three functions on the same array; the results are cached per
@@ -189,12 +198,7 @@ class AlignJob:
     # -- inputs ---------------------------------------------------------------------------
     def load_pcm(self, video_pcm, audio_pcm):
         """Host PCM: interleaved int16 (S, ch), or the reference's float16 (ch, S) arrays."""
-        def prep(p):
-            p = np.asarray(p)
-            if p.dtype == np.float16 and p.ndim == 2 and p.shape[0] in (1, 2) and p.shape[1] > 2:
-                return _interleaved(p)
-            return p
-        v, a = prep(video_pcm), prep(audio_pcm)
+        v, a = host_pcm(video_pcm), host_pcm(audio_pcm)
         self._timed("set_pcm", self.pair.set_pcm, VIDEO, v)
         self._timed("set_pcm", self.pair.set_pcm, AUDIO, a)
         self.h2d_bytes += v.nbytes + a.nbytes

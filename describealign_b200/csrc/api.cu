@@ -458,6 +458,10 @@ extern "C" {
 
 static int export_points1(dab_pair *pr, int32_t *i_audio, int32_t *v_video, double *qual, int dst_on_device) {
   dab_ctx *ctx = pr->ctx;
+  if (pr->points_from_index) {
+    dab_set_err(ctx, "export_points1: the points of stage_a_against are ranks into the index's hashed frames, not this pair's");
+    return DAB_E_STATE;
+  }
   StreamScope scope__(pr->stream);
   ApiTimer timer__(&pr->api_us[3]);
   DAB_CUDA(cudaSetDevice(ctx->device));
@@ -488,6 +492,87 @@ int dab_pair_get_points1(dab_pair *pr, int32_t *i_audio, int32_t *v_video, doubl
 int dab_pair_export_points1(dab_pair *pr, int32_t *i_audio, int32_t *v_video, double *qual, int dst_on_device) {
   if (!pr) return DAB_E_ARG;
   return export_points1(pr, i_audio, v_video, qual, dst_on_device);
+}
+
+static void index_destroy(dab_index *ix) {
+  DevBuf *bs[] = {&ix->V.ms, &ix->V.nrm, &ix->V.pack, &ix->V.code, &ix->V.nq_flag, &ix->V.nq_list,
+                  &ix->tbl_start, &ix->tbl_items, &ix->v_rec, &ix->counters};
+  for (DevBuf *b : bs) free_buf(*b);
+  if (ix->ready) cudaEventDestroy(ix->ready);
+  delete ix;
+}
+
+int dab_index_build(dab_pair *src, dab_index **out) {
+  if (!src || !out) return DAB_E_ARG;
+  *out = nullptr;
+  dab_ctx *ctx = src->ctx;
+  StreamScope scope__(src->stream);
+  const Track &S = src->trk[DAB_TRACK_VIDEO];
+  if (!S.have_features) { dab_set_err(ctx, "index_build: the pair's video track has no features"); return DAB_E_STATE; }
+  if ((S.Le < S.L ? S.Le : S.L) < 2 * DAB_WIN) { dab_set_err(ctx, "index_build: track shorter than 82 frames"); return DAB_E_TOO_SHORT; }
+  DAB_CUDA(cudaSetDevice(ctx->device));
+  dab_index *ix = new (std::nothrow) dab_index();
+  if (!ix) return DAB_E_CUDA;
+  ix->ctx = ctx;
+  int rc = DAB_OK;
+  const cudaError_t e = cudaEventCreateWithFlags(&ix->ready, cudaEventDisableTiming);
+  if (e != cudaSuccess) { dab_set_err(ctx, std::string("index_build: ") + cudaGetErrorString(e)); rc = DAB_E_CUDA; }
+  if (rc == DAB_OK) rc = dab_build_index(src, ix);
+  if (rc != DAB_OK) {
+    dab_wait_stream(src->stream);
+    index_destroy(ix);
+    return rc;
+  }
+  *out = ix;
+  return DAB_OK;
+}
+
+int dab_index_free(dab_index *ix) {
+  if (!ix) return DAB_OK;
+  int idle = 0;
+  if (!ix->users.compare_exchange_strong(idle, -1)) {
+    dab_set_err(ix->ctx, "index_free: " + std::to_string(idle) + " stage_a_against call(s) still running against this index");
+    return DAB_E_STATE;
+  }
+  cudaSetDevice(ix->ctx->device);
+  index_destroy(ix);
+  return DAB_OK;
+}
+
+int dab_index_info(const dab_index *ix, int64_t out[4]) {
+  if (!ix || !out) return DAB_E_ARG;
+  out[0] = ix->V.L; out[1] = ix->n_vsel; out[2] = ix->n_entries; out[3] = ix->users.load();
+  return DAB_OK;
+}
+
+int dab_pair_stage_a_against(dab_pair *pr, const dab_index *ix, int64_t *n_points, int64_t *n_path) {
+  if (!pr || !ix) return DAB_E_ARG;
+  dab_ctx *ctx = pr->ctx;
+  StreamScope scope__(pr->stream);
+  ApiTimer timer__(&pr->api_us[1]);
+  if (ix->ctx->device != ctx->device) { dab_set_err(ctx, "stage_a_against: the index lives on another device"); return DAB_E_ARG; }
+  const Track &A = pr->trk[DAB_TRACK_AUDIO];
+  if (!A.have_features) { dab_set_err(ctx, "stage_a_against: features of the description track are required first"); return DAB_E_STATE; }
+  if ((A.Le < A.L ? A.Le : A.L) < 2 * DAB_WIN) { dab_set_err(ctx, "stage_a_against: track shorter than 82 frames"); return DAB_E_TOO_SHORT; }
+  int u = ix->users.load();
+  do {
+    if (u < 0) { dab_set_err(ctx, "stage_a_against: the index is being freed"); return DAB_E_STATE; }
+  } while (!ix->users.compare_exchange_weak(u, u + 1));
+  struct Release {
+    const dab_index *ix;
+    ~Release() { ix->users.fetch_sub(1); }
+  } release__{ix};
+  DAB_CUDA(cudaSetDevice(ctx->device));
+  int rc = DAB_E_CAPACITY;
+  for (int attempt = 0; attempt < DAB_STAGE_A_ATTEMPTS && rc == DAB_E_CAPACITY; ++attempt) {
+    DAB_TRY(dab_enqueue_stage_a_against(pr, ix));
+    DAB_CUDA(dab_wait_stream(pr->stream));
+    rc = dab_collect_stage_a_against(pr, ix);
+  }
+  DAB_TRY(rc);
+  if (n_points) *n_points = pr->n_points1;
+  if (n_path) *n_path = pr->n_path1;
+  return DAB_OK;
 }
 
 int dab_pair_stage_a_match(dab_pair *pr, int64_t row_lo, int64_t row_hi, int64_t *n_points) {

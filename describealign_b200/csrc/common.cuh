@@ -99,6 +99,7 @@ struct dab_pair {
   int64_t n_points1 = 0, n_path1 = 0;
   int64_t cap_entries = 0, cap_cand = 0, cap_points1 = 0;   // capacities of device-sized buffers (grown on overflow)
   bool matched = false;        // tables / hashed-frame list of the current features are built
+  bool points_from_index = false;   // the pass-1 points are ranks into a shared index's hashed-frame list
   // stage B
   DevBuf a_scaled, v_scaled;   // f32 (n,3)
   DevBuf corridors;            // dab_corridor[]
@@ -124,6 +125,20 @@ struct dab_pair {
   // host time spent inside the library's calls for this pair since the last set_pcm (microseconds):
   // [0] set_pcm / set_features, [1] stage A, [2] stage B, [3] get_* copies
   int64_t api_us[4] = {0, 0, 0, 0};
+};
+
+// The video side of the match stage, built once per video and then only read: any number of pairs, each on its
+// own stream, run their description track against it (dab_pair_stage_a_against).  V holds the prep buffers (ms,
+// nrm, digit packs and codes, not-quiet flags and the hashed-frame list) but no features.
+struct dab_index {
+  dab_ctx *ctx = nullptr;           // the context of the pair it was built from (device, error messages)
+  Track V;
+  DevBuf tbl_start, tbl_items;      // hash tables, sized when the index is built
+  DevBuf v_rec;                     // records of the hashed frames (gate)
+  DevBuf counters;                  // the build's device counts
+  int64_t n_vsel = 0, n_entries = 0, cap_entries = 0;
+  cudaEvent_t ready = nullptr;      // recorded after the last command of the build; every user's stream waits on it
+  mutable std::atomic<int> users{0};   // stage-A calls running against the index; -1 once it is being freed
 };
 
 inline void dab_set_err(dab_ctx *ctx, const std::string &msg) {
@@ -222,6 +237,10 @@ int dab_check_stage_a_inputs(dab_pair *pr, const char *who);
 int dab_enqueue_stage_a(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp);
 int dab_enqueue_stage_a_dp(dab_pair *pr);      // DP 1 + traceback over the pair's points
 int dab_collect_stage_a(dab_pair *pr, bool with_dp);
+// shared video index: build (synchronous: the tables' capacity is settled here) and the match stage against it
+int dab_build_index(dab_pair *src, dab_index *ix);
+int dab_enqueue_stage_a_against(dab_pair *pr, const dab_index *ix);
+int dab_collect_stage_a_against(dab_pair *pr, const dab_index *ix);
 void dab_collect_stage_a_dp(dab_pair *pr);
 int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *v_video, const double *qual,
                            int64_t n, int src_on_device);

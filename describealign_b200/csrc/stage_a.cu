@@ -1014,45 +1014,46 @@ static __global__ void check_capacity_kernel(int32_t *dc, int word, int need_wor
   if ((int64_t)dc[word] > cap) { dc[word] = 0; atomicOr(&dc[DC_OVERFLOW], bit); }
 }
 
-static int prep_track(dab_pair *pr, int track) {
+// Prep of one track's features `in` into the stage-A buffers of `out` (the same track, or a video index).
+static int prep_track(dab_pair *pr, const Track &in, Track &out, bool is_video) {
   dab_ctx *ctx = pr->ctx;
-  Track &tk = pr->trk[track];
+  const Track &tk = in;
   const int64_t Lmax = tk.Le > tk.L ? tk.Le : tk.L;
   const int64_t Lmin = tk.Le < tk.L ? tk.Le : tk.L;
   const int64_t nc = Lmax - 40;     // stride of the code arrays (energy may have one more)
-  tk.n_codes = Lmin - 40;
-  DAB_TRY(dab_ensure(ctx, tk.ms, sizeof(double) * (size_t)(5 * Lmax)));
-  DAB_TRY(dab_ensure(ctx, tk.nrm, sizeof(double) * (size_t)(3 * nc)));
-  DAB_TRY(dab_ensure(ctx, tk.pack, sizeof(uint32_t) * (size_t)(5 * nc)));
-  DAB_TRY(dab_ensure(ctx, tk.code, sizeof(int32_t) * (size_t)(5 * nc)));
+  out.n_codes = Lmin - 40;
+  DAB_TRY(dab_ensure(ctx, out.ms, sizeof(double) * (size_t)(5 * Lmax)));
+  DAB_TRY(dab_ensure(ctx, out.nrm, sizeof(double) * (size_t)(3 * nc)));
+  DAB_TRY(dab_ensure(ctx, out.pack, sizeof(uint32_t) * (size_t)(5 * nc)));
+  DAB_TRY(dab_ensure(ctx, out.code, sizeof(int32_t) * (size_t)(5 * nc)));
   PrepArgs pa;
   pa.f32[0] = tk.energy.as<float>(); pa.f32[1] = tk.zc.as<float>();
   pa.f32[2] = tk.b0.as<float>(); pa.f32[3] = tk.b1.as<float>();
   pa.f64 = tk.b2.as<double>();
   pa.len[0] = tk.Le; pa.len[1] = pa.len[2] = pa.len[3] = pa.len[4] = tk.L;
-  pa.Lp = Lmin; pa.ms = tk.ms.as<double>(); pa.stride = Lmax;
+  pa.Lp = Lmin; pa.ms = out.ms.as<double>(); pa.stride = Lmax;
   dim3 g1((unsigned)cdiv(Lmax, 256 * MS_TILES), 5);
   meansub_kernel<<<g1, 256, 0, pr->stream>>>(pa);
   CodeArgs ca;
-  ca.ms = tk.ms.as<double>(); ca.stride = Lmax;
+  ca.ms = out.ms.as<double>(); ca.stride = Lmax;
   for (int f = 0; f < 5; ++f) ca.len[f] = pa.len[f];
-  ca.nrm = tk.nrm.as<double>(); ca.nstride = nc;
-  ca.pack = tk.pack.as<uint32_t>(); ca.code = tk.code.as<int32_t>();
-  ca.is_video = track == DAB_TRACK_VIDEO;
+  ca.nrm = out.nrm.as<double>(); ca.nstride = nc;
+  ca.pack = out.pack.as<uint32_t>(); ca.code = out.code.as<int32_t>();
+  ca.is_video = is_video;
   dim3 g2((unsigned)cdiv(nc, 256), 5);
   norm_codes_kernel<<<g2, 256, 0, pr->stream>>>(ca);
   ctx->launches += 2;
   // not-quiet selection: t < len(energy) - 41 with energy[t] > .5
   const int64_t nqn = tk.Le - 41;
-  DAB_TRY(dab_ensure(ctx, tk.nq_flag, sizeof(int32_t) * (size_t)(2 * (nqn + 2))));
-  DAB_TRY(dab_ensure(ctx, tk.nq_list, sizeof(int32_t) * (size_t)(nqn + 2)));
-  int32_t *flag = tk.nq_flag.as<int32_t>();
+  DAB_TRY(dab_ensure(ctx, out.nq_flag, sizeof(int32_t) * (size_t)(2 * (nqn + 2))));
+  DAB_TRY(dab_ensure(ctx, out.nq_list, sizeof(int32_t) * (size_t)(nqn + 2)));
+  int32_t *flag = out.nq_flag.as<int32_t>();
   int32_t *off = flag + (nqn + 1);
   notquiet_flag_kernel<<<(unsigned)cdiv(nqn, 256), 256, 0, pr->stream>>>(tk.have_gate ? tk.gate.as<float>() : tk.energy.as<float>(), nqn, flag);
   ctx->launches += 1;
   DAB_TRY(dab_exclusive_scan(pr, flag, off, nqn));
-  compact_kernel<<<(unsigned)cdiv(nqn, 256), 256, 0, pr->stream>>>(flag, off, nqn, track == DAB_TRACK_VIDEO ? 4 : 1,
-                                                                  tk.nq_list.as<int32_t>());
+  compact_kernel<<<(unsigned)cdiv(nqn, 256), 256, 0, pr->stream>>>(flag, off, nqn, is_video ? 4 : 1,
+                                                                  out.nq_list.as<int32_t>());
   ctx->launches += 1;
   DAB_CUDA(cudaGetLastError());
   return DAB_OK;
@@ -1076,49 +1077,40 @@ static int ensure_hann(dab_ctx *ctx) {
 // Capacities of the buffers whose fill level only the device knows (table entries, candidates).  They
 // start from what pairs of this size normally need and double when a run overflows (the overflow bit
 // comes back with the counts; the stage is then run again - rare, and only ever during the first pairs).
+static int64_t first_entries_cap(const Track &V) {
+  return 5 * 16 * ((V.Le - 41 + 3) / 4 + 1) + 4096;     // ~10 expanded entries per frame and table (SURVEY.md D)
+}
+static int64_t first_cand_cap(const Track &A) {
+  return 2 * (A.Le - 41) + 4096;                         // < 1 candidate per query on matching tracks
+}
 static void default_caps(dab_pair *pr) {
-  Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
-  const int64_t vsel_ub = (V.Le - 41 + 3) / 4 + 1;
-  const int64_t q_ub = A.Le - 41;
-  const int64_t want_e = 5 * 16 * vsel_ub + 4096;        // ~10 expanded entries per frame and table (SURVEY.md D)
-  const int64_t want_c = 2 * q_ub + 4096;                // < 1 candidate per query on matching tracks
+  const int64_t want_e = first_entries_cap(pr->trk[DAB_TRACK_VIDEO]);
+  const int64_t want_c = first_cand_cap(pr->trk[DAB_TRACK_AUDIO]);
   if (pr->cap_entries < want_e) pr->cap_entries = want_e;
   if (pr->cap_cand < want_c) pr->cap_cand = want_c;
 }
 
-// ---- match stage, enqueued without a host round trip: prep, codes, lists, tables, gate, scoring ----
-static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
+// The video side of the match stage as the gate, scoring and DP 1 read it: the video track's prep buffers, its
+// tables and the records of its hashed frames.  Either the pair's own (enqueue_match) or a shared index's.
+struct VideoSide {
+  const Track *V;
+  const int32_t *start, *items;
+  const uint4 *rec;
+};
+
+static int64_t video_sel_ub(const Track &V) { return (V.Le - 41 + 3) / 4 + 1; }
+
+// tables over the hashed video frames (dc[DC_N_VSEL] of them) into start / items; the pair's table scratch counts
+static int enqueue_tables(dab_pair *pr, const Track &V, int32_t *dc, int64_t cap_e, DevBuf &tbl_start, DevBuf &tbl_items) {
   dab_ctx *ctx = pr->ctx;
-  DAB_TRY(ensure_hann(ctx));
-  Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
   cudaStream_t st = pr->stream;
-  pr->n_points1 = pr->n_path1 = 0;
-  default_caps(pr);
-  const int64_t v_nq = V.Le - 41, a_nq = A.Le - 41;
-  const int64_t vsel_ub = (v_nq + 3) / 4 + 1, q_ub = a_nq > 0 ? a_nq : 1;
-  const int64_t cap_e = pr->cap_entries, cap_c = pr->cap_cand;
-
-  DAB_TRY(dab_ensure(ctx, pr->counters, sizeof(int32_t) * DC_WORDS));
-  int32_t *dc = pr->counters.as<int32_t>();
-  DAB_CUDA(cudaEventRecord(pr->ev[4], st));
-  DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, st));
-  DAB_TRY(prep_track(pr, DAB_TRACK_VIDEO));
-  DAB_TRY(prep_track(pr, DAB_TRACK_AUDIO));
-  counts_lists_kernel<<<1, 32, 0, st>>>(dc, V.nq_flag.as<int32_t>() + (v_nq + 1), v_nq, A.nq_flag.as<int32_t>() + (a_nq + 1), a_nq,
-                                        row_lo, row_hi);
-  ctx->launches += 1;
-  DAB_CUDA(cudaEventRecord(pr->ev[5], st));
-  pr->stats.n_video_frames = V.L; pr->stats.n_audio_frames = A.L;
-
-  // ---- tables ----
+  const int64_t vsel_ub = video_sel_ub(V);
   const int64_t nslots = 5LL * DAB_NCODE;
-  DAB_TRY(dab_ensure(ctx, pr->tbl_count, sizeof(int32_t) * (size_t)(nslots + 1)));
-  DAB_TRY(dab_ensure(ctx, pr->tbl_start, sizeof(int32_t) * (size_t)(nslots + 2)));
-  DAB_TRY(dab_ensure(ctx, pr->tbl_items, sizeof(int32_t) * (size_t)(cap_e + 1)));
-  DAB_CUDA(cudaMemsetAsync(pr->tbl_count.p, 0, sizeof(int32_t) * (size_t)(nslots + 1), st));
   const int64_t v_nstride = (V.Le > V.L ? V.Le : V.L) - 40;
-  const int64_t a_nstride = (A.Le > A.L ? A.Le : A.L) - 40;
-  DAB_CUDA(cudaEventRecord(pr->ev[6], st));
+  DAB_TRY(dab_ensure(ctx, pr->tbl_count, sizeof(int32_t) * (size_t)(nslots + 1)));
+  DAB_TRY(dab_ensure(ctx, tbl_start, sizeof(int32_t) * (size_t)(nslots + 2)));
+  DAB_TRY(dab_ensure(ctx, tbl_items, sizeof(int32_t) * (size_t)(cap_e + 1)));
+  DAB_CUDA(cudaMemsetAsync(pr->tbl_count.p, 0, sizeof(int32_t) * (size_t)(nslots + 1), st));
   dim3 gt((unsigned)cdiv(vsel_ub, 128), 5);
   DAB_TRY(dab_ensure(ctx, pr->tbl_ecount, sizeof(int32_t) * (size_t)(2 * (5 * vsel_ub + 2))));
   DAB_TRY(dab_ensure(ctx, pr->tbl_pos, sizeof(int32_t) * (size_t)(cap_e + 1)));
@@ -1128,12 +1120,35 @@ static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
   check_capacity_kernel<<<1, 32, 0, st>>>(dc, DC_N_ENTRIES, DC_NEED_ENTRIES, cap_e, DAB_OVF_ENTRIES);
   table_kernel<false><<<gt, 128, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, vsel_ub, ebase,
                                           pr->tbl_pos.as<int32_t>(), pr->tbl_count.as<int32_t>(), nullptr, nullptr, cap_e);
-  DAB_TRY(dab_exclusive_scan(pr, pr->tbl_count.as<int32_t>(), pr->tbl_start.as<int32_t>(), nslots));
+  DAB_TRY(dab_exclusive_scan(pr, pr->tbl_count.as<int32_t>(), tbl_start.as<int32_t>(), nslots));
   table_kernel<true><<<gt, 128, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, vsel_ub, ebase,
-                                         pr->tbl_pos.as<int32_t>(), pr->tbl_count.as<int32_t>(), pr->tbl_start.as<int32_t>(),
-                                         pr->tbl_items.as<int32_t>(), cap_e);
+                                         pr->tbl_pos.as<int32_t>(), pr->tbl_count.as<int32_t>(), tbl_start.as<int32_t>(),
+                                         tbl_items.as<int32_t>(), cap_e);
   ctx->launches += 4;
-  DAB_CUDA(cudaEventRecord(pr->ev[7], st));
+  return DAB_OK;
+}
+
+static int enqueue_video_records(dab_pair *pr, const Track &V, const int32_t *dc, DevBuf &rec) {
+  dab_ctx *ctx = pr->ctx;
+  const int64_t vsel_ub = video_sel_ub(V);
+  const int64_t v_nstride = (V.Le > V.L ? V.Le : V.L) - 40;
+  DAB_TRY(dab_ensure(ctx, rec, sizeof(uint4) * 2 * (size_t)(vsel_ub + 1)));
+  video_records_kernel<<<(unsigned)cdiv(vsel_ub, 256), 256, 0, pr->stream>>>(V.pack.as<uint32_t>(), v_nstride,
+                                                                            V.nq_list.as<int32_t>(), dc, rec.as<uint4>());
+  ctx->launches += 1;
+  return DAB_OK;
+}
+
+// gate + scoring + compaction of the pair's audio queries against `vs`: the points go to pr->pt_*
+static int enqueue_gate_score(dab_pair *pr, const VideoSide &vs, int32_t *dc) {
+  dab_ctx *ctx = pr->ctx;
+  const Track &V = *vs.V, &A = pr->trk[DAB_TRACK_AUDIO];
+  cudaStream_t st = pr->stream;
+  const int64_t a_nq = A.Le - 41;
+  const int64_t q_ub = a_nq > 0 ? a_nq : 1;
+  const int64_t cap_c = pr->cap_cand;
+  const int64_t v_nstride = (V.Le > V.L ? V.Le : V.L) - 40;
+  const int64_t a_nstride = (A.Le > A.L ? A.Le : A.L) - 40;
 
   // ---- gate: count, scan, fill ----
   DAB_TRY(dab_ensure(ctx, pr->row_count, sizeof(int32_t) * (size_t)(q_ub + 2)));
@@ -1144,12 +1159,8 @@ static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
   GateArgs ga;
   ga.a_code = A.code.as<int32_t>(); ga.a_pack = A.pack.as<uint32_t>(); ga.a_nstride = a_nstride;
   ga.a_list = A.nq_list.as<int32_t>(); ga.dc = dc; ga.q_cap = q_ub;
-  DAB_TRY(dab_ensure(ctx, pr->v_rec, sizeof(uint4) * 2 * (size_t)(vsel_ub + 1)));
-  video_records_kernel<<<(unsigned)cdiv(vsel_ub, 256), 256, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc,
-                                                                    pr->v_rec.as<uint4>());
-  ctx->launches += 1;
-  ga.v_rec = pr->v_rec.as<uint4>();
-  ga.start = pr->tbl_start.as<int32_t>(); ga.items = pr->tbl_items.as<int32_t>();
+  ga.v_rec = vs.rec;
+  ga.start = vs.start; ga.items = vs.items;
   ga.row_count = pr->row_count.as<int32_t>(); ga.row_off = pr->row_off.as<int32_t>();
   ga.cand_tmp = pr->cand_tmp.as<int32_t>(); ga.cand_s = pr->cand_s.as<int32_t>(); ga.cand_i = pr->cand_i.as<int32_t>();
   ga.cand_cap = cap_c;
@@ -1199,20 +1210,50 @@ static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
       pr->pt_q.as<double>());
   ctx->launches += 2;
   DAB_CUDA(cudaEventRecord(pr->ev[11], st));
-  for (int s = 2; s <= 5; ++s) pr->ev_used[s] = true;
   pr->cap_points1 = cap_c;
+  return DAB_OK;
+}
+
+// ---- match stage, enqueued without a host round trip: prep, codes, lists, tables, gate, scoring ----
+static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
+  dab_ctx *ctx = pr->ctx;
+  DAB_TRY(ensure_hann(ctx));
+  Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
+  cudaStream_t st = pr->stream;
+  pr->n_points1 = pr->n_path1 = 0;
+  pr->points_from_index = false;
+  default_caps(pr);
+  const int64_t v_nq = V.Le - 41, a_nq = A.Le - 41;
+
+  DAB_TRY(dab_ensure(ctx, pr->counters, sizeof(int32_t) * DC_WORDS));
+  int32_t *dc = pr->counters.as<int32_t>();
+  DAB_CUDA(cudaEventRecord(pr->ev[4], st));
+  DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, st));
+  DAB_TRY(prep_track(pr, V, V, true));
+  DAB_TRY(prep_track(pr, A, A, false));
+  counts_lists_kernel<<<1, 32, 0, st>>>(dc, V.nq_flag.as<int32_t>() + (v_nq + 1), v_nq, A.nq_flag.as<int32_t>() + (a_nq + 1), a_nq,
+                                        row_lo, row_hi);
+  ctx->launches += 1;
+  DAB_CUDA(cudaEventRecord(pr->ev[5], st));
+  pr->stats.n_video_frames = V.L; pr->stats.n_audio_frames = A.L;
+
+  DAB_CUDA(cudaEventRecord(pr->ev[6], st));
+  DAB_TRY(enqueue_tables(pr, V, dc, pr->cap_entries, pr->tbl_start, pr->tbl_items));
+  DAB_CUDA(cudaEventRecord(pr->ev[7], st));
+  DAB_TRY(enqueue_video_records(pr, V, dc, pr->v_rec));
+  DAB_TRY(enqueue_gate_score(pr, VideoSide{&V, pr->tbl_start.as<int32_t>(), pr->tbl_items.as<int32_t>(), pr->v_rec.as<uint4>()}, dc));
+  for (int s = 2; s <= 5; ++s) pr->ev_used[s] = true;
   DAB_CUDA(cudaGetLastError());
   return DAB_OK;
 }
 
 // ---- DP #1 + traceback over pr->pt_* (dc[DC_N_PTS1] points sorted by (audio frame, video rank)) ----
-int dab_enqueue_stage_a_dp(dab_pair *pr) {
+static int enqueue_dp1(dab_pair *pr, const Track &V) {
   dab_ctx *ctx = pr->ctx;
-  Track &V = pr->trk[DAB_TRACK_VIDEO];
   cudaStream_t st = pr->stream;
   int32_t *dc = pr->counters.as<int32_t>();
   const int64_t cap_p = pr->cap_points1 > 0 ? pr->cap_points1 : 1;
-  const int64_t vsel_ub = (V.Le - 41 + 3) / 4 + 1;
+  const int64_t vsel_ub = video_sel_ub(V);
   DAB_CUDA(cudaEventRecord(pr->ev[12], st));
   if (vsel_ub > (1LL << (5 * DP_LEVELS))) { dab_set_err(ctx, "too many hashed video frames for the DP tree"); return DAB_E_CAPACITY; }
   int64_t lv[DP_LEVELS], tot = 0;
@@ -1241,6 +1282,8 @@ int dab_enqueue_stage_a_dp(dab_pair *pr) {
   DAB_CUDA(cudaGetLastError());
   return DAB_OK;
 }
+
+int dab_enqueue_stage_a_dp(dab_pair *pr) { return enqueue_dp1(pr, pr->trk[DAB_TRACK_VIDEO]); }
 
 int dab_enqueue_stage_a(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp) {
   DAB_TRY(enqueue_match(pr, row_lo, row_hi));
@@ -1271,12 +1314,11 @@ void dab_collect_stage_a_dp(dab_pair *pr) {
   pr->stats.n_path1 = pr->n_path1;
 }
 
-int dab_collect_stage_a(dab_pair *pr, bool with_dp) {
+// the counts of a match stage (+ DP 1), whichever video side it ran against
+static int collect_match(dab_pair *pr, bool with_dp) {
   dab_ctx *ctx = pr->ctx;
   const int32_t *hc = reinterpret_cast<const int32_t *>(pr->h_counters);
-  Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
-  V.n_list = hc[DC_N_VSEL];
-  A.n_list = hc[DC_N_AQ_ALL];
+  pr->trk[DAB_TRACK_AUDIO].n_list = hc[DC_N_AQ_ALL];
   pr->stats.n_video_selected = hc[DC_N_VSEL];
   pr->stats.n_audio_queries = hc[DC_N_Q];
   pr->stats.n_table_entries = hc[DC_N_ENTRIES];
@@ -1294,7 +1336,89 @@ int dab_collect_stage_a(dab_pair *pr, bool with_dp) {
   pr->n_points1 = hc[DC_N_PTS1];
   pr->stats.n_points1 = pr->n_points1;
   if (with_dp) dab_collect_stage_a_dp(pr);
+  return DAB_OK;
+}
+
+int dab_collect_stage_a(dab_pair *pr, bool with_dp) {
+  pr->trk[DAB_TRACK_VIDEO].n_list = reinterpret_cast<const int32_t *>(pr->h_counters)[DC_N_VSEL];
+  DAB_TRY(collect_match(pr, with_dp));
   pr->matched = true;
+  return DAB_OK;
+}
+
+// ---- shared video index: the video side of the match stage, built once, read by any number of pairs --------
+int dab_build_index(dab_pair *src, dab_index *ix) {
+  dab_ctx *ctx = src->ctx;
+  DAB_TRY(ensure_hann(ctx));
+  const Track &S = src->trk[DAB_TRACK_VIDEO];
+  Track &V = ix->V;
+  V.S = S.S; V.ch = S.ch; V.L = S.L; V.Le = S.Le; V.have_features = true;
+  cudaStream_t st = src->stream;
+  const int64_t v_nq = V.Le - 41;
+  int64_t cap_e = first_entries_cap(V);
+  DAB_TRY(dab_ensure(ctx, ix->counters, sizeof(int32_t) * DC_WORDS));
+  int32_t *dc = ix->counters.as<int32_t>();
+  const int32_t *hc = reinterpret_cast<const int32_t *>(src->h_counters);
+  for (int attempt = 0; attempt < DAB_STAGE_A_ATTEMPTS; ++attempt) {
+    DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, st));
+    DAB_TRY(prep_track(src, S, V, true));
+    // DC_N_VNQ and DC_N_VSEL; the audio words it also writes are never read from the index's block
+    const int32_t *v_off = V.nq_flag.as<int32_t>() + (v_nq + 1);
+    counts_lists_kernel<<<1, 32, 0, st>>>(dc, v_off, v_nq, v_off, v_nq, 0, 0);
+    ctx->launches += 1;
+    DAB_TRY(enqueue_tables(src, V, dc, cap_e, ix->tbl_start, ix->tbl_items));
+    DAB_TRY(enqueue_video_records(src, V, dc, ix->v_rec));
+    DAB_CUDA(dab_readback(src, src->h_counters, dc, sizeof(int32_t) * DC_WORDS));
+    DAB_CUDA(dab_wait_stream(st));
+    if (!(hc[DC_OVERFLOW] & DAB_OVF_ENTRIES)) {
+      V.n_list = ix->n_vsel = hc[DC_N_VSEL];
+      ix->n_entries = hc[DC_N_ENTRIES];
+      ix->cap_entries = cap_e;
+      DAB_CUDA(cudaEventRecord(ix->ready, st));
+      DAB_CUDA(cudaGetLastError());
+      return DAB_OK;
+    }
+    cap_e = std::max<int64_t>(2 * cap_e, hc[DC_NEED_ENTRIES]);
+  }
+  dab_set_err(ctx, "dab_index_build: the hash tables overflowed on every attempt");
+  return DAB_E_CAPACITY;
+}
+
+// Match stage + DP 1 of the pair's description track against a built index: audio prep, gate, scoring, DP 1,
+// traceback and the counts, enqueued without a host round trip.  The index is only read.
+int dab_enqueue_stage_a_against(dab_pair *pr, const dab_index *ix) {
+  dab_ctx *ctx = pr->ctx;
+  DAB_TRY(ensure_hann(ctx));
+  const Track &V = ix->V;
+  Track &A = pr->trk[DAB_TRACK_AUDIO];
+  cudaStream_t st = pr->stream;
+  pr->n_points1 = pr->n_path1 = 0;
+  pr->matched = false;              // the pair's own tables and hashed-frame list are not those of these points
+  pr->points_from_index = true;
+  pr->cap_cand = std::max<int64_t>(pr->cap_cand, first_cand_cap(A));
+  const int64_t v_nq = V.Le - 41, a_nq = A.Le - 41;
+
+  DAB_TRY(dab_ensure(ctx, pr->counters, sizeof(int32_t) * DC_WORDS));
+  int32_t *dc = pr->counters.as<int32_t>();
+  DAB_CUDA(cudaStreamWaitEvent(st, ix->ready, 0));
+  DAB_CUDA(cudaEventRecord(pr->ev[4], st));
+  DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, st));
+  DAB_TRY(prep_track(pr, A, A, false));
+  counts_lists_kernel<<<1, 32, 0, st>>>(dc, V.nq_flag.as<int32_t>() + (v_nq + 1), v_nq, A.nq_flag.as<int32_t>() + (a_nq + 1), a_nq,
+                                        0, INT64_MAX);
+  ctx->launches += 1;
+  DAB_CUDA(cudaEventRecord(pr->ev[5], st));
+  pr->stats.n_video_frames = V.L; pr->stats.n_audio_frames = A.L;
+  DAB_TRY(enqueue_gate_score(pr, VideoSide{&V, ix->tbl_start.as<int32_t>(), ix->tbl_items.as<int32_t>(), ix->v_rec.as<uint4>()}, dc));
+  pr->ev_used[2] = pr->ev_used[4] = pr->ev_used[5] = true;
+  pr->ev_used[3] = false;           // no tables are built
+  DAB_TRY(enqueue_dp1(pr, V));
+  return dab_enqueue_counts(pr);
+}
+
+int dab_collect_stage_a_against(dab_pair *pr, const dab_index *ix) {
+  DAB_TRY(collect_match(pr, true));
+  pr->stats.n_table_entries = ix->n_entries;
   return DAB_OK;
 }
 
@@ -1362,6 +1486,7 @@ int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *
   pr->n_points1 = n;
   pr->stats.n_points1 = n;
   pr->n_path1 = 0;
+  pr->points_from_index = false;
   if (pr->cap_points1 < n) pr->cap_points1 = n;   // DP 1 sizes its buffers from it
   return DAB_OK;
 }

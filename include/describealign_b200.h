@@ -186,6 +186,28 @@ int dab_pair_get_path1(dab_pair *pair, int32_t *x_audio, int32_t *y_video);
 /* pass-1 match points sorted by (audio frame, video frame); any pointer may be NULL. */
 int dab_pair_get_points1(dab_pair *pair, int32_t *i_audio, int32_t *v_video, double *qual);
 
+/* ---- stage A of many combinations: one video index shared by many descriptions ----------------
+ * Which description belongs to which video is decided by stage A itself (its pass-1 path length against
+ * the reference's minimum, :698-699); the video side of stage A (prep, codes, hashed-frame list, hash
+ * tables) depends on the video track only, so it is built once per video.
+ * dab_index_build: the video side of `src`'s video track (features required) into a new index, on src's
+ *   stream; blocks until the index's table capacity is settled, then src may be reused.  The index is
+ *   read-only from then on; an event on it marks it ready and every user's stream waits on it.
+ * dab_pair_stage_a_against: prep of `pair`'s description track (features of the audio track required),
+ *   then gate, scoring, DP 1 and traceback against the index, enqueued without a host round trip; grows and
+ *   reruns on a candidate overflow like dab_pair_stage_a.  Blocks until the counts are back; nothing else
+ *   leaves the device (dab_pair_get_path1 copies the path on request; dab_pair_get_stats has the candidate
+ *   count).  The points are ranks into the index's hashed frames: dab_pair_get_points1 / export_points1
+ *   refuse them, and dab_pair_dp1 / import_points1 need the pair's own stage_a_match again.  Any number of
+ *   pairs, each on its own stream and host thread, may run against one index at once.
+ * dab_index_free: DAB_E_STATE (nothing freed) while a dab_pair_stage_a_against call on the index is running.
+ * dab_index_info: out[0] video frames, [1] hashed frames, [2] table entries, [3] calls running against it. */
+typedef struct dab_index dab_index;
+int dab_index_build(dab_pair *src, dab_index **out);
+int dab_index_free(dab_index *index);
+int dab_index_info(const dab_index *index, int64_t out[4]);
+int dab_pair_stage_a_against(dab_pair *pair, const dab_index *index, int64_t *n_points, int64_t *n_path);
+
 /* ---- stage A in two steps, for one very long pair split over several GPUs (SURVEY.md 8e) ----
  * dab_pair_stage_a_match: prep + codes + tables for the whole pair, then gate + scoring only for the
  * audio frames row_lo <= i < row_hi (pass 0, INT64_MAX for all rows); the match points stay on the
