@@ -267,7 +267,7 @@ void dab_pair_destroy(dab_pair *pr) {
     DevBuf *bs[] = {&k.pcm, &k.feat_ticket, &k.energy, &k.zc, &k.b0, &k.b1, &k.b2, &k.gate, &k.ms, &k.nrm, &k.pack, &k.code, &k.nq_flag, &k.nq_list};
     for (DevBuf *b : bs) free_buf(*b);
   }
-  DevBuf *bs[] = {&pr->scan_tmp, &pr->tbl_count, &pr->tbl_start, &pr->tbl_items, &pr->tbl_ecount, &pr->tbl_pos, &pr->v_rec, &pr->clusters, &pr->refine_partial, &pr->maxes, &pr->row_count, &pr->row_off, &pr->row_stash, &pr->gate_rec, &pr->gate_best, &pr->gate_big,
+  DevBuf *bs[] = {&pr->scan_tmp, &pr->tbl_start, &pr->tbl_items, &pr->tbl_sb, &pr->tbl_ent, &pr->v_rec, &pr->clusters, &pr->refine_partial, &pr->maxes, &pr->row_count, &pr->row_off, &pr->row_stash, &pr->gate_rec, &pr->gate_best, &pr->gate_big,
                   &pr->cand_tmp, &pr->cand_s, &pr->cand_i, &pr->cand_q, &pr->keep_flag, &pr->keep_off, &pr->pt_i,
                   &pr->pt_s, &pr->pt_q, &pr->counters, &pr->tree1, &pr->back1, &pr->dpres,
                   &pr->path1_x, &pr->path1_y, &pr->a_scaled, &pr->v_scaled, &pr->corridors,

@@ -75,11 +75,10 @@ struct dab_pair {
   DevBuf scan_tmp;            // single-pass scan: ticket counter + tile status words
   unsigned int scan_epoch = 0;
   // tables
-  DevBuf tbl_count;   // i32 [5*NCODE + 1]
   DevBuf tbl_start;   // i32 [5*NCODE + 1]
   DevBuf tbl_items;   // i32 sel-ranks
-  DevBuf tbl_ecount;  // i32 [2][5 * vsel_cap + 1]: codes per (frame, table) and their exclusive scan
-  DevBuf tbl_pos;     // i32 [entries]: position of every expanded entry inside its bucket
+  DevBuf tbl_sb;      // i32: per super-bucket of 4096 slots its entry count, offset (+ total) and scatter cursor
+  DevBuf tbl_ent;     // u32 x2 [entries]: (slot within its super-bucket, rank), grouped by super-bucket
   DevBuf v_rec;       // uint4[2] per hashed video frame: its five digit packs (gate)
   // gate / scoring
   DevBuf row_count, row_off;   // i32 [n_queries + 1]

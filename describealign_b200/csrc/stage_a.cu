@@ -304,8 +304,30 @@ __global__ void compact_kernel(const int32_t *flag, const int32_t *off, int64_t 
 }
 
 // ------------------------------------------------------------------------------------------
-// tables
+// tables: a two-level counting sort of the expanded entries by slot f * 7^7 + code
 // ------------------------------------------------------------------------------------------
+// A hashed video frame is stored under every code reachable through its flagged digits (2^flags codes per table,
+// :630-633).  A C2 pair expands 5 x 69 k frames to 3.7 M entries over 4.1 M slots, 88 % of which stay empty, so
+// the slots are cut into super-buckets of TB_SB: entries are first sorted by super-bucket (high bits of the slot),
+// then every super-bucket sorts its own entries by local slot (low bits) in shared memory.  Nothing touches all
+// 4.1 M slots except the coalesced write of start[], and no global atomic is issued per entry.
+//   table_count_kernel    thread per hashed frame: its record (below) and a shared-memory histogram of the
+//                         super-buckets of its entries; one global add per non-zero bin and CTA
+//   table_scan_kernel     one CTA: offsets of the super-buckets; the entry total against the capacity
+//   table_scatter_kernel  the same CTAs again: one range per (CTA, super-bucket) reserved by one atomic, the
+//                         entries written into it as (local slot, rank)
+//   table_sort_kernel     CTA per super-bucket: TB_SB counters in shared memory, start[] of its slots, items[] in
+//                         its own range.  The order of the ranks inside a bucket is free (the gate orders what it
+//                         finds by rank).
+constexpr int TB_SB_BITS = 12, TB_SB = 1 << TB_SB_BITS;
+constexpr int64_t TB_NSLOTS = 5LL * DAB_NCODE;
+constexpr int TB_NSB = (int)((TB_NSLOTS + TB_SB - 1) / TB_SB);     // 1006, the last one partial
+constexpr int TB_THREADS = 256;                                   // count / scatter: one hashed frame per thread
+constexpr int TS_THREADS = 512, TS_UNROLL = 4;                    // sort: entries in chunks of TS_THREADS x TS_UNROLL
+constexpr int TB_SCAN_THREADS = 1024;
+static_assert(TB_NSB <= TB_SCAN_THREADS, "one super-bucket count per thread of the scan");
+static_assert(TB_SB == TS_THREADS * 8, "the sort's block scan gives every thread 8 consecutive counters");
+
 __device__ __forceinline__ int32_t pack_to_code(uint32_t pk) {
   int32_t c = 0, p7 = 1;
 #pragma unroll
@@ -316,73 +338,160 @@ __device__ __forceinline__ int32_t pack_to_code(uint32_t pk) {
   return c;
 }
 
-// One thread per (selected video frame, table).  A frame is stored under every code reachable through its
-// flagged digits (2^flags codes, :630-633).  Three steps without a second round of atomics:
-//   table_expand_kernel   how many codes each (frame, table) expands to -> scan -> where its entries' bucket
-//                         positions are kept
-//   table_kernel<false>   atomicAdd on the code's counter; the value it returns IS the entry's position in
-//                         its bucket and is kept
-//   table_kernel<true>    after the scan of the counters: items[start[code] + position] = frame, plain stores
-__global__ void table_expand_kernel(const uint32_t *pack, int64_t nstride, const int32_t *sel, const int32_t *dc, int64_t vsel_cap,
-                                    int32_t *ecount) {
-  const int f = blockIdx.y;
-  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (s >= vsel_cap) return;
-  int32_t c = 0;
-  if (s < dc[DC_N_VSEL]) c = 1 << __popc(pack[(int64_t)f * nstride + sel[s]] & 0x8888888u);
-  ecount[(int64_t)f * vsel_cap + s] = c;
+// fn(slot) for every slot f * 7^7 + code the digit word pk of table f is stored under
+template <typename F>
+__device__ __forceinline__ void for_each_slot(int f, uint32_t pk, F &&fn) {
+  const int32_t P7[7] = {1, 7, 49, 343, 2401, 16807, 117649};
+  const uint32_t fl = pk & 0x8888888u;             // flag bits, one per nibble
+  const int32_t base = f * DAB_NCODE + pack_to_code(pk);
+  uint32_t sub = fl;
+  while (true) {
+    int32_t c = base;
+#pragma unroll
+    for (int k = 0; k < 7; ++k)
+      if (sub & (8u << (4 * k))) c += P7[k];
+    fn(c);
+    if (sub == 0) break;
+    sub = (sub - 1) & fl;
+  }
 }
 
-template <bool FILL>
-__global__ void table_kernel(const uint32_t *pack, int64_t nstride, const int32_t *sel, const int32_t *dc, int64_t vsel_cap,
-                             const int32_t *ebase, int32_t *tpos, int32_t *count, const int32_t *start, int32_t *items,
-                             int64_t items_cap) {
-  const int f = blockIdx.y;
-  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (s >= dc[DC_N_VSEL]) return;
+// The five digit words (one digit per nibble, see digits_match) of every hashed video frame side by side (32 bytes
+// per frame, indexed by the frame's rank in the hashed list): a bucket entry then costs the gate ONE 32-byte sector
+// instead of a rank -> frame look-up plus five gathers from five arrays.  The count pass writes them; the scatter
+// pass reads its digit words back from them.
+__global__ void __launch_bounds__(TB_THREADS) table_count_kernel(const uint32_t *pack, int64_t nstride, const int32_t *sel,
+                                                                  const int32_t *dc, uint4 *rec, int32_t *sb_count) {
+  __shared__ int hist[TB_NSB];
+  for (int b = threadIdx.x; b < TB_NSB; b += TB_THREADS) hist[b] = 0;
+  __syncthreads();
+  const int64_t s = (int64_t)blockIdx.x * TB_THREADS + threadIdx.x;
+  if (s < dc[DC_N_VSEL]) {
+    const int32_t v = sel[s];
+    uint32_t p[5];
+#pragma unroll
+    for (int f = 0; f < 5; ++f) p[f] = pack[(int64_t)f * nstride + v];
+    rec[2 * s] = make_uint4(p[0], p[1], p[2], p[3]);
+    rec[2 * s + 1] = make_uint4(p[4], (uint32_t)v, 0u, 0u);
+#pragma unroll
+    for (int f = 0; f < 5; ++f) for_each_slot(f, p[f], [&](int32_t slot) { atomicAdd(&hist[slot >> TB_SB_BITS], 1); });
+  }
+  __syncthreads();
+  for (int b = threadIdx.x; b < TB_NSB; b += TB_THREADS) {
+    const int n = hist[b];
+    if (n) atomicAdd(&sb_count[b], n);
+  }
+}
+
+// sb_off[b] = first entry of super-bucket b (sb_off[TB_NSB] = total), the scatter's cursors = the same; the total
+// goes to DC_NEED_ENTRIES and, unless it exceeds the capacity (overflow bit, count 0), to DC_N_ENTRIES
+__global__ void __launch_bounds__(TB_SCAN_THREADS) table_scan_kernel(int32_t *dc, int64_t cap, const int32_t *sb_count,
+                                                                      int32_t *sb_off, int32_t *sb_cursor) {
+  __shared__ int sm[33];
+  const int b = threadIdx.x;
+  int total;
+  const int ex = block_exclusive_scan(b < TB_NSB ? sb_count[b] : 0, &total, sm);
+  if (b < TB_NSB) { sb_off[b] = ex; sb_cursor[b] = ex; }
+  if (b == 0) {
+    sb_off[TB_NSB] = total;
+    dc[DC_NEED_ENTRIES] = total;
+    if ((int64_t)total > cap) { dc[DC_N_ENTRIES] = 0; atomicOr(&dc[DC_OVERFLOW], DAB_OVF_ENTRIES); }
+    else dc[DC_N_ENTRIES] = total;
+  }
+}
+
+// ent[] = (local slot, rank) of every entry, grouped by super-bucket (any order inside one)
+__global__ void __launch_bounds__(TB_THREADS) table_scatter_kernel(const uint4 *rec, const int32_t *dc, int32_t *sb_cursor,
+                                                                    uint2 *ent) {
+  __shared__ int pos[TB_NSB];
   if (dc[DC_OVERFLOW] & DAB_OVF_ENTRIES) return;
-  const uint32_t pk = pack[(int64_t)f * nstride + sel[s]];
-  const uint32_t fl = pk & 0x8888888u;             // flag bits, one per nibble
-  const int32_t base = pack_to_code(pk);
-  const int32_t P7[7] = {1, 7, 49, 343, 2401, 16807, 117649};
-  int64_t e = ebase[(int64_t)f * vsel_cap + s];
-  // four codes per step: the four atomics (count pass) / the four position and start loads (fill pass) are
-  // issued before the first result is used, so their latencies overlap instead of adding up
-  uint32_t sub = fl;
-  bool more = true;
-  while (more) {
-    int64_t slot[4];
-    bool live[4];
+  for (int b = threadIdx.x; b < TB_NSB; b += TB_THREADS) pos[b] = 0;
+  __syncthreads();
+  const int64_t s = (int64_t)blockIdx.x * TB_THREADS + threadIdx.x;
+  const bool live = s < dc[DC_N_VSEL];
+  uint32_t p[5] = {0u, 0u, 0u, 0u, 0u};
+  if (live) {
+    const uint4 r0 = rec[2 * s], r1 = rec[2 * s + 1];
+    p[0] = r0.x; p[1] = r0.y; p[2] = r0.z; p[3] = r0.w; p[4] = r1.x;
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      live[u] = more;
-      int32_t c = base;
+    for (int f = 0; f < 5; ++f) for_each_slot(f, p[f], [&](int32_t slot) { atomicAdd(&pos[slot >> TB_SB_BITS], 1); });
+  }
+  __syncthreads();
+  // this CTA's range in every super-bucket it reaches; pos[] then holds the next free entry of each range
+  for (int b = threadIdx.x; b < TB_NSB; b += TB_THREADS) {
+    const int n = pos[b];
+    if (n) pos[b] = atomicAdd(&sb_cursor[b], n);
+  }
+  __syncthreads();
+  if (live) {
 #pragma unroll
-      for (int k = 0; k < 7; ++k)
-        if (sub & (8u << (4 * k))) c += P7[k];
-      slot[u] = (int64_t)f * DAB_NCODE + c;
-      if (more) { if (sub == 0) more = false; else sub = (sub - 1) & fl; }
+    for (int f = 0; f < 5; ++f)
+      for_each_slot(f, p[f], [&](int32_t slot) {
+        const int at = atomicAdd(&pos[slot >> TB_SB_BITS], 1);
+        ent[at] = make_uint2((uint32_t)slot & (TB_SB - 1), (uint32_t)s);
+      });
+  }
+}
+
+// start[] of the super-bucket's TB_SB slots and its entries' ranks in items[].  Its entries are read twice (count,
+// then place), TS_THREADS x TS_UNROLL at a time, so a super-bucket of any size is sorted in the same shared memory.
+// After an entries overflow every start is 0 (empty tables), as the gate expects.
+__global__ void __launch_bounds__(TS_THREADS) table_sort_kernel(const int32_t *dc, const int32_t *sb_off, const uint2 *ent,
+                                                                 int32_t *start, int32_t *items) {
+  __shared__ __align__(16) int cnt[TB_SB];
+  __shared__ int sm[33];
+  const int tid = threadIdx.x;
+  const int sb = blockIdx.x;
+  const bool ovf = (dc[DC_OVERFLOW] & DAB_OVF_ENTRIES) != 0;
+  const int lo = ovf ? 0 : sb_off[sb], hi = ovf ? 0 : sb_off[sb + 1];
+  for (int j = tid; j < TB_SB; j += TS_THREADS) cnt[j] = 0;
+  __syncthreads();
+  for (int e0 = lo + tid; e0 < hi; e0 += TS_THREADS * TS_UNROLL) {
+    uint32_t key[TS_UNROLL];
+#pragma unroll
+    for (int u = 0; u < TS_UNROLL; ++u) {
+      const int e = e0 + u * TS_THREADS;
+      key[u] = e < hi ? ent[e].x : (uint32_t)TB_SB;
     }
-    int32_t v0[4], v1[4];
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      v0[u] = v1[u] = 0;
-      if (live[u] && e + u < items_cap) {
-        if (!FILL) v0[u] = atomicAdd(&count[slot[u]], 1);
-        else { v0[u] = tpos[e + u]; v1[u] = start[slot[u]]; }
-      }
+    for (int u = 0; u < TS_UNROLL; ++u)
+      if (key[u] < (uint32_t)TB_SB) atomicAdd(&cnt[key[u]], 1);
+  }
+  __syncthreads();
+  // exclusive scan of the counters, 8 consecutive ones per thread: the slots' starts, written coalesced
+  const int4 c0 = *reinterpret_cast<const int4 *>(&cnt[tid * 8]);
+  const int4 c1 = *reinterpret_cast<const int4 *>(&cnt[tid * 8 + 4]);
+  const int v[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
+  int total;
+  const int ex = block_exclusive_scan(v[0] + v[1] + v[2] + v[3] + v[4] + v[5] + v[6] + v[7], &total, sm);
+  int st[8];
+  st[0] = lo + ex;
+#pragma unroll
+  for (int k = 1; k < 8; ++k) st[k] = st[k - 1] + v[k - 1];
+  const int64_t slot0 = (int64_t)sb * TB_SB + tid * 8;
+  if (slot0 + 8 <= TB_NSLOTS) {
+    reinterpret_cast<int4 *>(start + slot0)[0] = make_int4(st[0], st[1], st[2], st[3]);
+    reinterpret_cast<int4 *>(start + slot0)[1] = make_int4(st[4], st[5], st[6], st[7]);
+  } else {
+#pragma unroll
+    for (int k = 0; k < 8; ++k)
+      if (slot0 + k < TB_NSLOTS) start[slot0 + k] = st[k];
+  }
+  if (sb == TB_NSB - 1 && tid == 0) start[TB_NSLOTS] = hi;    // the total (0 after an overflow)
+  // counters become the slots' cursors (block_exclusive_scan's barriers order every read of cnt before this)
+  *reinterpret_cast<int4 *>(&cnt[tid * 8]) = make_int4(st[0], st[1], st[2], st[3]);
+  *reinterpret_cast<int4 *>(&cnt[tid * 8 + 4]) = make_int4(st[4], st[5], st[6], st[7]);
+  __syncthreads();
+  for (int e0 = lo + tid; e0 < hi; e0 += TS_THREADS * TS_UNROLL) {
+    uint2 x[TS_UNROLL];
+#pragma unroll
+    for (int u = 0; u < TS_UNROLL; ++u) {
+      const int e = e0 + u * TS_THREADS;
+      x[u] = e < hi ? ent[e] : make_uint2((uint32_t)TB_SB, 0u);
     }
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      if (live[u] && e + u < items_cap) {
-        if (!FILL) tpos[e + u] = v0[u];
-        else {
-          const int64_t at = (int64_t)v1[u] + v0[u];
-          if (at < items_cap) items[at] = (int32_t)s;
-        }
-      }
-    }
-    e += 4;
+    for (int u = 0; u < TS_UNROLL; ++u)
+      if (x[u].x < (uint32_t)TB_SB) items[atomicAdd(&cnt[x[u].x], 1)] = (int32_t)x[u].y;
   }
 }
 
@@ -401,21 +510,6 @@ __global__ void table_kernel(const uint32_t *pack, int64_t nstride, const int32_
 __device__ __forceinline__ bool digits_match(uint32_t a_guarded, uint32_t v) {
   const uint32_t d = (a_guarded - (v & 0x7777777u)) ^ 0x8888888u;
   return (d & ~((v >> 3) & 0x1111111u)) == 0u;
-}
-
-// The five digit words (one digit per nibble, see digits_match) of every hashed video frame side by side
-// (32 bytes per frame, indexed by the
-// frame's rank in the hashed list): a bucket entry then costs the gate ONE 32-byte sector instead of a
-// rank -> frame look-up plus five gathers from five arrays.
-__global__ void video_records_kernel(const uint32_t *pack, int64_t nstride, const int32_t *sel, const int32_t *dc, uint4 *rec) {
-  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (s >= dc[DC_N_VSEL]) return;
-  const int32_t v = sel[s];
-  uint4 r0, r1;
-  r0.x = pack[v]; r0.y = pack[nstride + v]; r0.z = pack[2 * nstride + v]; r0.w = pack[3 * nstride + v];
-  r1.x = pack[4 * nstride + v]; r1.y = (uint32_t)v; r1.z = 0u; r1.w = 0u;
-  rec[2 * s] = r0;
-  rec[2 * s + 1] = r1;
 }
 
 constexpr int GATE_STASH = 4;   // rows with at most this many candidates (nearly all) are not enumerated a second time
@@ -1100,42 +1194,30 @@ struct VideoSide {
 
 static int64_t video_sel_ub(const Track &V) { return (V.Le - 41 + 3) / 4 + 1; }
 
-// tables over the hashed video frames (dc[DC_N_VSEL] of them) into start / items; the pair's table scratch counts
-static int enqueue_tables(dab_pair *pr, const Track &V, int32_t *dc, int64_t cap_e, DevBuf &tbl_start, DevBuf &tbl_items) {
+// tables over the hashed video frames (dc[DC_N_VSEL] of them) into start / items, and the frames' records into rec;
+// the pair's table scratch holds the super-bucket counts and the entries between the passes
+static int enqueue_tables(dab_pair *pr, const Track &V, int32_t *dc, int64_t cap_e, DevBuf &tbl_start, DevBuf &tbl_items,
+                          DevBuf &rec) {
   dab_ctx *ctx = pr->ctx;
   cudaStream_t st = pr->stream;
   const int64_t vsel_ub = video_sel_ub(V);
-  const int64_t nslots = 5LL * DAB_NCODE;
   const int64_t v_nstride = (V.Le > V.L ? V.Le : V.L) - 40;
-  DAB_TRY(dab_ensure(ctx, pr->tbl_count, sizeof(int32_t) * (size_t)(nslots + 1)));
-  DAB_TRY(dab_ensure(ctx, tbl_start, sizeof(int32_t) * (size_t)(nslots + 2)));
+  DAB_TRY(dab_ensure(ctx, tbl_start, sizeof(int32_t) * (size_t)(TB_NSLOTS + 2)));
   DAB_TRY(dab_ensure(ctx, tbl_items, sizeof(int32_t) * (size_t)(cap_e + 1)));
-  DAB_CUDA(cudaMemsetAsync(pr->tbl_count.p, 0, sizeof(int32_t) * (size_t)(nslots + 1), st));
-  dim3 gt((unsigned)cdiv(vsel_ub, 128), 5);
-  DAB_TRY(dab_ensure(ctx, pr->tbl_ecount, sizeof(int32_t) * (size_t)(2 * (5 * vsel_ub + 2))));
-  DAB_TRY(dab_ensure(ctx, pr->tbl_pos, sizeof(int32_t) * (size_t)(cap_e + 1)));
-  int32_t *ecount = pr->tbl_ecount.as<int32_t>(), *ebase = ecount + (5 * vsel_ub + 1);
-  table_expand_kernel<<<gt, 128, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, vsel_ub, ecount);
-  DAB_TRY(dab_exclusive_scan(pr, ecount, ebase, 5 * vsel_ub, nullptr, dc + DC_N_ENTRIES));
-  check_capacity_kernel<<<1, 32, 0, st>>>(dc, DC_N_ENTRIES, DC_NEED_ENTRIES, cap_e, DAB_OVF_ENTRIES);
-  table_kernel<false><<<gt, 128, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, vsel_ub, ebase,
-                                          pr->tbl_pos.as<int32_t>(), pr->tbl_count.as<int32_t>(), nullptr, nullptr, cap_e);
-  DAB_TRY(dab_exclusive_scan(pr, pr->tbl_count.as<int32_t>(), tbl_start.as<int32_t>(), nslots));
-  table_kernel<true><<<gt, 128, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, vsel_ub, ebase,
-                                         pr->tbl_pos.as<int32_t>(), pr->tbl_count.as<int32_t>(), tbl_start.as<int32_t>(),
-                                         tbl_items.as<int32_t>(), cap_e);
-  ctx->launches += 4;
-  return DAB_OK;
-}
-
-static int enqueue_video_records(dab_pair *pr, const Track &V, const int32_t *dc, DevBuf &rec) {
-  dab_ctx *ctx = pr->ctx;
-  const int64_t vsel_ub = video_sel_ub(V);
-  const int64_t v_nstride = (V.Le > V.L ? V.Le : V.L) - 40;
   DAB_TRY(dab_ensure(ctx, rec, sizeof(uint4) * 2 * (size_t)(vsel_ub + 1)));
-  video_records_kernel<<<(unsigned)cdiv(vsel_ub, 256), 256, 0, pr->stream>>>(V.pack.as<uint32_t>(), v_nstride,
-                                                                            V.nq_list.as<int32_t>(), dc, rec.as<uint4>());
-  ctx->launches += 1;
+  DAB_TRY(dab_ensure(ctx, pr->tbl_sb, sizeof(int32_t) * (size_t)(3 * TB_NSB + 1)));
+  DAB_TRY(dab_ensure(ctx, pr->tbl_ent, sizeof(uint2) * (size_t)(cap_e + 1)));
+  int32_t *sb_count = pr->tbl_sb.as<int32_t>(), *sb_off = sb_count + TB_NSB, *sb_cursor = sb_off + (TB_NSB + 1);
+  DAB_CUDA(cudaMemsetAsync(sb_count, 0, sizeof(int32_t) * TB_NSB, st));
+  const unsigned nb = (unsigned)cdiv(vsel_ub, TB_THREADS);
+  table_count_kernel<<<nb, TB_THREADS, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, rec.as<uint4>(),
+                                                sb_count);
+  table_scan_kernel<<<1, TB_SCAN_THREADS, 0, st>>>(dc, cap_e, sb_count, sb_off, sb_cursor);
+  table_scatter_kernel<<<nb, TB_THREADS, 0, st>>>(rec.as<uint4>(), dc, sb_cursor, pr->tbl_ent.as<uint2>());
+  table_sort_kernel<<<TB_NSB, TS_THREADS, 0, st>>>(dc, sb_off, pr->tbl_ent.as<uint2>(), tbl_start.as<int32_t>(),
+                                                   tbl_items.as<int32_t>());
+  ctx->launches += 4;
+  DAB_CUDA(cudaGetLastError());
   return DAB_OK;
 }
 
@@ -1238,9 +1320,8 @@ static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
   pr->stats.n_video_frames = V.L; pr->stats.n_audio_frames = A.L;
 
   DAB_CUDA(cudaEventRecord(pr->ev[6], st));
-  DAB_TRY(enqueue_tables(pr, V, dc, pr->cap_entries, pr->tbl_start, pr->tbl_items));
+  DAB_TRY(enqueue_tables(pr, V, dc, pr->cap_entries, pr->tbl_start, pr->tbl_items, pr->v_rec));
   DAB_CUDA(cudaEventRecord(pr->ev[7], st));
-  DAB_TRY(enqueue_video_records(pr, V, dc, pr->v_rec));
   DAB_TRY(enqueue_gate_score(pr, VideoSide{&V, pr->tbl_start.as<int32_t>(), pr->tbl_items.as<int32_t>(), pr->v_rec.as<uint4>()}, dc));
   for (int s = 2; s <= 5; ++s) pr->ev_used[s] = true;
   DAB_CUDA(cudaGetLastError());
@@ -1366,8 +1447,7 @@ int dab_build_index(dab_pair *src, dab_index *ix) {
     const int32_t *v_off = V.nq_flag.as<int32_t>() + (v_nq + 1);
     counts_lists_kernel<<<1, 32, 0, st>>>(dc, v_off, v_nq, v_off, v_nq, 0, 0);
     ctx->launches += 1;
-    DAB_TRY(enqueue_tables(src, V, dc, cap_e, ix->tbl_start, ix->tbl_items));
-    DAB_TRY(enqueue_video_records(src, V, dc, ix->v_rec));
+    DAB_TRY(enqueue_tables(src, V, dc, cap_e, ix->tbl_start, ix->tbl_items, ix->v_rec));
     DAB_CUDA(dab_readback(src, src->h_counters, dc, sizeof(int32_t) * DC_WORDS));
     DAB_CUDA(dab_wait_stream(st));
     if (!(hc[DC_OVERFLOW] & DAB_OVF_ENTRIES)) {
