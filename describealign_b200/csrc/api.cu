@@ -264,7 +264,7 @@ void dab_pair_destroy(dab_pair *pr) {
   if (pr->stream) dab_wait_stream(pr->stream);
   for (int t = 0; t < 2; ++t) {
     Track &k = pr->trk[t];
-    DevBuf *bs[] = {&k.pcm, &k.feat_ticket, &k.energy, &k.zc, &k.b0, &k.b1, &k.b2, &k.gate, &k.ms, &k.nrm, &k.pack, &k.code, &k.nq_flag, &k.nq_list};
+    DevBuf *bs[] = {&k.pcm, &k.feat_ticket, &k.feat_mid, &k.energy, &k.zc, &k.b0, &k.b1, &k.b2, &k.gate, &k.ms, &k.nrm, &k.pack, &k.code, &k.nq_flag, &k.nq_list};
     for (DevBuf *b : bs) free_buf(*b);
   }
   DevBuf *bs[] = {&pr->scan_tmp, &pr->tbl_start, &pr->tbl_items, &pr->tbl_sb, &pr->tbl_ent, &pr->v_rec, &pr->clusters, &pr->refine_partial, &pr->maxes, &pr->row_count, &pr->row_off, &pr->row_stash, &pr->gate_rec, &pr->gate_best, &pr->gate_big,

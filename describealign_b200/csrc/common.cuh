@@ -42,6 +42,7 @@ struct Track {
   DevBuf pcm;          // staging for host PCM
   DevBuf energy, zc, b0, b1, b2;   // f32 x4, f64
   DevBuf feat_ticket;  // u32: tile ticket of the persistent feature kernel
+  DevBuf feat_mid;     // per-frame intermediates between the two feature kernels (features.cu: FeatMid), 212 B per frame
   DevBuf gate;         // the separate *_energy argument of align() when it is not features[0] (:629, :657)
   bool have_gate = false;
   // stage A prep (features 0..2 keep ms / nrm for scoring; 3, 4 only feed the codes)

@@ -1,23 +1,25 @@
 // Feature extraction for one track: the five 210 Hz feature vectors of the reference
 // (get_energy describealign.py:545-555, get_zero_crossings :557-566, downsample_blur
-// :568-573, get_freq_bands :575-593) in ONE pass over the PCM.
+// :568-573, get_freq_bands :575-593) in two kernels.
 //
-// One CTA produces FT consecutive output frames.  It stages the samples of frames
-// [t0-8, t0+FT+8) plus 40 samples of filter halo in shared memory as float16 (the
-// reference's own sample type, :156) with 16-byte loads, derives every intermediate of the
-// polyphase filter bank (lp1 @8820 Hz, lp2 @1260 Hz, the three residual band energies,
-// 105-sample block energies, per-frame zero-crossing counts) in shared memory, and writes
-// only the five outputs.  HBM traffic: the PCM once (+ halo re-reads, served from L2) and
-// 24 B per frame.  The Hann tables live in shared memory as well: they are indexed by the
-// phase, which differs between the threads of a warp, and divergent __constant__ reads
-// serialise (the first version of this kernel spent 85 % of its cycles in that unit).
+// features_kernel makes one pass over the PCM.  One CTA produces the per-frame intermediates of FT consecutive
+// frames.  It stages the samples of frames [t0-8, t0+FT+8) plus 40 samples of filter halo in shared memory as float16
+// (the reference's own sample type, :156) with 16-byte loads, derives lp1 @8820 Hz and lp2 @1260 Hz of the polyphase
+// filter bank in shared memory, and writes per frame the 42 + 6 residual band energies, the band-2 frame energy, the
+// two 105-sample block energies and the zero-crossing count (212 B) to a per-track scratch buffer.
+// bands_kernel reads that scratch back and runs the 42 + 6 polyphase 15-tap filters at 210 Hz and the five outputs
+// (24 B per frame).  The split sits where the least data crosses: the 210 Hz stage is bound by the f32->f64
+// converts of the XU pipe, the 8820 Hz stage by the FMA / ALU / LSU pipes, and in one CTA each waited on the other
+// at the barriers of every tile.  Apart, the small 210 Hz CTAs share SMs with other pairs' ALU-bound kernels.
+// The Hann tables of features_kernel live in shared memory: they are indexed by the phase, which differs between the
+// threads of a warp, and divergent __constant__ reads serialise.
 //
 // Bit-exactness (SURVEY.md B.1-B.3): every sum is evaluated in the order numpy / OpenBLAS
 // use in the reference - parallelism is across outputs, never across the taps of one
 // output - with separately rounded multiplies and adds (-fmad=false), f32 products
 // accumulated in f64 where numpy does, and glibc's log10f restated in IEEE operations.
 // The arithmetic cost of those fixed orders (about 6 500 instructions per frame, of which
-// 630 f32->f64 conversions) is what bounds this kernel, not HBM.
+// 630 f32->f64 conversions) is what bounds these kernels, not HBM.
 #include <cuda_fp16.h>
 
 #include <atomic>
@@ -35,7 +37,6 @@ constexpr int NTAB = 772;         // 630 + 90 + 21 + 15 + 13 = 769 floats, padde
 
 template <int CH> struct Tile {
   static constexpr int FT = CH == 1 ? 100 : 48;      // output frames per tile
-  static constexpr int TC = CH == 1 ? 10 : 8;         // frames per phase task: 48 * FT / TC tasks (480 / 288), one round of the 512 threads
   static constexpr int NF = FT + 2 * FH;              // frames staged
   static constexpr int NS = NF * 210 + 2 * PADS;      // samples staged (multiple of 8)
   static constexpr int N1 = NF * 42 + 14;             // lp1 entries staged (+-7)
@@ -44,16 +45,15 @@ template <int CH> struct Tile {
   static constexpr int O_SIG = O_TAB + NTAB * 4;
   static constexpr int O_RAW = O_SIG + (NS + 16) * 2;                           // stereo only: half2 per sample
   static constexpr int O_LP1 = O_RAW + (CH == 2 ? NF * 210 * 4 : 0);
-  static constexpr int O_BE0 = O_LP1 + ((N1 * 4 + 15) & ~15);
-  static constexpr int O_LP2 = O_BE0 + NF * 42 * 4;
-  static constexpr int O_BE1 = O_LP2 + NF * 6 * 4;
-  static constexpr int O_BE2 = O_BE1 + NF * 6 * 4;
-  static constexpr int O_EB = O_BE2 + NF * 8;
-  static constexpr int O_ZI = O_EB + 2 * NF * 4;
-  static constexpr int O_P1 = O_ZI + NF * 4;                                    // band-1 phase sums FT*6
-  static constexpr int BYTES = O_P1 + FT * 6 * 4;
-  static_assert(NS % 8 == 0 && N1 % 2 == 0 && (NS * 2) % 16 == 0 && O_SIG % 16 == 0 && FT * 42 <= N1, "tile layout");
+  static constexpr int O_ZI = O_LP1 + ((N1 * 4 + 15) & ~15);
+  static constexpr int BYTES = O_ZI + NF * 4;
+  static_assert(NS % 8 == 0 && N1 % 2 == 0 && (NS * 2) % 16 == 0 && O_SIG % 16 == 0, "tile layout");
 };
+
+// bands_kernel: FR output frames per CTA, one thread per (phase, run of TC frames), 48 phases
+constexpr int FR = 32;
+constexpr int TC = 8;
+constexpr int THREADS2 = 48 * FR / TC;
 
 __device__ float g_tables[NTAB];   // w630 | w90 | w21 | w15 | w13
 // "native numpy" mode (SURVEY.md B.4): numpy's SIMD log10 differs from glibc's log10f by up to 2 ulp on about
@@ -138,6 +138,16 @@ __device__ __forceinline__ __half mid_half(__half l, __half r) {
   return __float2half_rn(s / 2.0f);
 }
 
+// Per-frame intermediates of a track, frames [0, L) (eb: blocks [0, 2 Le)), written by features_kernel and read by
+// bands_kernel.  Frame-major: a warp over consecutive phases of one frame reads consecutive addresses.
+struct FeatMid {
+  float *be0;     // [L][42] band-0 residual energies at 8820 Hz
+  float *be1;     // [L][6]  band-1 residual energies at 1260 Hz
+  double *be2;    // [L]     band-2 frame energies
+  float *eb;      // [2 Le]  105-sample block energies (0 past the last block)
+  int *zi;        // [L]     zero crossings
+};
+
 struct FeatArgs {
   const void *pcm;
   int64_t S;      // samples per channel
@@ -147,6 +157,13 @@ struct FeatArgs {
   int vec_ok;     // pcm is 16-byte aligned
   int64_t tiles;  // tiles of FT output frames
   unsigned int *ticket;   // next tile (zeroed before the launch)
+  FeatMid mid;
+};
+
+// 210 Hz kernel: the scratch written by features_kernel in, the five features out
+struct BandArgs {
+  FeatMid mid;
+  int64_t L, Le;
   float *energy, *zc, *b0, *b1;
   double *b2;
 };
@@ -238,35 +255,29 @@ __device__ __forceinline__ void bulk_load(void *dst_smem, const void *src_gmem, 
                : "memory");
 }
 
-// Persistent kernel: 2 CTAs per SM, each taking tiles of FT output frames from an atomic ticket.  Per tile:
+// Persistent kernel: 2 CTAs per SM, each taking tiles of FT frames from an atomic ticket.  Per tile:
 //   S0   the staged signal arrives (bulk copy issued during the previous tile, converted int16 -> float16 in place;
 //        edge tiles and stereo tracks are staged by the threads themselves)
 //   S1   lp1 = downsample_blur(m, 5, 3) and, from the same register window, the band-0 residual energies
-//   S2   block energies, zero crossings, lp2 = downsample_blur(lp1, 7, 3) with the band-1 residual energies from
-//        the same window and the band-2 frame energies by warp shuffles; the signal buffer is dead after this
-//        stage: the next tile's bulk copy is issued here and overlaps S3 / S4
-//   S3   the 42 + 6 polyphase 15-tap filters at 210 Hz (f32 products accumulated in f64)
-//   S4   the five outputs
+//   S2a  block energies, S2b zero crossings: like S1 they read only the signal, so the three share one phase; the
+//        signal buffer is dead after it: the next tile's bulk copy is issued here and overlaps S2c
+//   S2c  lp2 = downsample_blur(lp1, 7, 3) with the band-1 residual energies from the same window and the band-2
+//        frame energies by warp shuffles
+// The halo frames [t0-8, t0) and [t0+FT, t0+FT+8) are computed (lp2 needs them) but only the FT frames of the tile
+// itself are written to the scratch.
 template <int FMT, int CH>
 __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
   using T = Tile<CH>;
-  constexpr int FT = T::FT, NF = T::NF, NS = T::NS, N1 = T::N1, TC = T::TC;
+  constexpr int FT = T::FT, NF = T::NF, NS = T::NS, N1 = T::N1;
   extern __shared__ __align__(16) unsigned char smem[];
   __shared__ __align__(8) uint64_t s_bar;
   __shared__ int s_next;
   float *tab = reinterpret_cast<float *>(smem + T::O_TAB);
-  const float *w630 = tab, *w90 = tab + 630, *w21 = tab + 720, *w15 = tab + 741, *w13 = tab + 756;
+  const float *w21 = tab + 720, *w15 = tab + 741;
   __half *sig = reinterpret_cast<__half *>(smem + T::O_SIG);
   __half2 *raw = reinterpret_cast<__half2 *>(smem + T::O_RAW);   // stereo: (left, right) of frame samples
   float *lp1 = reinterpret_cast<float *>(smem + T::O_LP1);
-  float *ph = lp1;                                                  // band-0 phase sums reuse lp1's space
-  float *be0 = reinterpret_cast<float *>(smem + T::O_BE0);
-  float *lp2 = reinterpret_cast<float *>(smem + T::O_LP2);
-  float *be1 = reinterpret_cast<float *>(smem + T::O_BE1);
-  double *be2 = reinterpret_cast<double *>(smem + T::O_BE2);
-  float *eb = reinterpret_cast<float *>(smem + T::O_EB);
   int *zi = reinterpret_cast<int *>(smem + T::O_ZI);
-  float *p1 = reinterpret_cast<float *>(smem + T::O_P1);
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int64_t Sb = a.L * 210;                         // band signal length (:577)
@@ -301,8 +312,7 @@ __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
     const int64_t f0 = t0 - FH;                           // first staged frame (may be < 0)
     const int64_t s0 = f0 * 210 - PADS;                   // first staged sample (may be < 0)
 
-    // ---- S0: the mono / mid signal as float16, zero outside [0, Sb).  (Nothing the previous tile's output stage
-    //      still reads is written here: a warp that is done with S4 starts on the next tile's signal at once.) ------
+    // ---- S0: the mono / mid signal as float16, zero outside [0, Sb); the zero-crossing counts cleared ---------
     if (bulk_ok(tile)) {
       mbar_wait(&s_bar, parity);
       parity ^= 1u;
@@ -366,6 +376,7 @@ __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
         *reinterpret_cast<uint4 *>(sig + 8 * v) = *reinterpret_cast<const uint4 *>(h);
       }
     }
+    for (int k = tid; k < NF; k += THREADS) zi[k] = 0;     // the previous tile copied its counts out before its last barrier
     __syncthreads();
 
     // ---- S1: lp1 = downsample_blur(m, 5, 3): 5 phases x 3 taps, f32 accumulators (B.2 ii).  Two adjacent
@@ -374,7 +385,8 @@ __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
     //      (x - lp1[k])^2 over the MIDDLE five samples of the very window lp1[k] was filtered from, so it is
     //      formed here from the registers ---------------------------------------------------------------------
     const int64_t n1_first = f0 * 42 - 7;          // global lp1 index of lp1[0]
-    for (int k = tid; k < NF; k += THREADS) zi[k] = 0;     // every thread is past the previous tile's S4 (barrier above)
+    // the next tile; every thread has read s_next of this one before the barrier above, and reads this after S2b
+    if (tid == 0) s_next = (int)atomicAdd(a.ticket, 1u);
     {
     const float w15r[15] = {w15[0], w15[1], w15[2], w15[3], w15[4], w15[5], w15[6], w15[7],
                             w15[8], w15[9], w15[10], w15[11], w15[12], w15[13], w15[14]};
@@ -410,15 +422,15 @@ __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
         const float2 d = __fadd2_rn(make_float2(x[5 + i], x[10 + i]), nlo);        // x - lo
         acc = (i == 0) ? __fmul2_rn(d, d) : mul2_then_add(acc, d, d);
       }
+      // staged frame of lp1 entry k is (k - 7) / 42; the scratch takes the tile's own frames FH .. FH + FT - 1
       const int kb = k - 7;
-      if (kb >= 0 && kb < NF * 42) be0[kb] = in0 ? acc.x : 0.0f;
-      if (kb + 1 >= 0 && kb + 1 < NF * 42) be0[kb + 1] = in1 ? acc.y : 0.0f;
+      if (in0 && kb >= FH * 42 && kb < (FH + FT) * 42) a.mid.be0[n] = acc.x;
+      if (in1 && kb + 1 >= FH * 42 && kb + 1 < (FH + FT) * 42) a.mid.be0[n + 1] = acc.y;
     }
     }
-    __syncthreads();
 
-    // ---- S2a: block energies (einsum order): 2 threads per 105-sample block, each running two of the four
-    //      lane accumulators as one packed f32x2 -------------------------------------------------------------
+    // ---- S2a (no barrier before it: it reads only the signal): block energies (einsum order), 2 threads per
+    //      105-sample block, each running two of the four lane accumulators as one packed f32x2 -----------------
     for (int k0 = 0; k0 < 2 * NF * 2; k0 += THREADS) {     // whole warps stay in the loop: it ends in a shuffle
       const int k = k0 + tid;
       const bool on = k < 2 * NF * 2;
@@ -443,7 +455,7 @@ __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
       }
       const float s01 = acc.x + acc.y;                          // l0 + l1  /  l2 + l3
       const float o2 = __shfl_xor_sync(0xffffffffu, s01, 1);
-      if (on && l == 0) eb[kb] = valid ? (s01 + o2) / (float)(105 * CH) : 0.0f;
+      if (on && l == 0 && kb >= 2 * FH && kb < 2 * (FH + FT) && b < 2 * a.Le) a.mid.eb[b] = valid ? (s01 + o2) / (float)(105 * CH) : 0.0f;
     }
 
     // ---- S2b: zero crossings.  Sign changes between neighbouring samples, two samples (mono) or both
@@ -489,6 +501,14 @@ __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
       }
     }
 
+    __syncthreads();   // sig is dead from here on: it receives the next tile while S2c runs
+    const int64_t next = s_next;
+    if (tid == 0 && bulk_ok(next)) bulk_issue(next);
+    for (int k = tid; k < FT; k += THREADS) {
+      const int64_t f = t0 + k;
+      if (f < a.L) a.mid.zi[f] = zi[FH + k];
+    }
+
     // ---- S2c: lp2 = downsample_blur(lp1, 7, 3), 7 phases x 3 taps (f32), the band-1 residual energy at
     //      1260 Hz from the middle seven entries of the same window, and the band-2 energy of a frame
     //      (f64, :583/:588) from its six lp2 values by shuffles: a warp takes five frames (30 lanes) ----------
@@ -523,7 +543,8 @@ __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
             r1 = (i == 0) ? sq : r1 + sq;
           }
         }
-        if (act) { lp2[k] = total; be1[k] = r1; }
+        const bool own = act && kf >= FH && kf < FH + FT;
+        if (own && n2 >= 0 && n2 < len2) a.mid.be1[n2] = r1;
         double acc2 = 0.0;
 #pragma unroll
         for (int i = 0; i < 6; ++i) {
@@ -531,109 +552,120 @@ __global__ void __launch_bounds__(THREADS, 2) features_kernel(FeatArgs a) {
           const double sq = x * x;
           acc2 = (i == 0) ? sq : acc2 + sq;
         }
-        if (act && i6 == 0) {
+        if (own && i6 == 0) {
           const int64_t f = f0 + kf;
-          be2[kf] = (f >= 0 && f < a.L) ? acc2 : 0.0;
+          if (f >= 0 && f < a.L) a.mid.be2[f] = acc2;
         }
       }
     }
-    __syncthreads();   // sig and lp1 are dead from here on: ph reuses lp1's space, sig receives the next tile
+    __syncthreads();   // lp1 and zi are dead from here on
+    tile = next;
+  }
+}
 
-    if (tid == 0) {
-      const int64_t nt = (int64_t)atomicAdd(a.ticket, 1u);
-      s_next = (int)nt;
-      if (bulk_ok(nt)) bulk_issue(nt);
+// The 210 Hz stage: a plain grid, one CTA per FR output frames.
+//   S3   band 0: 42 phases x 15 taps and band 1: 6 phases x 15 taps; each phase = f32 products accumulated in f64
+//        (B.2 iii).  One thread per (phase, run of TC frames), its window read from the scratch into registers
+//   S4   the five outputs, four thread roles per frame (one role per warp)
+// Scratch frames outside [0, L) (blocks outside [0, 2 Le)) read as zero, as the reference's zero padding does.
+template <int CH>
+__global__ void __launch_bounds__(THREADS2, 6) bands_kernel(BandArgs a) {
+  __shared__ float ph[FR * 42];
+  __shared__ float p1[FR * 6];
+  const float *w630 = g_tables, *w90 = g_tables + 630, *w15 = g_tables + 741, *w13 = g_tables + 756;
+  const int tid = threadIdx.x;
+  const int64_t t0 = (int64_t)blockIdx.x * FR;      // first output frame of this CTA
+
+  {
+    const int ch = tid / 48, pp = tid - ch * 48;
+    const bool b0 = pp < 42;
+    const int p = b0 ? pp : pp - 42;
+    const int np = b0 ? 42 : 6;
+    const float *src = (b0 ? a.mid.be0 : a.mid.be1) + p;
+    const float *w = (b0 ? w630 : w90) + p;
+    float *dst = (b0 ? ph : p1) + p;
+    const int tb = ch * TC;
+    // output frame t0 + tb + t uses frames t0 + tb + t - 7 .. + 7 (tap j <-> window entry t + j)
+    const int64_t fw = t0 + tb - 7;
+    float win[14 + TC], wr[15];
+    if (fw >= 0 && fw + 14 + TC <= a.L) {
+      const float *s = src + fw * np;
+#pragma unroll
+      for (int e = 0; e < 14 + TC; ++e) win[e] = __ldg(s + e * np);
+    } else {
+#pragma unroll
+      for (int e = 0; e < 14 + TC; ++e) win[e] = (fw + e >= 0 && fw + e < a.L) ? __ldg(src + (fw + e) * np) : 0.0f;
     }
-
-    // ---- S3: band 0: 42 phases x 15 taps and band 1: 6 phases x 15 taps; each phase = f32 products
-    //      accumulated in f64 (B.2 iii).  One thread per (phase, run of TC frames), window in registers.
-    {
-      constexpr int NCH = (FT + TC - 1) / TC;
-      for (int u = tid; u < 48 * NCH; u += THREADS) {
-        const int ch = u / 48, pp = u - ch * 48;
-        const bool b0 = pp < 42;
-        const int p = b0 ? pp : pp - 42;
-        const int np = b0 ? 42 : 6;
-        const float *src = (b0 ? be0 : be1) + p;
-        const float *w = (b0 ? w630 : w90) + p;
-        float *dst = (b0 ? ph : p1) + p;
-        const int tb = ch * TC;
-        // output frame t0 + t uses staged frames t + 1 .. t + 15 (tap j <-> frame t + 1 + j)
-        float win[14 + TC], wr[15];
 #pragma unroll
-        for (int e = 0; e < 14 + TC; ++e) win[e] = (tb + 1 + e < NF) ? src[(tb + 1 + e) * np] : 0.0f;
+    for (int j = 0; j < 15; ++j) wr[j] = __ldg(w + (14 - j) * np);
 #pragma unroll
-        for (int j = 0; j < 15; ++j) wr[j] = w[(14 - j) * np];
+    for (int t = 0; t < TC; ++t) {
+      if (t0 + tb + t < a.L) {
+        double acc = 0.0;
 #pragma unroll
-        for (int t = 0; t < TC; ++t) {
-          if (tb + t < FT) {
-            double acc = 0.0;
-#pragma unroll
-            for (int j = 0; j < 15; ++j) {
-              const float prod = win[t + j] * wr[j];
-              acc += (double)prod;
-            }
-            dst[(tb + t) * np] = (float)acc;
-          }
+        for (int j = 0; j < 15; ++j) {
+          const float prod = win[t + j] * wr[j];
+          acc += (double)prod;
         }
+        dst[(tb + t) * np] = (float)acc;
       }
     }
-    __syncthreads();
+  }
+  __syncthreads();
 
-    // ---- S4: outputs: four thread roles per frame ---------------------------------------------------------
-    for (int u = tid; u < 4 * FT; u += THREADS) {
-      const int role = u / FT, t = u - role * FT;
-      const int64_t f = t0 + t;
-      if (role == 0) {
-        if (f < a.L) {
-          // band 0: phases added sequentially in f32 (B.2 v), /210, log10(1+x)/2
-          float tot = 0.0f;
+  if (tid < 4 * FR) {
+    const int role = tid / FR, t = tid - role * FR;
+    const int64_t f = t0 + t;
+    if (role == 0) {
+      if (f < a.L) {
+        // band 0: phases added sequentially in f32 (B.2 v), /210, log10(1+x)/2
+        float tot = 0.0f;
 #pragma unroll 6
-          for (int p = 0; p < 42; ++p) tot = tot + ph[t * 42 + p];
-          a.b0[f] = host_log10f(1.0f + tot / 210.0f) / 2.0f;
-        }
-      } else if (role == 1) {
-        if (f < a.L) {
-          float tot = 0.0f;
+        for (int p = 0; p < 42; ++p) tot = tot + ph[t * 42 + p];
+        a.b0[f] = host_log10f(1.0f + tot / 210.0f) / 2.0f;
+      }
+    } else if (role == 1) {
+      if (f < a.L) {
+        float tot = 0.0f;
 #pragma unroll
-          for (int p = 0; p < 6; ++p) tot = tot + p1[t * 6 + p];
-          a.b1[f] = host_log10f(1.0f + tot / 210.0f) / 2.0f;
-          // zero crossings: 13-tap Hann over frames f-6 .. f+6
-          double acc = 0.0;
+        for (int p = 0; p < 6; ++p) tot = tot + p1[t * 6 + p];
+        a.b1[f] = host_log10f(1.0f + tot / 210.0f) / 2.0f;
+        // zero crossings: 13-tap Hann over frames f-6 .. f+6
+        double acc = 0.0;
 #pragma unroll
-          for (int j = 0; j < 13; ++j) {
-            float z = (float)zi[t + FH - 6 + j];
-            if (CH == 1) z = z * 2.0f;
-            const float prod = z * w13[12 - j];
-            acc += (double)prod;
-          }
-          a.zc[f] = (float)acc;
+        for (int j = 0; j < 13; ++j) {
+          const int64_t g = f - 6 + j;
+          float z = (g >= 0 && g < a.L) ? (float)a.mid.zi[g] : 0.0f;
+          if (CH == 1) z = z * 2.0f;
+          const float prod = z * w13[12 - j];
+          acc += (double)prod;
         }
-      } else if (role == 2) {
-        if (f < a.L) {
-          // band 2: one 15-tap f64 filter = OpenBLAS ddot tail, a sequential FMA chain (B.2 iv)
-          double acc = 0.0;
+        a.zc[f] = (float)acc;
+      }
+    } else if (role == 2) {
+      if (f < a.L) {
+        // band 2: one 15-tap f64 filter = OpenBLAS ddot tail, a sequential FMA chain (B.2 iv)
+        double acc = 0.0;
 #pragma unroll
-          for (int j = 0; j < 15; ++j) acc = fma((double)w15[14 - j], be2[t + 1 + j], acc);
-          a.b2[f] = log10(1.0 + acc / 210.0) / 2.0;
+        for (int j = 0; j < 15; ++j) {
+          const int64_t g = f - 7 + j;
+          acc = fma((double)w15[14 - j], (g >= 0 && g < a.L) ? a.mid.be2[g] : 0.0, acc);
         }
-      } else {
-        if (f < a.Le) {
-          // energy: 13-tap Hann over blocks 2f-6 .. 2f+6, log10(1+x)/2, every second block (:553-555)
-          double acc = 0.0;
+        a.b2[f] = log10(1.0 + acc / 210.0) / 2.0;
+      }
+    } else {
+      if (f < a.Le) {
+        // energy: 13-tap Hann over blocks 2f-6 .. 2f+6, log10(1+x)/2, every second block (:553-555)
+        double acc = 0.0;
 #pragma unroll
-          for (int j = 0; j < 13; ++j) {
-            const float prod = eb[2 * (t + FH) - 6 + j] * w13[12 - j];
-            acc += (double)prod;
-          }
-          a.energy[f] = host_log10f(1.0f + (float)acc) / 2.0f;
+        for (int j = 0; j < 13; ++j) {
+          const int64_t b = 2 * f - 6 + j;
+          const float prod = ((b >= 0 && b < 2 * a.Le) ? a.mid.eb[b] : 0.0f) * w13[12 - j];
+          acc += (double)prod;
         }
+        a.energy[f] = host_log10f(1.0f + (float)acc) / 2.0f;
       }
     }
-    // No barrier here: S4 reads ph (= lp1's space), p1, zi, eb and be2, all of which are next written after the next
-    // tile's first barrier, which no thread passes before every thread has left S4.  s_next was written before the S3
-    // barrier of this tile and is rewritten after the S2 barrier of the next one.
-    tile = s_next;
   }
 }
 
@@ -669,7 +701,7 @@ std::mutex g_fix_mu;
 void *g_fix_buf[64] = {};      // per device: the uploaded correction table
 
 template <int FMT, int CH>
-int launch(dab_pair *pr, const FeatArgs &fa_in, int64_t frames) {
+int launch(dab_pair *pr, const FeatArgs &fa_in, const BandArgs &ba, int64_t frames) {
   dab_ctx *ctx = pr->ctx;
   const int64_t tiles = cdiv(frames, Tile<CH>::FT);
   if (tiles <= 0) return DAB_OK;
@@ -681,6 +713,9 @@ int launch(dab_pair *pr, const FeatArgs &fa_in, int64_t frames) {
   DAB_CUDA(cudaMemsetAsync(fa.ticket, 0, sizeof(unsigned int), pr->stream));
   const int64_t grid = tiles < 2 * (int64_t)ctx->sm_count ? tiles : 2 * (int64_t)ctx->sm_count;
   features_kernel<FMT, CH><<<(unsigned)grid, THREADS, smem, pr->stream>>>(fa);
+  DAB_LAUNCHED(pr);
+  DAB_CUDA(cudaGetLastError());
+  bands_kernel<CH><<<(unsigned)cdiv(frames, FR), THREADS2, 0, pr->stream>>>(ba);
   DAB_LAUNCHED(pr);
   DAB_CUDA(cudaGetLastError());
   return DAB_OK;
@@ -748,18 +783,33 @@ int dab_run_features(dab_pair *pr, int track, const void *d_pcm, int format) {
   DAB_TRY(dab_ensure(ctx, tk.b1, sizeof(float) * (size_t)(L + 1)));
   DAB_TRY(dab_ensure(ctx, tk.b2, sizeof(double) * (size_t)(L + 1)));
   DAB_TRY(dab_ensure(ctx, tk.feat_ticket, 64));
+  // the scratch between the two kernels: 212 B per frame, each section 256-byte aligned
+  size_t off = 0;
+  auto section = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
+  const size_t o_be2 = section(sizeof(double) * (size_t)L), o_be0 = section(sizeof(float) * 42 * (size_t)L),
+               o_be1 = section(sizeof(float) * 6 * (size_t)L), o_eb = section(sizeof(float) * 2 * (size_t)Le),
+               o_zi = section(sizeof(int) * (size_t)L);
+  DAB_TRY(dab_ensure(ctx, tk.feat_mid, off + 256));
+  unsigned char *mid = tk.feat_mid.as<unsigned char>();
+  FeatMid fm;
+  fm.be0 = reinterpret_cast<float *>(mid + o_be0); fm.be1 = reinterpret_cast<float *>(mid + o_be1);
+  fm.be2 = reinterpret_cast<double *>(mid + o_be2); fm.eb = reinterpret_cast<float *>(mid + o_eb);
+  fm.zi = reinterpret_cast<int *>(mid + o_zi);
   FeatArgs fa;
   fa.tiles = 0;
   fa.ticket = tk.feat_ticket.as<unsigned int>();
   fa.pcm = d_pcm; fa.S = tk.S; fa.L = L; fa.nb = nb; fa.Le = Le;
   fa.vec_ok = (reinterpret_cast<uintptr_t>(d_pcm) & 15u) == 0;
-  fa.energy = tk.energy.as<float>(); fa.zc = tk.zc.as<float>();
-  fa.b0 = tk.b0.as<float>(); fa.b1 = tk.b1.as<float>(); fa.b2 = tk.b2.as<double>();
+  fa.mid = fm;
+  BandArgs ba;
+  ba.mid = fm; ba.L = L; ba.Le = Le;
+  ba.energy = tk.energy.as<float>(); ba.zc = tk.zc.as<float>();
+  ba.b0 = tk.b0.as<float>(); ba.b1 = tk.b1.as<float>(); ba.b2 = tk.b2.as<double>();
   const int64_t frames = Le > L ? Le : L;
-  if (format == DAB_PCM_S16 && tk.ch == 1) DAB_TRY((launch<DAB_PCM_S16, 1>(pr, fa, frames)));
-  else if (format == DAB_PCM_S16 && tk.ch == 2) DAB_TRY((launch<DAB_PCM_S16, 2>(pr, fa, frames)));
-  else if (format == DAB_PCM_F16 && tk.ch == 1) DAB_TRY((launch<DAB_PCM_F16, 1>(pr, fa, frames)));
-  else if (format == DAB_PCM_F16 && tk.ch == 2) DAB_TRY((launch<DAB_PCM_F16, 2>(pr, fa, frames)));
+  if (format == DAB_PCM_S16 && tk.ch == 1) DAB_TRY((launch<DAB_PCM_S16, 1>(pr, fa, ba, frames)));
+  else if (format == DAB_PCM_S16 && tk.ch == 2) DAB_TRY((launch<DAB_PCM_S16, 2>(pr, fa, ba, frames)));
+  else if (format == DAB_PCM_F16 && tk.ch == 1) DAB_TRY((launch<DAB_PCM_F16, 1>(pr, fa, ba, frames)));
+  else if (format == DAB_PCM_F16 && tk.ch == 2) DAB_TRY((launch<DAB_PCM_F16, 2>(pr, fa, ba, frames)));
   else { dab_set_err(ctx, "unsupported PCM format / channel count"); return DAB_E_ARG; }
   tk.have_features = true;
   return DAB_OK;
