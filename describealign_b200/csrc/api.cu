@@ -84,6 +84,15 @@ static void free_buf(DevBuf &b) {
   b.cap = 0;
 }
 
+static void free_prep(Prep &p) {
+  for (DevBuf *b : {&p.ms, &p.nrm, &p.pack, &p.code, &p.nq_flag, &p.nq_list}) free_buf(*b);
+}
+
+static void free_video_side(VideoSide &vs) {
+  free_prep(vs.prep);
+  for (DevBuf *b : {&vs.tbl_start, &vs.tbl_items, &vs.v_rec}) free_buf(*b);
+}
+
 extern "C" {
 
 int dab_abi_version(void) { return DAB_ABI_VERSION; }
@@ -228,6 +237,26 @@ cudaError_t dab_readback(dab_pair *pr, void *host_dst, const void *dev_src, size
   return cudaGetLastError();
 }
 
+// a stage-A step enqueued on the pair's stream, waited for and collected; run again while the collect reports an
+// overflow (it has grown the buffer)
+template <typename Enqueue, typename Collect>
+static int grow_and_retry(dab_pair *pr, Enqueue enqueue, Collect collect) {
+  dab_ctx *ctx = pr->ctx;
+  int rc = DAB_E_CAPACITY;
+  for (int attempt = 0; attempt < DAB_STAGE_A_ATTEMPTS && rc == DAB_E_CAPACITY; ++attempt) {
+    DAB_TRY(enqueue());
+    DAB_CUDA(dab_wait_stream(pr->stream));
+    rc = collect();
+  }
+  return rc;
+}
+
+// stage A against a shared index, or against the pair's own video side (ix null)
+static int stage_a_sync(dab_pair *pr, const dab_index *ix, int64_t row_lo, int64_t row_hi, bool with_dp) {
+  return grow_and_retry(pr, [&] { return dab_enqueue_stage_a(pr, ix, row_lo, row_hi, with_dp); },
+                        [&] { return dab_collect_stage_a(pr, ix, with_dp); });
+}
+
 extern "C" {
 
 void dab_pair_destroy(dab_pair *pr);
@@ -264,10 +293,12 @@ void dab_pair_destroy(dab_pair *pr) {
   if (pr->stream) dab_wait_stream(pr->stream);
   for (int t = 0; t < 2; ++t) {
     Track &k = pr->trk[t];
-    DevBuf *bs[] = {&k.pcm, &k.feat_ticket, &k.feat_mid, &k.energy, &k.zc, &k.b0, &k.b1, &k.b2, &k.gate, &k.ms, &k.nrm, &k.pack, &k.code, &k.nq_flag, &k.nq_list};
+    DevBuf *bs[] = {&k.pcm, &k.feat_ticket, &k.feat_mid, &k.energy, &k.zc, &k.b0, &k.b1, &k.b2, &k.gate};
     for (DevBuf *b : bs) free_buf(*b);
   }
-  DevBuf *bs[] = {&pr->scan_tmp, &pr->tbl_start, &pr->tbl_items, &pr->tbl_sb, &pr->tbl_ent, &pr->v_rec, &pr->clusters, &pr->refine_partial, &pr->maxes, &pr->row_count, &pr->row_off, &pr->row_stash, &pr->gate_rec, &pr->gate_best, &pr->gate_big,
+  free_prep(pr->prep_a);
+  free_video_side(pr->video);
+  DevBuf *bs[] = {&pr->scan_tmp, &pr->tbl_sb, &pr->tbl_ent, &pr->clusters, &pr->refine_partial, &pr->maxes, &pr->row_count, &pr->row_off, &pr->row_stash, &pr->gate_rec, &pr->gate_best, &pr->gate_big,
                   &pr->cand_tmp, &pr->cand_s, &pr->cand_i, &pr->cand_q, &pr->keep_flag, &pr->keep_off, &pr->pt_i,
                   &pr->pt_s, &pr->pt_q, &pr->counters, &pr->tree1, &pr->back1, &pr->dpres,
                   &pr->path1_x, &pr->path1_y, &pr->a_scaled, &pr->v_scaled, &pr->corridors,
@@ -309,7 +340,7 @@ int dab_pair_set_pcm(dab_pair *pr, int track, const void *pcm, int64_t samples, 
   tk.ch = channels;
   tk.have_features = false;
   tk.have_gate = false;
-  pr->matched = false;
+  if (pr->points_side == &pr->video) pr->points_side = nullptr;
   if (track == DAB_TRACK_VIDEO) { pr->api_us[1] = pr->api_us[2] = pr->api_us[3] = 0; }
   const void *d_pcm = pcm;
   cudaEvent_t e0 = pr->ev[2 * track], e1 = pr->ev[2 * track + 1];
@@ -343,7 +374,7 @@ int dab_pair_set_features(dab_pair *pr, int track, const float *energy, int64_t 
   tk.Le = n_energy;
   tk.S = n * 210;
   tk.have_gate = false;
-  pr->matched = false;
+  if (pr->points_side == &pr->video) pr->points_side = nullptr;
   DAB_TRY(dab_ensure(ctx, tk.energy, sizeof(float) * (size_t)(n_energy + 1)));
   DAB_TRY(dab_ensure(ctx, tk.zc, sizeof(float) * (size_t)(n + 1)));
   DAB_TRY(dab_ensure(ctx, tk.b0, sizeof(float) * (size_t)(n + 1)));
@@ -373,7 +404,7 @@ int dab_pair_set_gate_energy(dab_pair *pr, int track, const float *energy, int64
   DAB_CUDA(cudaMemcpyAsync(tk.gate.p, energy, sizeof(float) * (size_t)n_energy, cudaMemcpyHostToDevice, pr->stream));
   DAB_CUDA(dab_wait_stream(pr->stream));
   tk.have_gate = true;
-  pr->matched = false;
+  if (pr->points_side == &pr->video) pr->points_side = nullptr;
   return DAB_OK;
 }
 
@@ -406,18 +437,6 @@ int dab_pair_get_features(dab_pair *pr, int track, float *energy, float *zc, flo
   return DAB_OK;
 }
 
-// stage A enqueued, waited for and collected; run again while a buffer overflows
-static int stage_a_sync(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp) {
-  dab_ctx *ctx = pr->ctx;
-  int rc = DAB_E_CAPACITY;
-  for (int attempt = 0; attempt < DAB_STAGE_A_ATTEMPTS && rc == DAB_E_CAPACITY; ++attempt) {
-    DAB_TRY(dab_enqueue_stage_a(pr, row_lo, row_hi, with_dp));
-    DAB_CUDA(dab_wait_stream(pr->stream));
-    rc = dab_collect_stage_a(pr, with_dp);
-  }
-  return rc;
-}
-
 int dab_pair_stage_a(dab_pair *pr, int64_t *n_points, int64_t *n_path) {
   if (!pr) return DAB_E_ARG;
   dab_ctx *ctx = pr->ctx;
@@ -425,7 +444,7 @@ int dab_pair_stage_a(dab_pair *pr, int64_t *n_points, int64_t *n_path) {
   ApiTimer timer__(&pr->api_us[1]);
   DAB_TRY(dab_check_stage_a_inputs(pr, "stage_a"));
   DAB_CUDA(cudaSetDevice(ctx->device));
-  DAB_TRY(stage_a_sync(pr, 0, INT64_MAX, true));
+  DAB_TRY(stage_a_sync(pr, nullptr, 0, INT64_MAX, true));
   if (n_points) *n_points = pr->n_points1;
   if (n_path) *n_path = pr->n_path1;
   return DAB_OK;
@@ -458,7 +477,7 @@ extern "C" {
 
 static int export_points1(dab_pair *pr, int32_t *i_audio, int32_t *v_video, double *qual, int dst_on_device) {
   dab_ctx *ctx = pr->ctx;
-  if (pr->points_from_index) {
+  if (pr->points_side && pr->points_side != &pr->video) {
     dab_set_err(ctx, "export_points1: the points of stage_a_against are ranks into the index's hashed frames, not this pair's");
     return DAB_E_STATE;
   }
@@ -474,7 +493,7 @@ static int export_points1(dab_pair *pr, int32_t *i_audio, int32_t *v_video, doub
     if (v_video) {
       DAB_TRY(dab_ensure(ctx, pr->cand_tmp, sizeof(int32_t) * (size_t)(n + 1)));
       ranks_to_frames_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(pr->pt_s.as<int32_t>(),
-                                                                      pr->trk[DAB_TRACK_VIDEO].nq_list.as<int32_t>(), n,
+                                                                      pr->video.prep.nq_list.as<int32_t>(), n,
                                                                       pr->cand_tmp.as<int32_t>());
       ctx->launches += 1;
       DAB_CUDA(cudaMemcpyAsync(v_video, pr->cand_tmp.p, sizeof(int32_t) * (size_t)n, kind, st));
@@ -495,9 +514,8 @@ int dab_pair_export_points1(dab_pair *pr, int32_t *i_audio, int32_t *v_video, do
 }
 
 static void index_destroy(dab_index *ix) {
-  DevBuf *bs[] = {&ix->V.ms, &ix->V.nrm, &ix->V.pack, &ix->V.code, &ix->V.nq_flag, &ix->V.nq_list,
-                  &ix->tbl_start, &ix->tbl_items, &ix->v_rec, &ix->counters};
-  for (DevBuf *b : bs) free_buf(*b);
+  free_video_side(ix->side);
+  free_buf(ix->counters);
   if (ix->ready) cudaEventDestroy(ix->ready);
   delete ix;
 }
@@ -517,7 +535,10 @@ int dab_index_build(dab_pair *src, dab_index **out) {
   int rc = DAB_OK;
   const cudaError_t e = cudaEventCreateWithFlags(&ix->ready, cudaEventDisableTiming);
   if (e != cudaSuccess) { dab_set_err(ctx, std::string("index_build: ") + cudaGetErrorString(e)); rc = DAB_E_CUDA; }
-  if (rc == DAB_OK) rc = dab_build_index(src, ix);
+  if (rc == DAB_OK) {
+    rc = grow_and_retry(src, [&] { return dab_enqueue_index(src, ix); }, [&] { return dab_collect_index(src, ix); });
+    if (rc == DAB_E_CAPACITY) dab_set_err(ctx, "dab_index_build: the hash tables overflowed on every attempt");
+  }
   if (rc != DAB_OK) {
     dab_wait_stream(src->stream);
     index_destroy(ix);
@@ -541,7 +562,7 @@ int dab_index_free(dab_index *ix) {
 
 int dab_index_info(const dab_index *ix, int64_t out[4]) {
   if (!ix || !out) return DAB_E_ARG;
-  out[0] = ix->V.L; out[1] = ix->n_vsel; out[2] = ix->n_entries; out[3] = ix->users.load();
+  out[0] = ix->side.prep.L; out[1] = ix->side.n_vsel; out[2] = ix->side.n_entries; out[3] = ix->users.load();
   return DAB_OK;
 }
 
@@ -563,13 +584,7 @@ int dab_pair_stage_a_against(dab_pair *pr, const dab_index *ix, int64_t *n_point
     ~Release() { ix->users.fetch_sub(1); }
   } release__{ix};
   DAB_CUDA(cudaSetDevice(ctx->device));
-  int rc = DAB_E_CAPACITY;
-  for (int attempt = 0; attempt < DAB_STAGE_A_ATTEMPTS && rc == DAB_E_CAPACITY; ++attempt) {
-    DAB_TRY(dab_enqueue_stage_a_against(pr, ix));
-    DAB_CUDA(dab_wait_stream(pr->stream));
-    rc = dab_collect_stage_a_against(pr, ix);
-  }
-  DAB_TRY(rc);
+  DAB_TRY(stage_a_sync(pr, ix, 0, INT64_MAX, true));
   if (n_points) *n_points = pr->n_points1;
   if (n_path) *n_path = pr->n_path1;
   return DAB_OK;
@@ -583,7 +598,7 @@ int dab_pair_stage_a_match(dab_pair *pr, int64_t row_lo, int64_t row_hi, int64_t
   if (row_lo < 0 || row_hi < row_lo) { dab_set_err(ctx, "dab_pair_stage_a_match: invalid row range"); return DAB_E_ARG; }
   DAB_TRY(dab_check_stage_a_inputs(pr, "stage_a_match"));
   DAB_CUDA(cudaSetDevice(ctx->device));
-  DAB_TRY(stage_a_sync(pr, row_lo, row_hi, false));
+  DAB_TRY(stage_a_sync(pr, nullptr, row_lo, row_hi, false));
   if (n_points) *n_points = pr->n_points1;
   return DAB_OK;
 }
@@ -594,7 +609,7 @@ int dab_pair_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t 
   dab_ctx *ctx = pr->ctx;
   StreamScope scope__(pr->stream);
   if (n < 0 || (n > 0 && (!i_audio || !v_video || !qual))) { dab_set_err(ctx, "dab_pair_import_points1: invalid argument"); return DAB_E_ARG; }
-  if (!pr->matched) { dab_set_err(ctx, "import_points1: run stage_a_match on this pair first (it builds the hashed-frame list)"); return DAB_E_STATE; }
+  if (pr->points_side != &pr->video) { dab_set_err(ctx, "import_points1: run stage_a_match on this pair first (it builds the hashed-frame list)"); return DAB_E_STATE; }
   DAB_CUDA(cudaSetDevice(ctx->device));
   return dab_run_import_points1(pr, i_audio, v_video, qual, n, src_on_device);
 }
@@ -604,7 +619,7 @@ int dab_pair_dp1(dab_pair *pr, int64_t *n_path) {
   dab_ctx *ctx = pr->ctx;
   StreamScope scope__(pr->stream);
   ApiTimer timer__(&pr->api_us[1]);
-  if (!pr->matched) { dab_set_err(ctx, "dp1: no match points (run stage_a_match / import_points1 first)"); return DAB_E_STATE; }
+  if (pr->points_side != &pr->video) { dab_set_err(ctx, "dp1: no match points (run stage_a_match / import_points1 first)"); return DAB_E_STATE; }
   DAB_CUDA(cudaSetDevice(ctx->device));
   DAB_TRY(dab_enqueue_stage_a_dp(pr));
   DAB_TRY(dab_enqueue_counts(pr));

@@ -32,7 +32,7 @@ struct dab_ctx {
   int opt_dp2_impl = 0;      // 0 scan kernel (dp2_scan.cuh), 2 generic tree DP (both exact; the tests compare them)
 };
 
-// Features and prep data of one track, device resident.
+// Features of one track, device resident.
 struct Track {
   int64_t S = 0;       // samples per channel
   int ch = 1;
@@ -45,15 +45,29 @@ struct Track {
   DevBuf feat_mid;     // per-frame intermediates between the two feature kernels (features.cu: FeatMid), 212 B per frame
   DevBuf gate;         // the separate *_energy argument of align() when it is not features[0] (:629, :657)
   bool have_gate = false;
-  // stage A prep (features 0..2 keep ms / nrm for scoring; 3, 4 only feed the codes)
+};
+
+// Stage-A prep of one track's features (features 0..2 keep ms / nrm for scoring; 3, 4 only feed the codes)
+struct Prep {
+  int64_t L = 0, Le = 0;   // the feature lengths it was made from
   DevBuf ms;           // f64 [3][Lp]   Lp = min feature length
   DevBuf nrm;          // f64 [3][Lp-40]
   DevBuf pack;         // u32 [5][Lp-40] one digit per nibble (bits 0-2), bit 3 of the nibble = flag (video)
   DevBuf code;         // i32 [5][Lp-40] base-7 code (audio: lookup key)
-  DevBuf nq_flag;      // i32 [n] not-quiet flags, then reused
+  DevBuf nq_flag;      // i32 [n] not-quiet flags, then their exclusive scan
   DevBuf nq_list;      // i32 selected frame list (video: every 4th not-quiet; audio: all not-quiet)
-  int64_t n_codes = 0; // Lp - 40
-  int64_t n_list = 0;
+};
+
+// The video side of the match stage, as the gate, scoring and DP 1 read it: the video track's prep, the hash tables
+// over its hashed frames and the records of those frames.  A pair builds its own in every stage-A run; a shared
+// index (dab_index) builds one once, and any number of pairs then only read it.
+struct VideoSide {
+  Prep prep;
+  DevBuf tbl_start;   // i32 [5*NCODE + 1]
+  DevBuf tbl_items;   // i32 sel-ranks
+  DevBuf v_rec;       // uint4[2] per hashed video frame: its five digit packs (gate)
+  int64_t n_vsel = 0, n_entries = 0;   // hashed frames, table entries
+  int64_t cap_entries = 0;             // capacity of the tables (grown on overflow)
 };
 
 // What one stage-B call decided, read by every later step of that call (points, DP 2, the exchange of
@@ -75,12 +89,15 @@ struct dab_pair {
   // scan scratch
   DevBuf scan_tmp;            // single-pass scan: ticket counter + tile status words
   unsigned int scan_epoch = 0;
-  // tables
-  DevBuf tbl_start;   // i32 [5*NCODE + 1]
-  DevBuf tbl_items;   // i32 sel-ranks
+  // stage A
+  Prep prep_a;                // of the audio track
+  VideoSide video;            // of the video track
+  // the video side whose hashed frames the pass-1 points refer to: &video, a shared index's (export refused), or
+  // null (a run in flight, or the own side out of date after new features).  Only compared, never read through.
+  const VideoSide *points_side = nullptr;
+  // table build scratch
   DevBuf tbl_sb;      // i32: per super-bucket of 4096 slots its entry count, offset (+ total) and scatter cursor
   DevBuf tbl_ent;     // u32 x2 [entries]: (slot within its super-bucket, rank), grouped by super-bucket
-  DevBuf v_rec;       // uint4[2] per hashed video frame: its five digit packs (gate)
   // gate / scoring
   DevBuf row_count, row_off;   // i32 [n_queries + 1]
   DevBuf row_stash;            // i32 [n_queries][4]: first candidates of each row (gate count pass)
@@ -97,9 +114,7 @@ struct dab_pair {
   DevBuf dpres;                // i32/i64 results (end id, path len)
   DevBuf path1_x, path1_y;     // i32
   int64_t n_points1 = 0, n_path1 = 0;
-  int64_t cap_entries = 0, cap_cand = 0, cap_points1 = 0;   // capacities of device-sized buffers (grown on overflow)
-  bool matched = false;        // tables / hashed-frame list of the current features are built
-  bool points_from_index = false;   // the pass-1 points are ranks into a shared index's hashed-frame list
+  int64_t cap_cand = 0, cap_points1 = 0;   // capacities of device-sized buffers (grown on overflow)
   // stage B
   DevBuf a_scaled, v_scaled;   // f32 (n,3)
   DevBuf corridors;            // dab_corridor[]
@@ -127,16 +142,12 @@ struct dab_pair {
   int64_t api_us[4] = {0, 0, 0, 0};
 };
 
-// The video side of the match stage, built once per video and then only read: any number of pairs, each on its
-// own stream, run their description track against it (dab_pair_stage_a_against).  V holds the prep buffers (ms,
-// nrm, digit packs and codes, not-quiet flags and the hashed-frame list) but no features.
+// A video side built once per video and then only read: any number of pairs, each on its own stream, run their
+// description track against it (dab_pair_stage_a_against).
 struct dab_index {
   dab_ctx *ctx = nullptr;           // the context of the pair it was built from (device, error messages)
-  Track V;
-  DevBuf tbl_start, tbl_items;      // hash tables, sized when the index is built
-  DevBuf v_rec;                     // records of the hashed frames (gate)
+  VideoSide side;
   DevBuf counters;                  // the build's device counts
-  int64_t n_vsel = 0, n_entries = 0, cap_entries = 0;
   cudaEvent_t ready = nullptr;      // recorded after the last command of the build; every user's stream waits on it
   mutable std::atomic<int> users{0};   // stage-A calls running against the index; -1 once it is being freed
 };
@@ -233,15 +244,16 @@ int dab_enqueue_counts(dab_pair *pr);
 // entries overflow leaves the tables empty, so the candidate total is only known one run later: three runs at most.
 constexpr int DAB_STAGE_A_ATTEMPTS = 8;
 int dab_check_stage_a_inputs(dab_pair *pr, const char *who);
-// match points of audio rows [row_lo, row_hi), then DP 1 + traceback if with_dp, then the counts
-int dab_enqueue_stage_a(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp);
-int dab_enqueue_stage_a_dp(dab_pair *pr);      // DP 1 + traceback over the pair's points
-int dab_collect_stage_a(dab_pair *pr, bool with_dp);
-// shared video index: build (synchronous: the tables' capacity is settled here) and the match stage against it
-int dab_build_index(dab_pair *src, dab_index *ix);
-int dab_enqueue_stage_a_against(dab_pair *pr, const dab_index *ix);
-int dab_collect_stage_a_against(dab_pair *pr, const dab_index *ix);
+// match points of audio rows [row_lo, row_hi) against a shared index (ix), or against the pair's own video side,
+// built in the same run; then DP 1 + traceback if with_dp, then the counts
+int dab_enqueue_stage_a(dab_pair *pr, const dab_index *ix, int64_t row_lo, int64_t row_hi, bool with_dp);
+int dab_collect_stage_a(dab_pair *pr, const dab_index *ix, bool with_dp);
+int dab_enqueue_stage_a_dp(dab_pair *pr);      // DP 1 + traceback over the pair's points (its own video side)
 void dab_collect_stage_a_dp(dab_pair *pr);
+// the video side of src's video track into ix, then the counts (to src's mapped page); the collect records
+// ix->ready, or grows the tables after an overflow and returns DAB_E_CAPACITY
+int dab_enqueue_index(dab_pair *src, dab_index *ix);
+int dab_collect_index(dab_pair *src, dab_index *ix);
 int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *v_video, const double *qual,
                            int64_t n, int src_on_device);
 // Stage B.  Its sizes come from pr->plan_b, set by device planning from clusters or by the explicit upload of

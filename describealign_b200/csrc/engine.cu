@@ -114,7 +114,7 @@ void enqueue_a(dab_engine *e, int slot, bool upload) {
               DAB_EVENT_STAGE_A);
   }
   ENG_TRY(dab_check_stage_a_inputs(pr, "stage_a"), DAB_EVENT_STAGE_A);
-  ENG_TRY(dab_enqueue_stage_a(pr, 0, INT64_MAX, true), DAB_EVENT_STAGE_A);
+  ENG_TRY(dab_enqueue_stage_a(pr, nullptr, 0, INT64_MAX, true), DAB_EVENT_STAGE_A);
   ENG_CUDA(cudaEventRecord(s.ev, pr->stream), DAB_EVENT_STAGE_A);
   s.state = S_A_RUN;
   s.host_us += now_us() - t0;
@@ -127,7 +127,7 @@ void after_a(dab_engine *e, int slot) {
   dab_pair *pr = s.pair;
   StreamScope scope__(pr->stream);
   const int64_t t0 = now_us();
-  const int rc = dab_collect_stage_a(pr, true);
+  const int rc = dab_collect_stage_a(pr, nullptr, true);
   if (rc == DAB_E_CAPACITY && ++s.attempts < DAB_STAGE_A_ATTEMPTS) { enqueue_a(e, slot, false); return; }
   ENG_TRY(rc, DAB_EVENT_STAGE_A);
   cudaStream_t st = pr->stream;

@@ -14,6 +14,10 @@
 // reference becomes a counting-sort CSR (start[code], items[]) per table: 7^7 = 823 543
 // codes x 5 tables x 4 B = 16.5 MB of starts, L2 resident.  The gate is evaluated as an
 // integer predicate on packed 3-bit digits, so a bucket entry costs five 4-byte loads.
+//
+// The video's prep, select and tables make up a VideoSide (common.cuh).  dab_enqueue_stage_a builds the pair's own
+// in the same run, or runs against a shared index, built once by dab_enqueue_index; gate, scoring and DP 1 only
+// read the side they are given.
 #include "common.cuh"
 #include "hann_tables.h"
 
@@ -1108,14 +1112,14 @@ static __global__ void check_capacity_kernel(int32_t *dc, int word, int need_wor
   if ((int64_t)dc[word] > cap) { dc[word] = 0; atomicOr(&dc[DC_OVERFLOW], bit); }
 }
 
-// Prep of one track's features `in` into the stage-A buffers of `out` (the same track, or a video index).
-static int prep_track(dab_pair *pr, const Track &in, Track &out, bool is_video) {
+// Prep of one track's features `in` into `out` (the pair's audio prep, or the prep of a video side).
+static int prep_track(dab_pair *pr, const Track &in, Prep &out, bool is_video) {
   dab_ctx *ctx = pr->ctx;
   const Track &tk = in;
   const int64_t Lmax = tk.Le > tk.L ? tk.Le : tk.L;
   const int64_t Lmin = tk.Le < tk.L ? tk.Le : tk.L;
   const int64_t nc = Lmax - 40;     // stride of the code arrays (energy may have one more)
-  out.n_codes = Lmin - 40;
+  out.L = tk.L; out.Le = tk.Le;
   DAB_TRY(dab_ensure(ctx, out.ms, sizeof(double) * (size_t)(5 * Lmax)));
   DAB_TRY(dab_ensure(ctx, out.nrm, sizeof(double) * (size_t)(3 * nc)));
   DAB_TRY(dab_ensure(ctx, out.pack, sizeof(uint32_t) * (size_t)(5 * nc)));
@@ -1153,6 +1157,14 @@ static int prep_track(dab_pair *pr, const Track &in, Track &out, bool is_video) 
   return DAB_OK;
 }
 
+// counts_lists_kernel over the not-quiet scans of the video prep V and the audio prep A
+static void enqueue_counts_lists(dab_pair *pr, int32_t *dc, const Prep &V, const Prep &A, int64_t row_lo, int64_t row_hi) {
+  const int64_t v_nq = V.Le - 41, a_nq = A.Le - 41;
+  counts_lists_kernel<<<1, 32, 0, pr->stream>>>(dc, V.nq_flag.as<int32_t>() + (v_nq + 1), v_nq, A.nq_flag.as<int32_t>() + (a_nq + 1),
+                                                a_nq, row_lo, row_hi);
+  pr->ctx->launches += 1;
+}
+
 static int ensure_hann(dab_ctx *ctx) {
   static std::atomic<int> ready[64];
   int dev = 0;
@@ -1171,60 +1183,57 @@ static int ensure_hann(dab_ctx *ctx) {
 // Capacities of the buffers whose fill level only the device knows (table entries, candidates).  They
 // start from what pairs of this size normally need and double when a run overflows (the overflow bit
 // comes back with the counts; the stage is then run again - rare, and only ever during the first pairs).
-static int64_t first_entries_cap(const Track &V) {
-  return 5 * 16 * ((V.Le - 41 + 3) / 4 + 1) + 4096;     // ~10 expanded entries per frame and table (SURVEY.md D)
+static int64_t video_sel_ub(int64_t v_Le) { return (v_Le - 41 + 3) / 4 + 1; }
+static int64_t first_entries_cap(int64_t v_Le) {
+  return 5 * 16 * video_sel_ub(v_Le) + 4096;            // ~10 expanded entries per frame and table (SURVEY.md D)
 }
-static int64_t first_cand_cap(const Track &A) {
-  return 2 * (A.Le - 41) + 4096;                         // < 1 candidate per query on matching tracks
-}
-static void default_caps(dab_pair *pr) {
-  const int64_t want_e = first_entries_cap(pr->trk[DAB_TRACK_VIDEO]);
-  const int64_t want_c = first_cand_cap(pr->trk[DAB_TRACK_AUDIO]);
-  if (pr->cap_entries < want_e) pr->cap_entries = want_e;
-  if (pr->cap_cand < want_c) pr->cap_cand = want_c;
+static int64_t first_cand_cap(int64_t a_Le) {
+  return 2 * (a_Le - 41) + 4096;                         // < 1 candidate per query on matching tracks
 }
 
-// The video side of the match stage as the gate, scoring and DP 1 read it: the video track's prep buffers, its
-// tables and the records of its hashed frames.  Either the pair's own (enqueue_match) or a shared index's.
-struct VideoSide {
-  const Track *V;
-  const int32_t *start, *items;
-  const uint4 *rec;
-};
-
-static int64_t video_sel_ub(const Track &V) { return (V.Le - 41 + 3) / 4 + 1; }
-
-// tables over the hashed video frames (dc[DC_N_VSEL] of them) into start / items, and the frames' records into rec;
-// the pair's table scratch holds the super-bucket counts and the entries between the passes
-static int enqueue_tables(dab_pair *pr, const Track &V, int32_t *dc, int64_t cap_e, DevBuf &tbl_start, DevBuf &tbl_items,
-                          DevBuf &rec) {
+// tables over the hashed video frames (dc[DC_N_VSEL] of them) of the side's prep, and the frames' records; the
+// pair's table scratch holds the super-bucket counts and the entries between the passes
+static int enqueue_tables(dab_pair *pr, VideoSide &vs, int32_t *dc) {
   dab_ctx *ctx = pr->ctx;
   cudaStream_t st = pr->stream;
-  const int64_t vsel_ub = video_sel_ub(V);
+  const Prep &V = vs.prep;
+  const int64_t vsel_ub = video_sel_ub(V.Le);
   const int64_t v_nstride = (V.Le > V.L ? V.Le : V.L) - 40;
-  DAB_TRY(dab_ensure(ctx, tbl_start, sizeof(int32_t) * (size_t)(TB_NSLOTS + 2)));
-  DAB_TRY(dab_ensure(ctx, tbl_items, sizeof(int32_t) * (size_t)(cap_e + 1)));
-  DAB_TRY(dab_ensure(ctx, rec, sizeof(uint4) * 2 * (size_t)(vsel_ub + 1)));
+  vs.cap_entries = std::max<int64_t>(vs.cap_entries, first_entries_cap(V.Le));
+  const int64_t cap_e = vs.cap_entries;
+  DAB_TRY(dab_ensure(ctx, vs.tbl_start, sizeof(int32_t) * (size_t)(TB_NSLOTS + 2)));
+  DAB_TRY(dab_ensure(ctx, vs.tbl_items, sizeof(int32_t) * (size_t)(cap_e + 1)));
+  DAB_TRY(dab_ensure(ctx, vs.v_rec, sizeof(uint4) * 2 * (size_t)(vsel_ub + 1)));
   DAB_TRY(dab_ensure(ctx, pr->tbl_sb, sizeof(int32_t) * (size_t)(3 * TB_NSB + 1)));
   DAB_TRY(dab_ensure(ctx, pr->tbl_ent, sizeof(uint2) * (size_t)(cap_e + 1)));
   int32_t *sb_count = pr->tbl_sb.as<int32_t>(), *sb_off = sb_count + TB_NSB, *sb_cursor = sb_off + (TB_NSB + 1);
+  uint4 *rec = vs.v_rec.as<uint4>();
   DAB_CUDA(cudaMemsetAsync(sb_count, 0, sizeof(int32_t) * TB_NSB, st));
   const unsigned nb = (unsigned)cdiv(vsel_ub, TB_THREADS);
-  table_count_kernel<<<nb, TB_THREADS, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, rec.as<uint4>(),
-                                                sb_count);
+  table_count_kernel<<<nb, TB_THREADS, 0, st>>>(V.pack.as<uint32_t>(), v_nstride, V.nq_list.as<int32_t>(), dc, rec, sb_count);
   table_scan_kernel<<<1, TB_SCAN_THREADS, 0, st>>>(dc, cap_e, sb_count, sb_off, sb_cursor);
-  table_scatter_kernel<<<nb, TB_THREADS, 0, st>>>(rec.as<uint4>(), dc, sb_cursor, pr->tbl_ent.as<uint2>());
-  table_sort_kernel<<<TB_NSB, TS_THREADS, 0, st>>>(dc, sb_off, pr->tbl_ent.as<uint2>(), tbl_start.as<int32_t>(),
-                                                   tbl_items.as<int32_t>());
+  table_scatter_kernel<<<nb, TB_THREADS, 0, st>>>(rec, dc, sb_cursor, pr->tbl_ent.as<uint2>());
+  table_sort_kernel<<<TB_NSB, TS_THREADS, 0, st>>>(dc, sb_off, pr->tbl_ent.as<uint2>(), vs.tbl_start.as<int32_t>(),
+                                                   vs.tbl_items.as<int32_t>());
   ctx->launches += 4;
   DAB_CUDA(cudaGetLastError());
   return DAB_OK;
 }
 
+// The counts of a video side built in this run.  False after an entries overflow: the tables are empty and their
+// capacity has grown to at least the total the run needed.
+static bool collect_tables(VideoSide &vs, const int32_t *hc) {
+  vs.n_vsel = hc[DC_N_VSEL];
+  vs.n_entries = hc[DC_N_ENTRIES];
+  if (!(hc[DC_OVERFLOW] & DAB_OVF_ENTRIES)) return true;
+  vs.cap_entries = std::max<int64_t>(2 * vs.cap_entries, hc[DC_NEED_ENTRIES]);
+  return false;
+}
+
 // gate + scoring + compaction of the pair's audio queries against `vs`: the points go to pr->pt_*
 static int enqueue_gate_score(dab_pair *pr, const VideoSide &vs, int32_t *dc) {
   dab_ctx *ctx = pr->ctx;
-  const Track &V = *vs.V, &A = pr->trk[DAB_TRACK_AUDIO];
+  const Prep &V = vs.prep, &A = pr->prep_a;
   cudaStream_t st = pr->stream;
   const int64_t a_nq = A.Le - 41;
   const int64_t q_ub = a_nq > 0 ? a_nq : 1;
@@ -1241,8 +1250,8 @@ static int enqueue_gate_score(dab_pair *pr, const VideoSide &vs, int32_t *dc) {
   GateArgs ga;
   ga.a_code = A.code.as<int32_t>(); ga.a_pack = A.pack.as<uint32_t>(); ga.a_nstride = a_nstride;
   ga.a_list = A.nq_list.as<int32_t>(); ga.dc = dc; ga.q_cap = q_ub;
-  ga.v_rec = vs.rec;
-  ga.start = vs.start; ga.items = vs.items;
+  ga.v_rec = vs.v_rec.as<uint4>();
+  ga.start = vs.tbl_start.as<int32_t>(); ga.items = vs.tbl_items.as<int32_t>();
   ga.row_count = pr->row_count.as<int32_t>(); ga.row_off = pr->row_off.as<int32_t>();
   ga.cand_tmp = pr->cand_tmp.as<int32_t>(); ga.cand_s = pr->cand_s.as<int32_t>(); ga.cand_i = pr->cand_i.as<int32_t>();
   ga.cand_cap = cap_c;
@@ -1296,45 +1305,13 @@ static int enqueue_gate_score(dab_pair *pr, const VideoSide &vs, int32_t *dc) {
   return DAB_OK;
 }
 
-// ---- match stage, enqueued without a host round trip: prep, codes, lists, tables, gate, scoring ----
-static int enqueue_match(dab_pair *pr, int64_t row_lo, int64_t row_hi) {
-  dab_ctx *ctx = pr->ctx;
-  DAB_TRY(ensure_hann(ctx));
-  Track &V = pr->trk[DAB_TRACK_VIDEO], &A = pr->trk[DAB_TRACK_AUDIO];
-  cudaStream_t st = pr->stream;
-  pr->n_points1 = pr->n_path1 = 0;
-  pr->points_from_index = false;
-  default_caps(pr);
-  const int64_t v_nq = V.Le - 41, a_nq = A.Le - 41;
-
-  DAB_TRY(dab_ensure(ctx, pr->counters, sizeof(int32_t) * DC_WORDS));
-  int32_t *dc = pr->counters.as<int32_t>();
-  DAB_CUDA(cudaEventRecord(pr->ev[4], st));
-  DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, st));
-  DAB_TRY(prep_track(pr, V, V, true));
-  DAB_TRY(prep_track(pr, A, A, false));
-  counts_lists_kernel<<<1, 32, 0, st>>>(dc, V.nq_flag.as<int32_t>() + (v_nq + 1), v_nq, A.nq_flag.as<int32_t>() + (a_nq + 1), a_nq,
-                                        row_lo, row_hi);
-  ctx->launches += 1;
-  DAB_CUDA(cudaEventRecord(pr->ev[5], st));
-  pr->stats.n_video_frames = V.L; pr->stats.n_audio_frames = A.L;
-
-  DAB_CUDA(cudaEventRecord(pr->ev[6], st));
-  DAB_TRY(enqueue_tables(pr, V, dc, pr->cap_entries, pr->tbl_start, pr->tbl_items, pr->v_rec));
-  DAB_CUDA(cudaEventRecord(pr->ev[7], st));
-  DAB_TRY(enqueue_gate_score(pr, VideoSide{&V, pr->tbl_start.as<int32_t>(), pr->tbl_items.as<int32_t>(), pr->v_rec.as<uint4>()}, dc));
-  for (int s = 2; s <= 5; ++s) pr->ev_used[s] = true;
-  DAB_CUDA(cudaGetLastError());
-  return DAB_OK;
-}
-
-// ---- DP #1 + traceback over pr->pt_* (dc[DC_N_PTS1] points sorted by (audio frame, video rank)) ----
-static int enqueue_dp1(dab_pair *pr, const Track &V) {
+// ---- DP #1 + traceback over pr->pt_* (dc[DC_N_PTS1] points sorted by (audio frame, rank in vs's hashed frames)) ----
+static int enqueue_dp1(dab_pair *pr, const VideoSide &vs) {
   dab_ctx *ctx = pr->ctx;
   cudaStream_t st = pr->stream;
   int32_t *dc = pr->counters.as<int32_t>();
   const int64_t cap_p = pr->cap_points1 > 0 ? pr->cap_points1 : 1;
-  const int64_t vsel_ub = video_sel_ub(V);
+  const int64_t vsel_ub = video_sel_ub(vs.prep.Le);
   DAB_CUDA(cudaEventRecord(pr->ev[12], st));
   if (vsel_ub > (1LL << (5 * DP_LEVELS))) { dab_set_err(ctx, "too many hashed video frames for the DP tree"); return DAB_E_CAPACITY; }
   int64_t lv[DP_LEVELS], tot = 0;
@@ -1355,7 +1332,7 @@ static int enqueue_dp1(dab_pair *pr, const Track &V) {
   dp1_kernel<<<1, 32, 0, st>>>(da);
   ctx->launches += 2;
   Path1Out out;
-  out.pt_i = pr->pt_i.as<int32_t>(); out.pt_s = da.pt_s; out.v_sel = V.nq_list.as<int32_t>();
+  out.pt_i = pr->pt_i.as<int32_t>(); out.pt_s = da.pt_s; out.v_sel = vs.prep.nq_list.as<int32_t>();
   out.x = pr->path1_x.as<int32_t>(); out.y = pr->path1_y.as<int32_t>();
   DAB_TRY(dab_enqueue_traceback(pr, da.back, da.n_points, da.result, cap_p, dc + DC_N_PATH1, out));
   DAB_CUDA(cudaEventRecord(pr->ev[13], st));
@@ -1364,11 +1341,40 @@ static int enqueue_dp1(dab_pair *pr, const Track &V) {
   return DAB_OK;
 }
 
-int dab_enqueue_stage_a_dp(dab_pair *pr) { return enqueue_dp1(pr, pr->trk[DAB_TRACK_VIDEO]); }
+int dab_enqueue_stage_a_dp(dab_pair *pr) { return enqueue_dp1(pr, pr->video); }
 
-int dab_enqueue_stage_a(dab_pair *pr, int64_t row_lo, int64_t row_hi, bool with_dp) {
-  DAB_TRY(enqueue_match(pr, row_lo, row_hi));
-  if (with_dp) DAB_TRY(dab_enqueue_stage_a_dp(pr));
+// ---- stage A, enqueued without a host round trip: prep, codes, lists, tables (own video side only), gate,
+// scoring, then DP 1 + traceback if with_dp, then the counts ----
+int dab_enqueue_stage_a(dab_pair *pr, const dab_index *ix, int64_t row_lo, int64_t row_hi, bool with_dp) {
+  dab_ctx *ctx = pr->ctx;
+  DAB_TRY(ensure_hann(ctx));
+  const Track &A = pr->trk[DAB_TRACK_AUDIO];
+  const VideoSide &vs = ix ? ix->side : pr->video;
+  cudaStream_t st = pr->stream;
+  pr->n_points1 = pr->n_path1 = 0;
+  pr->points_side = nullptr;
+  pr->cap_cand = std::max<int64_t>(pr->cap_cand, first_cand_cap(A.Le));
+
+  DAB_TRY(dab_ensure(ctx, pr->counters, sizeof(int32_t) * DC_WORDS));
+  int32_t *dc = pr->counters.as<int32_t>();
+  if (ix) DAB_CUDA(cudaStreamWaitEvent(st, ix->ready, 0));
+  DAB_CUDA(cudaEventRecord(pr->ev[4], st));
+  DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, st));
+  if (!ix) DAB_TRY(prep_track(pr, pr->trk[DAB_TRACK_VIDEO], pr->video.prep, true));
+  DAB_TRY(prep_track(pr, A, pr->prep_a, false));
+  enqueue_counts_lists(pr, dc, vs.prep, pr->prep_a, row_lo, row_hi);
+  DAB_CUDA(cudaEventRecord(pr->ev[5], st));
+  pr->stats.n_video_frames = vs.prep.L; pr->stats.n_audio_frames = A.L;
+  if (!ix) {
+    DAB_CUDA(cudaEventRecord(pr->ev[6], st));
+    DAB_TRY(enqueue_tables(pr, pr->video, dc));
+    DAB_CUDA(cudaEventRecord(pr->ev[7], st));
+  }
+  DAB_TRY(enqueue_gate_score(pr, vs, dc));
+  pr->ev_used[2] = pr->ev_used[4] = pr->ev_used[5] = true;
+  pr->ev_used[3] = !ix;             // timing slot of the table build
+  if (with_dp) DAB_TRY(enqueue_dp1(pr, vs));
+  DAB_CUDA(cudaGetLastError());
   return dab_enqueue_counts(pr);
 }
 
@@ -1395,22 +1401,22 @@ void dab_collect_stage_a_dp(dab_pair *pr) {
   pr->stats.n_path1 = pr->n_path1;
 }
 
-// the counts of a match stage (+ DP 1), whichever video side it ran against
-static int collect_match(dab_pair *pr, bool with_dp) {
+// the counts of a stage-A run against the same video side as dab_enqueue_stage_a
+int dab_collect_stage_a(dab_pair *pr, const dab_index *ix, bool with_dp) {
   dab_ctx *ctx = pr->ctx;
   const int32_t *hc = reinterpret_cast<const int32_t *>(pr->h_counters);
-  pr->trk[DAB_TRACK_AUDIO].n_list = hc[DC_N_AQ_ALL];
+  const bool tables_ok = ix || collect_tables(pr->video, hc);   // the pair's own side was built in this run
+  const VideoSide &vs = ix ? ix->side : pr->video;
+  pr->points_side = &vs;
   pr->stats.n_video_selected = hc[DC_N_VSEL];
   pr->stats.n_audio_queries = hc[DC_N_Q];
-  pr->stats.n_table_entries = hc[DC_N_ENTRIES];
+  pr->stats.n_table_entries = vs.n_entries;
   pr->stats.n_enumerated = (int64_t)(((uint64_t)(uint32_t)hc[DC_ENUM_HI] << 32) | (uint32_t)hc[DC_ENUM_LO]);
   pr->stats.n_candidates = hc[DC_N_CAND];
-  const int ovf = hc[DC_OVERFLOW];
-  if (ovf & (DAB_OVF_ENTRIES | DAB_OVF_CAND)) {
+  if (!tables_ok || (hc[DC_OVERFLOW] & DAB_OVF_CAND)) {
     // doubled, and at least the total this run needed: repeated audio (a shared tone, a looped bed) can need
     // hundreds of times the first guess, more than doubling reaches within DAB_STAGE_A_ATTEMPTS runs
-    if (ovf & DAB_OVF_ENTRIES) pr->cap_entries = std::max<int64_t>(2 * pr->cap_entries, hc[DC_NEED_ENTRIES]);
-    if (ovf & DAB_OVF_CAND) pr->cap_cand = std::max<int64_t>(2 * pr->cap_cand, hc[DC_NEED_CAND]);
+    if (hc[DC_OVERFLOW] & DAB_OVF_CAND) pr->cap_cand = std::max<int64_t>(2 * pr->cap_cand, hc[DC_NEED_CAND]);
     dab_set_err(ctx, "stage A: a device buffer overflowed, capacity doubled");
     return DAB_E_CAPACITY;
   }
@@ -1420,85 +1426,27 @@ static int collect_match(dab_pair *pr, bool with_dp) {
   return DAB_OK;
 }
 
-int dab_collect_stage_a(dab_pair *pr, bool with_dp) {
-  pr->trk[DAB_TRACK_VIDEO].n_list = reinterpret_cast<const int32_t *>(pr->h_counters)[DC_N_VSEL];
-  DAB_TRY(collect_match(pr, with_dp));
-  pr->matched = true;
+// ---- shared video index: the video side of the match stage, built once, read by any number of pairs --------
+int dab_enqueue_index(dab_pair *src, dab_index *ix) {
+  dab_ctx *ctx = src->ctx;
+  DAB_TRY(ensure_hann(ctx));
+  VideoSide &vs = ix->side;
+  DAB_TRY(dab_ensure(ctx, ix->counters, sizeof(int32_t) * DC_WORDS));
+  int32_t *dc = ix->counters.as<int32_t>();
+  DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, src->stream));
+  DAB_TRY(prep_track(src, src->trk[DAB_TRACK_VIDEO], vs.prep, true));
+  // DC_N_VNQ and DC_N_VSEL; the audio words it also writes are never read from the index's block
+  enqueue_counts_lists(src, dc, vs.prep, vs.prep, 0, 0);
+  DAB_TRY(enqueue_tables(src, vs, dc));
+  DAB_CUDA(dab_readback(src, src->h_counters, dc, sizeof(int32_t) * DC_WORDS));
   return DAB_OK;
 }
 
-// ---- shared video index: the video side of the match stage, built once, read by any number of pairs --------
-int dab_build_index(dab_pair *src, dab_index *ix) {
+int dab_collect_index(dab_pair *src, dab_index *ix) {
   dab_ctx *ctx = src->ctx;
-  DAB_TRY(ensure_hann(ctx));
-  const Track &S = src->trk[DAB_TRACK_VIDEO];
-  Track &V = ix->V;
-  V.S = S.S; V.ch = S.ch; V.L = S.L; V.Le = S.Le; V.have_features = true;
-  cudaStream_t st = src->stream;
-  const int64_t v_nq = V.Le - 41;
-  int64_t cap_e = first_entries_cap(V);
-  DAB_TRY(dab_ensure(ctx, ix->counters, sizeof(int32_t) * DC_WORDS));
-  int32_t *dc = ix->counters.as<int32_t>();
-  const int32_t *hc = reinterpret_cast<const int32_t *>(src->h_counters);
-  for (int attempt = 0; attempt < DAB_STAGE_A_ATTEMPTS; ++attempt) {
-    DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, st));
-    DAB_TRY(prep_track(src, S, V, true));
-    // DC_N_VNQ and DC_N_VSEL; the audio words it also writes are never read from the index's block
-    const int32_t *v_off = V.nq_flag.as<int32_t>() + (v_nq + 1);
-    counts_lists_kernel<<<1, 32, 0, st>>>(dc, v_off, v_nq, v_off, v_nq, 0, 0);
-    ctx->launches += 1;
-    DAB_TRY(enqueue_tables(src, V, dc, cap_e, ix->tbl_start, ix->tbl_items, ix->v_rec));
-    DAB_CUDA(dab_readback(src, src->h_counters, dc, sizeof(int32_t) * DC_WORDS));
-    DAB_CUDA(dab_wait_stream(st));
-    if (!(hc[DC_OVERFLOW] & DAB_OVF_ENTRIES)) {
-      V.n_list = ix->n_vsel = hc[DC_N_VSEL];
-      ix->n_entries = hc[DC_N_ENTRIES];
-      ix->cap_entries = cap_e;
-      DAB_CUDA(cudaEventRecord(ix->ready, st));
-      DAB_CUDA(cudaGetLastError());
-      return DAB_OK;
-    }
-    cap_e = std::max<int64_t>(2 * cap_e, hc[DC_NEED_ENTRIES]);
-  }
-  dab_set_err(ctx, "dab_index_build: the hash tables overflowed on every attempt");
-  return DAB_E_CAPACITY;
-}
-
-// Match stage + DP 1 of the pair's description track against a built index: audio prep, gate, scoring, DP 1,
-// traceback and the counts, enqueued without a host round trip.  The index is only read.
-int dab_enqueue_stage_a_against(dab_pair *pr, const dab_index *ix) {
-  dab_ctx *ctx = pr->ctx;
-  DAB_TRY(ensure_hann(ctx));
-  const Track &V = ix->V;
-  Track &A = pr->trk[DAB_TRACK_AUDIO];
-  cudaStream_t st = pr->stream;
-  pr->n_points1 = pr->n_path1 = 0;
-  pr->matched = false;              // the pair's own tables and hashed-frame list are not those of these points
-  pr->points_from_index = true;
-  pr->cap_cand = std::max<int64_t>(pr->cap_cand, first_cand_cap(A));
-  const int64_t v_nq = V.Le - 41, a_nq = A.Le - 41;
-
-  DAB_TRY(dab_ensure(ctx, pr->counters, sizeof(int32_t) * DC_WORDS));
-  int32_t *dc = pr->counters.as<int32_t>();
-  DAB_CUDA(cudaStreamWaitEvent(st, ix->ready, 0));
-  DAB_CUDA(cudaEventRecord(pr->ev[4], st));
-  DAB_CUDA(cudaMemsetAsync(dc, 0, sizeof(int32_t) * DC_WORDS, st));
-  DAB_TRY(prep_track(pr, A, A, false));
-  counts_lists_kernel<<<1, 32, 0, st>>>(dc, V.nq_flag.as<int32_t>() + (v_nq + 1), v_nq, A.nq_flag.as<int32_t>() + (a_nq + 1), a_nq,
-                                        0, INT64_MAX);
-  ctx->launches += 1;
-  DAB_CUDA(cudaEventRecord(pr->ev[5], st));
-  pr->stats.n_video_frames = V.L; pr->stats.n_audio_frames = A.L;
-  DAB_TRY(enqueue_gate_score(pr, VideoSide{&V, ix->tbl_start.as<int32_t>(), ix->tbl_items.as<int32_t>(), ix->v_rec.as<uint4>()}, dc));
-  pr->ev_used[2] = pr->ev_used[4] = pr->ev_used[5] = true;
-  pr->ev_used[3] = false;           // no tables are built
-  DAB_TRY(enqueue_dp1(pr, V));
-  return dab_enqueue_counts(pr);
-}
-
-int dab_collect_stage_a_against(dab_pair *pr, const dab_index *ix) {
-  DAB_TRY(collect_match(pr, true));
-  pr->stats.n_table_entries = ix->n_entries;
+  if (!collect_tables(ix->side, reinterpret_cast<const int32_t *>(src->h_counters))) return DAB_E_CAPACITY;
+  DAB_CUDA(cudaEventRecord(ix->ready, src->stream));
+  DAB_CUDA(cudaGetLastError());
   return DAB_OK;
 }
 
@@ -1533,7 +1481,7 @@ static __global__ void set_word_kernel(int32_t *dc, int word, int32_t value) {
 int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *v_video, const double *qual,
                            int64_t n, int src_on_device) {
   dab_ctx *ctx = pr->ctx;
-  Track &V = pr->trk[DAB_TRACK_VIDEO];
+  const VideoSide &V = pr->video;
   cudaStream_t st = pr->stream;
   const cudaMemcpyKind kind = src_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
   DAB_TRY(dab_ensure(ctx, pr->pt_i, sizeof(int32_t) * (size_t)(n + 1)));
@@ -1547,7 +1495,7 @@ int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *
     DAB_CUDA(cudaMemcpyAsync(pr->pt_q.p, qual, sizeof(double) * (size_t)n, kind, st));
     DAB_CUDA(cudaMemsetAsync(pr->dpres.as<int32_t>() + 8, 0, sizeof(int32_t), st));
     frames_to_ranks_kernel<<<(unsigned)cdiv(n, 256), 256, 0, st>>>(pr->pt_i.as<int32_t>(), pr->cand_tmp.as<int32_t>(), pr->pt_q.as<double>(), n,
-                                                                    V.nq_list.as<int32_t>(), (int32_t)V.n_list, pr->pt_s.as<int32_t>(),
+                                                                    V.prep.nq_list.as<int32_t>(), (int32_t)V.n_vsel, pr->pt_s.as<int32_t>(),
                                                                     pr->dpres.as<int32_t>() + 8);
     ctx->launches += 1;
     DAB_CUDA(dab_readback(pr, &pr->h_counters[22], pr->dpres.as<int32_t>() + 8, sizeof(int32_t)));
@@ -1566,7 +1514,6 @@ int dab_run_import_points1(dab_pair *pr, const int32_t *i_audio, const int32_t *
   pr->n_points1 = n;
   pr->stats.n_points1 = n;
   pr->n_path1 = 0;
-  pr->points_from_index = false;
   if (pr->cap_points1 < n) pr->cap_points1 = n;   // DP 1 sizes its buffers from it
   return DAB_OK;
 }

@@ -206,6 +206,71 @@ def test_free_is_refused_while_a_pair_runs_against_the_index(ctx, tracks):
         pair.close()
 
 
+def test_one_pair_switches_between_an_index_and_its_own_video_side(ctx, tracks):
+    """One pair with the features of a video and a description runs stage_a_against an index of that video,
+    stage_a, stage_a_against again, then stage_a_match over two row shards + import_points1 + dp1.  Every step
+    gives a fresh pair's stage_a() counts and path.  After stage_a_against the points are ranks into the index, so
+    points1, import_points1 and dp1 are refused (DAB_E_STATE); after the pair's own stage A they work again."""
+    from describealign_b200 import _cabi, batch
+    videos, descriptions = tracks
+    fresh = _cabi.Pair(ctx)
+    try:
+        fresh.set_pcm(_cabi.VIDEO, videos[0])
+        fresh.set_pcm(_cabi.AUDIO, descriptions[0])
+        want = fresh.stage_a() + (fresh.stats()["n_candidates"],)
+        want_points, want_path = fresh.points1(), fresh.path1()
+        features = [fresh.get_features(t) for t in (_cabi.VIDEO, _cabi.AUDIO)]
+    finally:
+        fresh.close()
+    assert want[1] > 0
+
+    pair = _cabi.Pair(ctx)
+    try:
+        for t in (_cabi.VIDEO, _cabi.AUDIO):
+            pair.set_features(t, features[t])
+        ix = _cabi.Index(pair)
+
+        def check_path():
+            x, y = pair.path1()
+            assert np.array_equal(x, want_path[0]) and np.array_equal(y, want_path[1])
+
+        def check_refused():
+            for call in (pair.points1, lambda: pair.import_points1(*want_points), pair.dp1):
+                with pytest.raises(_cabi.DabError, match="error 3:"):
+                    call()
+
+        def check_own_points():
+            got = pair.points1()
+            for g, w in zip(got, want_points):
+                assert np.array_equal(g, w)
+            pair.import_points1(*want_points)
+            assert pair.dp1() == want[1]
+            check_path()
+
+        for step in ("against", "own", "against"):
+            got = pair.stage_a_against(ix) if step == "against" else pair.stage_a()
+            assert got + (pair.stats()["n_candidates"],) == want, (step, got)
+            check_path()
+            if step == "against":
+                check_refused()
+            else:
+                check_own_points()
+
+        parts, n_cand = [], 0
+        for lo, hi in batch.row_shards(pair.feature_lens(_cabi.AUDIO)[0], 2):
+            pair.stage_a_match(lo, hi)
+            parts.append(pair.points1())
+            n_cand += pair.stats()["n_candidates"]
+        points = [np.concatenate([p[k] for p in parts]) for k in range(3)]
+        assert (len(points[0]), n_cand) == (want[0], want[2])
+        pair.import_points1(*points)
+        assert pair.dp1() == want[1]
+        check_path()
+        ix.free()
+    finally:
+        pair.close()
+
+
 def test_assign_recovers_pairs_and_flags_the_name_order(tracks):
     from describealign_b200 import pairing
     videos, descriptions = tracks
