@@ -102,7 +102,8 @@ struct dab_pair {
   DevBuf row_count, row_off;   // i32 [n_queries + 1]
   DevBuf row_stash;            // i32 [n_queries][4]: first candidates of each row (gate count pass)
   DevBuf gate_big;             // i32: rows with more than 4 candidates (work list of the fill pass)
-  DevBuf gate_rec, gate_best;  // per query: digit words + its two buckets (32 B); bucket entries to visit and their scan
+  DevBuf gate_rec;             // per query: digit words + its two buckets (32 B)
+  DevBuf gate_best;            // per query: i64 exclusive scan of the bucket entries to visit, then those i32 counts
   DevBuf cand_tmp, cand_s, cand_i;  // i32 [n_cand]
   DevBuf cand_q;               // f64 [n_cand]
   DevBuf keep_flag, keep_off;  // i32 [n_cand + 1]
@@ -200,10 +201,13 @@ cudaError_t dab_wait_stream(cudaStream_t st);
 cudaError_t dab_readback(dab_pair *pr, void *host_dst, const void *dev_src, size_t bytes);
 static inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
-// exclusive scan of n int32 values; out[n] receives the total (out has n + 1 entries).  n_dev (optional):
-// device-side count of valid elements (<= n; launches are sized for n); total_out (optional): device
-// word that also receives the total.
+// exclusive scan of n non-negative int32 values; out[n] receives the total (out has n + 1 entries).  n_dev
+// (optional): device-side count of valid elements (<= n; launches are sized for n); total_out (optional): device
+// word that also receives the total.  int32 sums saturate at INT32_MAX; the int64 scan writes its total to
+// total_out[0] (low word) and total_out[1] (high word).
 int dab_exclusive_scan(dab_pair *pr, const int32_t *in, int32_t *out, int64_t n, const int32_t *n_dev = nullptr,
+                       int32_t *total_out = nullptr);
+int dab_exclusive_scan(dab_pair *pr, const int32_t *in, int64_t *out, int64_t n, const int32_t *n_dev = nullptr,
                        int32_t *total_out = nullptr);
 
 // Counts that only the device knows while a stage is in flight (int32 words of dab_pair::counters).  Every
@@ -214,7 +218,7 @@ enum {
   DC_N_AQ_ALL = 1,     // not-quiet audio frames
   DC_N_ENTRIES = 2,    // expanded table entries
   DC_N_VSEL = 3,       // hashed video frames (every 4th not-quiet)
-  DC_ENUM_LO = 4, DC_ENUM_HI = 5,   // u64: bucket entries visited by the gate
+  DC_ENUM_LO = 4, DC_ENUM_HI = 5,   // u64: bucket entries visited by the gate (low, high word; written by its scan)
   DC_N_CAND = 6,
   DC_N_PTS1 = 7,
   DC_DP1_END = 8,      // end id (-1: no path), written by dp1_kernel
@@ -227,7 +231,8 @@ enum {
   DC_OVERFLOW_B = 17,  // stage B: bit 2 more than 32 corridors on one audio row
   DC_DP2_END = 18,     // end id, then the frontier value (double at words 20-21)
   DC_N_PATH2 = 19,     // path length, written by the traceback
-  DC_NEED_ENTRIES = 22, DC_NEED_CAND = 23,    // unclamped table-entry and candidate totals (sizes the next run)
+  DC_NEED_ENTRIES = 22, DC_NEED_CAND = 23,    // unclamped table-entry and candidate totals (sizes the next run;
+                                              // the candidate total saturates at INT32_MAX)
   DC_DP2_CNT = 24,     // 4 x u64 DP-2 work counters
   DC_WORDS = 32
 };
@@ -242,7 +247,10 @@ int dab_enqueue_counts(dab_pair *pr);
 // Stage A.  On a capacity overflow dab_collect_stage_a grows the buffer to at least the total the run needed and
 // returns DAB_E_CAPACITY: the caller enqueues the stage again, up to DAB_STAGE_A_ATTEMPTS runs in all.  An
 // entries overflow leaves the tables empty, so the candidate total is only known one run later: three runs at most.
+// A run that needs more candidates than the int32-indexed candidate arrays hold (DAB_MAX_CANDIDATES) is not run
+// again: the collect returns DAB_E_CAPACITY with the count, and the next enqueue refuses at once.
 constexpr int DAB_STAGE_A_ATTEMPTS = 8;
+constexpr int64_t DAB_MAX_CANDIDATES = 0x7ffffffeLL;   // INT32_MAX - 1: a candidate total of INT32_MAX is saturated
 int dab_check_stage_a_inputs(dab_pair *pr, const char *who);
 // match points of audio rows [row_lo, row_hi) against a shared index (ix), or against the pair's own video side,
 // built in the same run; then DP 1 + traceback if with_dp, then the counts

@@ -163,29 +163,38 @@ constexpr int SCAN_THREADS = 512;
 constexpr int SCAN_ITEMS = 8;
 constexpr int SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
 
-__device__ __forceinline__ int block_exclusive_scan(int v, int *total, int *smem /* >= 32 ints */) {
+template <typename T> struct PlainAdd {
+  __device__ static T add(T a, T b) { return a + b; }
+};
+
+// exclusive scan over the block; Op::add is the (associative) sum
+template <typename T, typename Op = PlainAdd<T>>
+__device__ __forceinline__ T block_exclusive_scan(T v, T *total, T *smem /* >= 33 */) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int inc = v;
+  T inc = v;
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) {
-    int y = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += y;
+    const T y = __shfl_up_sync(0xffffffffu, inc, o);
+    if (lane >= o) inc = Op::add(inc, y);
   }
   if (lane == 31) smem[warp] = inc;
   __syncthreads();
   if (warp == 0) {
-    int w = (lane < (int)(blockDim.x >> 5)) ? smem[lane] : 0;
-    int winc = w;
+    T winc = (lane < (int)(blockDim.x >> 5)) ? smem[lane] : T(0);
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-      int y = __shfl_up_sync(0xffffffffu, winc, o);
-      if (lane >= o) winc += y;
+      const T y = __shfl_up_sync(0xffffffffu, winc, o);
+      if (lane >= o) winc = Op::add(winc, y);
     }
-    smem[lane] = winc - w;
+    const T wex = __shfl_up_sync(0xffffffffu, winc, 1);
+    smem[lane] = lane ? wex : T(0);
     if (lane == 31) smem[32] = winc;
   }
   __syncthreads();
-  int res = inc - v + smem[warp];
+  // exclusive within the warp (a shuffle, not inc - v: a saturated sum cannot be undone), then the warps before it
+  T wex = __shfl_up_sync(0xffffffffu, inc, 1);
+  if (lane == 0) wex = 0;
+  const T res = Op::add(wex, smem[warp]);
   *total = smem[32];
   __syncthreads();
   return res;
@@ -205,21 +214,71 @@ __device__ __forceinline__ int64_t scan_len(int64_t n, const int32_t *n_dev) {
 // prefix.  Status words carry the epoch of the scan call, so the array needs no clearing between calls;
 // the last tile to finish resets the ticket counter.
 //   status[t] = epoch << 34 | kind << 32 | value      kind 1 = aggregate, 2 = inclusive prefix
-struct ScanArgs {
-  const int32_t *in;
-  int32_t *out;
-  int64_t n;
-  const int32_t *n_dev;
-  unsigned long long *status;      // [tiles]
-  unsigned int *ticket;            // [0] next tile, [1] tiles finished
-  unsigned int epoch;              // 1 .. 2^30 - 1, different from the previous call's on this array
-  int32_t *total_out;
+// The input is int32; the sums are T.  T = int32_t (list offsets, row counts, keep flags) adds with saturation at
+// INT32_MAX, which is associative over non-negative values: a total that does not fit reads INT32_MAX instead of
+// wrapping.  T = int64_t (the gate's entry prefix) spends two status words per tile, the low and the high half of the
+// value, each under the same epoch and kind.  A reader takes a pair only when both words carry this call's epoch and
+// the same kind: a tile publishes each kind once per call, so the two halves are of one publication, and a word left
+// by an earlier call (other epoch) or a half-updated pair (kinds differ) is read again.  The words are 64-bit
+// aligned stores, so each half is seen whole.
+template <typename T> struct ScanOps;
+template <> struct ScanOps<int32_t> {
+  static constexpr int WORDS = 1;
+  __device__ static int32_t add(int32_t a, int32_t b) { return (int32_t)min((uint32_t)a + (uint32_t)b, 0x7fffffffu); }
+};
+template <> struct ScanOps<int64_t> : PlainAdd<int64_t> {
+  static constexpr int WORDS = 2;
 };
 
-__global__ void __launch_bounds__(SCAN_THREADS) scan_onepass_kernel(ScanArgs a) {
-  __shared__ int sm[33];
+template <typename T>
+struct ScanArgs {
+  const int32_t *in;
+  T *out;
+  int64_t n;
+  const int32_t *n_dev;
+  unsigned long long *status;      // [tiles * ScanOps<T>::WORDS]
+  unsigned int *ticket;            // [0] next tile, [1] tiles finished
+  unsigned int epoch;              // 1 .. 2^30 - 1, different from the previous call's on this array
+  int32_t *total_out;              // the total's int32 words, low word first
+};
+
+template <typename T>
+__device__ __forceinline__ void scan_publish(volatile unsigned long long *st, unsigned int tile, unsigned long long tag,
+                                             unsigned long long kind, T value) {
+  const unsigned long long hdr = tag | (kind << 32);
+  if constexpr (ScanOps<T>::WORDS == 1) {
+    st[tile] = hdr | (uint32_t)value;
+  } else {
+    st[2 * (size_t)tile] = hdr | (uint32_t)(uint64_t)value;
+    st[2 * (size_t)tile + 1] = hdr | (uint32_t)((uint64_t)value >> 32);
+  }
+}
+
+// tile t's status in this call, waited for: its kind (1 aggregate, 2 inclusive prefix) and value
+template <typename T>
+__device__ __forceinline__ unsigned scan_wait(volatile unsigned long long *st, int t, unsigned int epoch, T &value) {
+  if constexpr (ScanOps<T>::WORDS == 1) {
+    unsigned long long w;
+    do { w = st[t]; } while ((w >> 34) != epoch);
+    value = (int32_t)(uint32_t)w;
+    return (unsigned)(w >> 32) & 3u;
+  } else {
+    unsigned long long lo, hi;
+    do {
+      lo = st[2 * (size_t)t];
+      hi = st[2 * (size_t)t + 1];
+    } while ((lo >> 34) != epoch || (hi >> 34) != epoch || ((lo ^ hi) >> 32) != 0ull);
+    value = (int64_t)(((hi & 0xffffffffull) << 32) | (lo & 0xffffffffull));
+    return (unsigned)(lo >> 32) & 3u;
+  }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(SCAN_THREADS) scan_onepass_kernel(ScanArgs<T> a) {
+  using Op = ScanOps<T>;
+  __shared__ T sm[33];
   __shared__ unsigned int s_tile;
-  __shared__ int s_prefix;
+  __shared__ T s_prefix;
   const int64_t n = scan_len(a.n, a.n_dev);
   if (threadIdx.x == 0) s_tile = atomicAdd(a.ticket, 1u);
   __syncthreads();
@@ -233,58 +292,62 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_onepass_kernel(ScanArgs a) 
     return;
   }
   const int64_t base = (int64_t)tile * SCAN_TILE + (int64_t)threadIdx.x * SCAN_ITEMS;
-  int v[SCAN_ITEMS];
-  int s = 0;
+  int32_t v[SCAN_ITEMS];
+  T s = 0;
 #pragma unroll
   for (int k = 0; k < SCAN_ITEMS; ++k) {
     v[k] = (base + k < n) ? a.in[base + k] : 0;
-    s += v[k];
+    s = Op::add(s, (T)v[k]);
   }
-  int total;
-  const int ex = block_exclusive_scan(s, &total, sm);
+  T total;
+  const T ex = block_exclusive_scan<T, Op>(s, &total, sm);
   if (threadIdx.x < 32) {
     // warp 0 publishes the tile's aggregate, then looks back 32 predecessors at a time
     const int lane = threadIdx.x;
     const unsigned long long tag = (unsigned long long)a.epoch << 34;
     volatile unsigned long long *st = a.status;
-    int prefix = 0;
+    T prefix = 0;
     if (tile > 0) {
-      if (lane == 0) { st[tile] = tag | (1ull << 32) | (unsigned int)total; __threadfence(); }
+      if (lane == 0) { scan_publish<T>(st, tile, tag, 1ull, total); __threadfence(); }
       int end = (int)tile;                      // tiles [.., end) are still to be accounted for
       while (end > 0) {
         const int t = end - 1 - lane;           // lane 0 = nearest predecessor
-        unsigned long long w = 0ull;
-        if (t >= 0) { do { w = st[t]; } while ((w >> 34) != a.epoch); }
-        const bool is_prefix = t >= 0 && ((w >> 32) & 3ull) == 2ull;
+        T w = 0;
+        const unsigned kind = t >= 0 ? scan_wait<T>(st, t, a.epoch, w) : 0u;
+        const bool is_prefix = kind == 2u;
         const unsigned pm = __ballot_sync(0xffffffffu, is_prefix);
         const int stop = pm ? __ffs(pm) - 1 : 32;             // nearest lane holding an inclusive prefix
-        int v = (t >= 0 && lane <= stop) ? (int)(unsigned int)w : 0;
+        T x = (t >= 0 && lane <= stop) ? w : T(0);
 #pragma unroll
-        for (int o = 16; o >= 1; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        prefix += v;
+        for (int o = 16; o >= 1; o >>= 1) x = Op::add(x, __shfl_xor_sync(0xffffffffu, x, o));
+        prefix = Op::add(prefix, x);
         if (pm) break;
         end -= 32;
       }
     }
     if (lane == 0) {
-      st[tile] = tag | (2ull << 32) | (unsigned int)(prefix + total);
+      scan_publish<T>(st, tile, tag, 2ull, Op::add(prefix, total));
       __threadfence();
       s_prefix = prefix;
     }
   }
   __syncthreads();
-  int run = ex + s_prefix;
+  T run = Op::add(ex, s_prefix);
 #pragma unroll
   for (int k = 0; k < SCAN_ITEMS; ++k) {
     if (base + k < n) a.out[base + k] = run;
-    run += v[k];
+    run = Op::add(run, (T)v[k]);
   }
   // the tile that holds position n (or the last tile) writes the total
   const int64_t last_tile = n / SCAN_TILE;
   if ((int64_t)tile == last_tile && threadIdx.x == 0) {
     // total of all elements = prefix of this tile + its own total (elements past n are zero)
-    a.out[n] = s_prefix + total;
-    if (a.total_out) *a.total_out = s_prefix + total;
+    const T all = Op::add(s_prefix, total);
+    a.out[n] = all;
+    if (a.total_out) {
+      a.total_out[0] = (int32_t)(uint32_t)(uint64_t)all;
+      if constexpr (ScanOps<T>::WORDS == 2) a.total_out[1] = (int32_t)(uint32_t)((uint64_t)all >> 32);
+    }
   }
   if (threadIdx.x == 0) {
     __threadfence();
@@ -647,7 +710,7 @@ __global__ void gate_fill_big_kernel(GateArgs g) {
 // cheapest buckets; their number ranges from none to several hundred, so a warp per query leaves most lanes
 // idle (ncu: 380 warp instructions per query for 33 entries on average).  Three steps:
 //   gate_plan_kernel      thread per query: digit words, the two buckets, their joint length `best`
-//   scan                  P = exclusive scan of best; its total is the number of entries to test
+//   scan                  P = exclusive scan of best in 64 bits; its total is the number of entries to test
 //   gate_entries_kernel   tiles of 2048 consecutive entries of the concatenated bucket lists; the tile finds
 //                         the queries it spans by a warp-wide 32-ary search in P, marks where each one starts,
 //                         spreads the owners by a max-scan, and every thread tests 8 consecutive entries.
@@ -698,7 +761,7 @@ __global__ void gate_plan_kernel(GateArgs g, GateQ *rec, int32_t *best_out) {
 constexpr int GE_THREADS = 256, GE_PER = 8, GE_TILE = GE_THREADS * GE_PER;
 
 // last index q in [0, n] with P[q] <= x (P non-decreasing, P[0] = 0 <= x), found by one warp: 32 probes per round
-__device__ __forceinline__ int warp_last_le(const int32_t *P, int n, int x, int lane) {
+__device__ __forceinline__ int warp_last_le(const int64_t *P, int n, int64_t x, int lane) {
   int lo = 0, hi = n + 1;                 // P[lo] <= x; hi == n + 1 or P[hi] > x
   while (hi - lo > 1) {
     const int step = (hi - lo + 31) / 32;
@@ -713,17 +776,18 @@ __device__ __forceinline__ int warp_last_le(const int32_t *P, int n, int x, int 
   return lo;
 }
 
-__global__ void __launch_bounds__(GE_THREADS) gate_entries_kernel(GateArgs g, const GateQ *rec, const int32_t *P) {
+// Entry positions are 64-bit (a long pair's queries visit more than 2^31 entries in all); the position of an entry
+// inside its query's two buckets is below that query's count, an int32.
+__global__ void __launch_bounds__(GE_THREADS) gate_entries_kernel(GateArgs g, const GateQ *rec, const int64_t *P) {
   __shared__ __align__(16) int owner[GE_TILE];
   __shared__ int s_q[2];
   __shared__ int s_wmax[GE_THREADS / 32];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int nq = g.dc[DC_N_Q];
-  const int total = g.dc[DC_ENUM_LO];
+  const int64_t total = (int64_t)(((uint64_t)(uint32_t)g.dc[DC_ENUM_HI] << 32) | (uint32_t)g.dc[DC_ENUM_LO]);
   if (g.dc[DC_OVERFLOW] & DAB_OVF_ENTRIES) return;
-  for (int64_t E0l = (int64_t)blockIdx.x * GE_TILE; E0l < total; E0l += (int64_t)gridDim.x * GE_TILE) {
-    const int E0 = (int)E0l;
-    const int E1 = E0 + GE_TILE < total ? E0 + GE_TILE : total;
+  for (int64_t E0 = (int64_t)blockIdx.x * GE_TILE; E0 < total; E0 += (int64_t)gridDim.x * GE_TILE) {
+    const int64_t E1 = E0 + GE_TILE < total ? E0 + GE_TILE : total;
     // the queries this tile spans: q0 owns entry E0, q1 owns entry E1 - 1 (both non-empty rows)
     if (warp < 2) {
       const int r = warp_last_le(P, nq, warp == 0 ? E0 : E1 - 1, lane);
@@ -736,8 +800,8 @@ __global__ void __launch_bounds__(GE_THREADS) gate_entries_kernel(GateArgs g, co
     // every later query that starts inside the tile marks its first entry (empty rows share a position with the
     // non-empty row that follows them: the largest index wins)
     for (int q = q0 + 1 + tid; q <= q1; q += GE_THREADS) {
-      const int pos = P[q] - E0;
-      if (pos > 0 && pos < GE_TILE) atomicMax(&owner[pos], q - q0);
+      const int64_t pos = P[q] - E0;
+      if (pos > 0 && pos < GE_TILE) atomicMax(&owner[(int)pos], q - q0);
     }
     __syncthreads();
     // inclusive max-scan: slot e belongs to the last marked query at or before it
@@ -768,12 +832,12 @@ __global__ void __launch_bounds__(GE_THREADS) gate_entries_kernel(GateArgs g, co
     __syncthreads();
 #pragma unroll
     for (int j = 0; j < GE_PER; ++j) {
-      const int e = E0 + j * GE_THREADS + tid;
+      const int64_t e = E0 + j * GE_THREADS + tid;
       if (e < E1) {
         const int q = q0 + owner[j * GE_THREADS + tid];
         const uint4 *rp = reinterpret_cast<const uint4 *>(rec + q);
         const uint4 x0 = __ldg(rp), x1 = __ldg(rp + 1);
-        const int el = e - P[q];
+        const int el = (int)(e - P[q]);
         const int ca = (int)(x1.w & 0x0fffffffu), fa = (int)(x1.w >> 28);
         const bool second = el >= ca;
         const int32_t s = g.items[second ? (int32_t)x1.z + (el - ca) : (int32_t)x1.y + el];
@@ -1066,27 +1130,37 @@ __global__ void fill_nodes_kernel(Node1 *p, int64_t n) {
 // ------------------------------------------------------------------------------------------
 // host drivers
 // ------------------------------------------------------------------------------------------
-int dab_exclusive_scan(dab_pair *pr, const int32_t *in, int32_t *out, int64_t n, const int32_t *n_dev,
-                       int32_t *total_out) {
+template <typename T>
+static int exclusive_scan(dab_pair *pr, const int32_t *in, T *out, int64_t n, const int32_t *n_dev, int32_t *total_out) {
   dab_ctx *ctx = pr->ctx;
   // tiles cover positions 0 .. n inclusive, so that the tile holding position n exists and writes the total
   const int nblocks = (int)(n / SCAN_TILE) + 1;
-  const size_t need = sizeof(unsigned long long) * (size_t)(nblocks + 2);
+  const size_t need = sizeof(unsigned long long) * (size_t)(ScanOps<T>::WORDS * nblocks + 2);
   if (need > pr->scan_tmp.cap || !pr->scan_tmp.p) {
     DAB_TRY(dab_ensure(ctx, pr->scan_tmp, need + 4096));
     DAB_CUDA(cudaMemsetAsync(pr->scan_tmp.p, 0, pr->scan_tmp.cap, pr->stream));   // epoch 0 = never written; ticket = 0
     pr->scan_epoch = 0;
   }
-  ScanArgs sa;
+  ScanArgs<T> sa;
   sa.in = in; sa.out = out; sa.n = n; sa.n_dev = n_dev; sa.total_out = total_out;
   sa.ticket = pr->scan_tmp.as<unsigned int>();
   sa.status = pr->scan_tmp.as<unsigned long long>() + 1;
   pr->scan_epoch = pr->scan_epoch >= 0x3ffffffe ? 1 : pr->scan_epoch + 1;
   sa.epoch = pr->scan_epoch;
-  scan_onepass_kernel<<<nblocks, SCAN_THREADS, 0, pr->stream>>>(sa);
+  scan_onepass_kernel<T><<<nblocks, SCAN_THREADS, 0, pr->stream>>>(sa);
   pr->ctx->launches += 1;
   DAB_CUDA(cudaGetLastError());
   return DAB_OK;
+}
+
+int dab_exclusive_scan(dab_pair *pr, const int32_t *in, int32_t *out, int64_t n, const int32_t *n_dev,
+                       int32_t *total_out) {
+  return exclusive_scan(pr, in, out, n, n_dev, total_out);
+}
+
+int dab_exclusive_scan(dab_pair *pr, const int32_t *in, int64_t *out, int64_t n, const int32_t *n_dev,
+                       int32_t *total_out) {
+  return exclusive_scan(pr, in, out, n, n_dev, total_out);
 }
 
 // derived counts after both tracks' not-quiet scans: hashed video frames, this shard's query range
@@ -1263,12 +1337,15 @@ static int enqueue_gate_score(dab_pair *pr, const VideoSide &vs, int32_t *dc) {
   DAB_CUDA(cudaEventRecord(pr->ev[8], st));
   // count pass, balanced over bucket entries (see gate_entries_kernel)
   DAB_TRY(dab_ensure(ctx, pr->gate_rec, sizeof(GateQ) * (size_t)(q_ub + 1)));
-  DAB_TRY(dab_ensure(ctx, pr->gate_best, sizeof(int32_t) * (size_t)(2 * (q_ub + 2))));
-  int32_t *g_best = pr->gate_best.as<int32_t>(), *g_P = g_best + (q_ub + 1);
+  DAB_TRY(dab_ensure(ctx, pr->gate_best, (sizeof(int64_t) + sizeof(int32_t)) * (size_t)(q_ub + 2)));
+  int64_t *g_P = pr->gate_best.as<int64_t>();
+  int32_t *g_best = reinterpret_cast<int32_t *>(g_P + (q_ub + 2));
   gate_plan_kernel<<<(unsigned)cdiv(q_ub, 128), 128, 0, st>>>(ga, pr->gate_rec.as<GateQ>(), g_best);
+  // 64-bit entry prefix; its total (the entries the gate visits) goes to DC_ENUM_LO / DC_ENUM_HI
   DAB_TRY(dab_exclusive_scan(pr, g_best, g_P, q_ub, nullptr, dc + DC_ENUM_LO));
   gate_entries_kernel<<<(unsigned)(8 * ctx->sm_count), GE_THREADS, 0, st>>>(ga, pr->gate_rec.as<GateQ>(), g_P);
   ctx->launches += 2;
+  // the candidate total saturates at INT32_MAX (int32 scan): a run that needs that many is refused by the collect
   DAB_TRY(dab_exclusive_scan(pr, pr->row_count.as<int32_t>(), pr->row_off.as<int32_t>(), q_ub, nullptr, dc + DC_N_CAND));
   check_capacity_kernel<<<1, 32, 0, st>>>(dc, DC_N_CAND, DC_NEED_CAND, cap_c, DAB_OVF_CAND);
   gate_fill_small_kernel<<<(unsigned)cdiv(q_ub, 256), 256, 0, st>>>(ga);
@@ -1345,8 +1422,18 @@ int dab_enqueue_stage_a_dp(dab_pair *pr) { return enqueue_dp1(pr, pr->video); }
 
 // ---- stage A, enqueued without a host round trip: prep, codes, lists, tables (own video side only), gate,
 // scoring, then DP 1 + traceback if with_dp, then the counts ----
+static const char *const kTooManyCandidates =
+    "stage A: the gate found 2147483647 or more candidates; the candidate arrays hold at most 2147483646";
+
 int dab_enqueue_stage_a(dab_pair *pr, const dab_index *ix, int64_t row_lo, int64_t row_hi, bool with_dp) {
   dab_ctx *ctx = pr->ctx;
+  if (pr->cap_cand > DAB_MAX_CANDIDATES) {
+    // the last run needed more candidates than the arrays can index (dab_collect_stage_a): not run again; the next
+    // call starts from the first guess
+    pr->cap_cand = 0;
+    dab_set_err(ctx, kTooManyCandidates);
+    return DAB_E_CAPACITY;
+  }
   DAB_TRY(ensure_hann(ctx));
   const Track &A = pr->trk[DAB_TRACK_AUDIO];
   const VideoSide &vs = ix ? ix->side : pr->video;
@@ -1414,9 +1501,15 @@ int dab_collect_stage_a(dab_pair *pr, const dab_index *ix, bool with_dp) {
   pr->stats.n_enumerated = (int64_t)(((uint64_t)(uint32_t)hc[DC_ENUM_HI] << 32) | (uint32_t)hc[DC_ENUM_LO]);
   pr->stats.n_candidates = hc[DC_N_CAND];
   if (!tables_ok || (hc[DC_OVERFLOW] & DAB_OVF_CAND)) {
+    if ((hc[DC_OVERFLOW] & DAB_OVF_CAND) && hc[DC_NEED_CAND] > DAB_MAX_CANDIDATES) {
+      pr->cap_cand = DAB_MAX_CANDIDATES + 1;     // over the limit: the next enqueue refuses instead of running again
+      dab_set_err(ctx, kTooManyCandidates);
+      return DAB_E_CAPACITY;
+    }
     // doubled, and at least the total this run needed: repeated audio (a shared tone, a looped bed) can need
     // hundreds of times the first guess, more than doubling reaches within DAB_STAGE_A_ATTEMPTS runs
-    if (hc[DC_OVERFLOW] & DAB_OVF_CAND) pr->cap_cand = std::max<int64_t>(2 * pr->cap_cand, hc[DC_NEED_CAND]);
+    if (hc[DC_OVERFLOW] & DAB_OVF_CAND)
+      pr->cap_cand = std::min(std::max<int64_t>(2 * pr->cap_cand, hc[DC_NEED_CAND]), DAB_MAX_CANDIDATES);
     dab_set_err(ctx, "stage A: a device buffer overflowed, capacity doubled");
     return DAB_E_CAPACITY;
   }
